@@ -2,6 +2,7 @@
 """bench.py -- point-pair distance evals/sec (fwd+bwd) of the HiT-ADV geometry hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl hitgeom|reference] [--workload c5shard|c1]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one forward+backward of the CW-kNN distance term (`ChamferkNNDist`, CW/kNN.py:104-108) over one
@@ -48,7 +49,12 @@ def parse():
     ap.add_argument("--no-subrecords", action="store_true",
                     help="skip the c1 / hitadv / collective sub-records of the default (c5shard) line")
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="CPU-baseline budget")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 C1_NAME = "C1: ChamferDist+HausdorffDist+KNNDist(k=5) fwd+bwd, 388x1024 clouds vs jittered copies"
@@ -190,21 +196,21 @@ def run_cpu(workload, N, budget_s, steps=None, warmup=0):
     ori_t, adv_t = torch.from_numpy(ori), torch.from_numpy(adv)
 
     def one():
+        """-> [(loss, grad)] of the step's calls"""
         if n >= 8192:  # one cloud at a time: the reference path needs ~1 GiB per [N,N] matrix at N=16384
-            for c in range(clouds):
-                step(adv_t[c : c + 1], ori_t[c : c + 1])
-        else:
-            step(adv_t, ori_t)
+            return [step(adv_t[c : c + 1], ori_t[c : c + 1]) for c in range(clouds)]
+        return [step(adv_t, ori_t)]
 
     for _ in range(warmup):
         one()
     t0 = time.time()
     for _ in range(steps):
-        one()
+        out = one()
     dt = (time.time() - t0) / steps
     sample = f"{clouds} cloud(s) x {n} points per step, {steps} step(s)" + ("" if n == N else f" (N reduced from {N}: host RAM)")
     return {"value": clouds * pairs_per_cloud(n) / dt, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample,
-            "ms_per_step": dt * 1e3}
+            "ms_per_step": dt * 1e3,
+            "outputs": {"loss": torch.stack([l.reshape(()) for l, _ in out]), "grad": torch.cat([g for _, g in out])}}
 
 
 def main_reference(args):
@@ -222,6 +228,8 @@ def main_reference(args):
             "cpu_baseline": {"value": r["value"], "unit": UNIT, "cores": r["cores"], "kind": "port", "sample": r["sample"]},
             "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, **r["outputs"])
     print(json.dumps(line), flush=True)
 
 
@@ -383,7 +391,7 @@ def distance_record(workload, B, N, name, steps, warmup, rank, world, local, wit
         # the same step with the three terms on ONE stream, for the record
         graph_serial, _ = capture(fwd_bwd_serial)
         torch.cuda.synchronize()
-        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(max(steps, 10))]
+        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         for s_, e_ in evs:
             l2_flush()
             s_.record()
@@ -409,9 +417,12 @@ def distance_record(workload, B, N, name, steps, warmup, rank, world, local, wit
     for s, e in evs:
         l2_flush()
         s.record()
-        step()
+        loss_dev = step().detach()  # detached, so the step's autograd graph is freed before the next step runs
         e.record()
     torch.cuda.synchronize()
+    # what the last timed step computed (config 1: the captured graph's output buffers, rewritten by any later replay)
+    grad_dev = (graph.hold[0] if small else adv_d.grad).detach().clone()
+    loss_dev = loss_dev.clone()
     if sampler:
         sampler.end()
     sharding.barrier()
@@ -432,14 +443,6 @@ def distance_record(workload, B, N, name, steps, warmup, rank, world, local, wit
     knn_ms, knn_n = _lib.prof_read("knn")
     _lib.prof_enable(False)
     clocks = sampler.stop() if sampler else {}
-    if small:
-        # the replays write into the gradient buffer that was current at capture time; the eager passes above replaced
-        # adv_d.grad (and the last one ran the one-stream order, which sums the three terms in another order)
-        step()
-        torch.cuda.synchronize()
-        grad_dev = graph.hold[0].detach().clone()
-    else:
-        grad_dev = adv_d.grad.detach().clone()
 
     # ---- the same step with temporal kNN seeds (attack-loop usage: KNNDist.temporal_seeds) -----------------------
     temporal = None
@@ -566,6 +569,7 @@ def distance_record(workload, B, N, name, steps, warmup, rank, world, local, wit
     if e2e is not None:
         rec["e2e"] = e2e
     rec["_grad_dev"] = grad_dev  # handed to the collective timing (config-5-size gather), dropped from the line
+    rec["_loss_dev"] = loss_dev
     return rec
 
 
@@ -640,6 +644,7 @@ def hitadv_record(rank, world, local, iters, warm_iters=5):
     modes = {}
     for graph in (False, True):
         tag = "graph" if graph else "eager"
+        n_iter = iters + CAPTURED_AFTER if graph else iters  # graph mode: `iters` replays after the eager lead-in
         try:
             attack_block(warm_iters, graph)(data_all[lo:hi], target_all[lo:hi])
             torch.cuda.synchronize()
@@ -647,7 +652,7 @@ def hitadv_record(rank, world, local, iters, warm_iters=5):
             launches0 = _lib.launch_count()
             timing = {}
             t0 = time.time()
-            adv_all, counters = sharding.run_sharded(attack_block(iters, graph), data_all, target_all, timing=timing)
+            adv_all, counters = sharding.run_sharded(attack_block(n_iter, graph), data_all, target_all, timing=timing)
             torch.cuda.synchronize()
             wall = time.time() - t0
             sharding.barrier()
@@ -665,7 +670,7 @@ def hitadv_record(rank, world, local, iters, warm_iters=5):
             modes[tag] = {"ms_per_iteration": it_ms, "cloud_iterations_per_s": world * B / (it_ms * 1e-3),
                           "attack_iters_per_s_per_batch": 1e3 / it_ms,
                           "iterations_timed": int(att.replays) if graph else iters,
-                          "e2e_ms_per_iteration": sharding.max_over_ranks(wall * 1e3 / iters),
+                          "e2e_ms_per_iteration": sharding.max_over_ranks(wall * 1e3 / n_iter),
                           "hitgeom_launches_per_iteration": int((_lib.launch_count() - launches0) // iters) if not graph else None,
                           "collective": {"op": "all_gather_into_tensor", "backend": "nccl" if world > 1 else "none (single rank)",
                                          "bytes_per_rank": timing.get("bytes_per_rank"), "bytes_total": timing.get("bytes_total"),
@@ -696,6 +701,25 @@ def hitadv_record(rank, world, local, iters, warm_iters=5):
             "note": "value = device time per inner iteration (CUDA events around the loop / the replayed iterations), max over ranks"}
 
 
+DUMP_ARRAY_BYTES = 48 << 20  # per array; the largest output is the only one near it, so a directory stays under 64 MB
+CAPTURED_AFTER = 3  # eager iterations HiT_ADV / CWKNN(graph=True) run before capturing one (hit_adv.py, cw_knn.py)
+
+
+def dump_outputs(path, **arrays):
+    """--dump-outputs: what a caller of the timed path receives from its last step, one DIR/<name>.npy per array,
+    float64 if it is float64 and float32 otherwise.  An array larger than DUMP_ARRAY_BYTES is sampled by whole clouds
+    (rows of its first axis), picked with a fixed seed from its shape alone, so runs with the same arguments store the
+    same clouds and two builds can be compared file for file."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            n = max(1, DUMP_ARRAY_BYTES // (a[0].nbytes or 1))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], n, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main_hitgeom(args):
     from hitgeom import _lib, sharding
 
@@ -705,7 +729,9 @@ def main_hitgeom(args):
     _lib.lib()  # fail loudly if the CUDA extension is missing
     B, N, name = workload_shape(args)
     rec = distance_record(args.workload, B, N, name, args.steps, args.warmup, rank, world, local)
-    grad_dev = rec.pop("_grad_dev")
+    grad_dev, loss_dev = rec.pop("_grad_dev"), rec.pop("_loss_dev")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss=loss_dev, grad=grad_dev)
     line = {"metric": METRIC, "value": rec["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
             "warmup": max(args.warmup, 3), "ms_per_step": rec["ms_per_step"], "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": rec["config"], "clocks": rec["clocks"],
@@ -722,15 +748,16 @@ def main_hitgeom(args):
         del grad_dev
         torch.cuda.empty_cache()
         try:
-            c1 = distance_record("c1", 388, 1024, C1_NAME, max(args.steps, 20), args.warmup, rank, world, local,
+            c1 = distance_record("c1", 388, 1024, C1_NAME, args.steps, args.warmup, rank, world, local,
                                  sampler_on=False)
             c1.pop("_grad_dev")
+            c1.pop("_loss_dev")
             line["c1"] = c1
         except Exception as e:  # noqa: BLE001
             line["c1"] = {"ok": False, "error": f"{type(e).__name__}: {e}"}
         torch.cuda.empty_cache()
         try:
-            line["hitadv"] = hitadv_record(rank, world, local, iters=max(20, 2 * args.steps))
+            line["hitadv"] = hitadv_record(rank, world, local, iters=args.steps)
         except Exception as e:  # noqa: BLE001
             line["hitadv"] = {"ok": False, "error": f"{type(e).__name__}: {e}"}
     if world > 1:
@@ -740,7 +767,7 @@ def main_hitgeom(args):
         return
     if world == 1 and not args.no_cpu_baseline:
         try:
-            r = run_cpu(args.workload, N, args.cpu_seconds)
+            r = run_cpu(args.workload, N, args.cpu_seconds, steps=args.steps)
             line["cpu_baseline"] = {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")}
         except Exception as e:  # the baseline must never take the GPU number down with it
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": os.cpu_count(), "kind": "port", "sample": f"failed: {e}"}
@@ -779,10 +806,11 @@ def hitadv_cpu(B, K, iters):
     model = PointNetCls(40, seed=0)
     torch.manual_seed(0)
     t0 = time.time()
-    hp.attack(model, data, target, dict(HITADV_HP, kappa=30.0, binary_step=1, num_iter=iters))
+    adv, succ, _ = hp.attack(model, data, target, dict(HITADV_HP, kappa=30.0, binary_step=1, num_iter=iters))
     dt = time.time() - t0
     return {"value": B * iters / dt, "unit": "cloud-iterations/s", "cores": os.cpu_count(), "kind": "port",
-            "sample": f"batch of {B} clouds x {K} points, {iters} iterations (incl. one-off setup)", "ms_per_step": dt / iters * 1e3}
+            "sample": f"batch of {B} clouds x {K} points, {iters} iterations (incl. one-off setup)", "ms_per_step": dt / iters * 1e3,
+            "outputs": {"adv": adv, "success": np.float64(succ)}}
 
 
 def main_hitadv(args):
@@ -793,7 +821,9 @@ def main_hitadv(args):
     if args.impl == "reference":
         if int(os.environ.get("RANK", "0")) != 0:
             return
-        r = hitadv_cpu(8, K, max(5, args.steps))
+        r = hitadv_cpu(8, K, args.steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, **r["outputs"])
         line = {"impl": "reference", "metric": HITADV_METRIC, "value": r["value"], "unit": r["unit"], "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": {"workload": name},
@@ -809,15 +839,15 @@ def main_hitadv(args):
     torch.cuda.set_device(dev)
     data, target = hitadv_inputs(B, K, 1234 + rank)
     model = PointNetCls(40, seed=0).to(dev)
-    steps = max(5, args.steps)
+    steps = args.steps
 
     def run(n_iter):
         att = HiT_ADV(model, UntargetedLogitsAdvLoss(kappa=30.0), clip_func=None, binary_step=1, num_iter=n_iter, **HITADV_HP)
         torch.manual_seed(0)
         t0 = time.time()
-        att.attack(data, target)
+        adv, succ = att.attack(data, target)
         torch.cuda.synchronize()
-        return att, time.time() - t0
+        return att, time.time() - t0, {"adv": adv, "success": np.float64(succ)}
 
     run(max(5, args.warmup))
     sampler = ClockSampler(local) if rank == 0 else None
@@ -825,9 +855,11 @@ def main_hitadv(args):
     launches0 = _lib.launch_count()
     if sampler:
         sampler.begin()
-    att, wall = run(steps)
+    att, wall, out = run(steps)
     if sampler:
         sampler.end()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **out)
     sharding.barrier()
     launches = (_lib.launch_count() - launches0) // steps
     loop_ms = sharding.max_over_ranks(att.loop_ms / steps)
@@ -853,7 +885,7 @@ def main_hitadv(args):
             from oracle import hitadv_port as hp
 
             torch.manual_seed(0)
-            n_ref = 6
+            n_ref = args.steps
             torch.cuda.synchronize()
             t0 = time.time()
             hp.attack(model, data.to(dev), target.to(dev), dict(HITADV_HP, kappa=30.0, binary_step=1, num_iter=n_ref))
@@ -869,7 +901,7 @@ def main_hitadv(args):
         except Exception as e:
             line["reference_torch_path_on_this_gpu"] = {"value": None, "what": f"failed: {e}"}
         try:
-            r = hitadv_cpu(8, K, 5)
+            r = hitadv_cpu(8, K, args.steps)
             line["cpu_baseline"] = {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")}
         except Exception as e:
             line["cpu_baseline"] = {"value": None, "unit": "cloud-iterations/s", "cores": os.cpu_count(), "kind": "port", "sample": f"failed: {e}"}
@@ -892,7 +924,8 @@ def cwknn_inputs(B, K, seed):
 
 
 def cwknn_port_run(B, K, iters, device):
-    """The reference loop (oracle/cwknn_port.py + oracle/torch_port.py, bit-identical to the reference classes on CPU)."""
+    """The reference loop (oracle/cwknn_port.py + oracle/torch_port.py, bit-identical to the reference classes on CPU)
+    -> (seconds, {"adv": adversarial clouds, "success": success count})."""
     from hitgeom import adv_utils, clip_utils
     from oracle import cwknn_port, torch_port
     from util_models import PointNetCls
@@ -903,11 +936,11 @@ def cwknn_port_run(B, K, iters, device):
     sync = torch.cuda.synchronize if device != "cpu" else (lambda: None)
     sync()
     t0 = time.time()
-    cwknn_port.attack(model, data, target, adv_utils.LogitsAdvLoss(kappa=CWKNN_HP["kappa"]), torch_port.chamfer_knn_dist,
-                      clip_utils.ClipPointsLinf(budget=CWKNN_HP["budget"]), attack_lr=CWKNN_HP["attack_lr"], num_iter=iters,
-                      device=device)
+    adv, succ = cwknn_port.attack(model, data, target, adv_utils.LogitsAdvLoss(kappa=CWKNN_HP["kappa"]),
+                                  torch_port.chamfer_knn_dist, clip_utils.ClipPointsLinf(budget=CWKNN_HP["budget"]),
+                                  attack_lr=CWKNN_HP["attack_lr"], num_iter=iters, device=device)
     sync()
-    return time.time() - t0
+    return time.time() - t0, {"adv": adv, "success": np.float64(succ)}
 
 
 def main_cwknn(args):
@@ -919,8 +952,10 @@ def main_cwknn(args):
         if int(os.environ.get("RANK", "0")) != 0:
             return
         torch.set_num_threads(os.cpu_count() or 1)
-        Bc, it = 16, max(5, args.steps)
-        dt = cwknn_port_run(Bc, K, it, "cpu")
+        Bc, it = 16, args.steps
+        dt, out = cwknn_port_run(Bc, K, it, "cpu")
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, **out)
         cb = {"value": Bc * it / dt, "unit": "cloud-iterations/s", "cores": os.cpu_count(), "kind": "port",
               "sample": f"batch of {Bc} clouds x {K} points, {it} iterations"}
         line = {"impl": "reference", "metric": CWKNN_METRIC, "value": cb["value"], "unit": cb["unit"], "n_gpus": args.gpus,
@@ -941,7 +976,8 @@ def main_cwknn(args):
     torch.cuda.set_device(dev)
     data, target = cwknn_inputs(B, K, 1234 + rank)
     model = PointNetCls(40, seed=0).to(dev)
-    iters = max(20, 10 * args.steps)
+    iters = args.steps
+    n_graph = iters + CAPTURED_AFTER  # the timed graph-mode call replays `iters` iterations after its eager lead-in
 
     def run(n_iter, graph):
         att = CWKNN(model, LogitsAdvLoss(kappa=CWKNN_HP["kappa"]), ChamferkNNDist(), ClipPointsLinf(budget=CWKNN_HP["budget"]),
@@ -949,9 +985,9 @@ def main_cwknn(args):
         torch.manual_seed(0)
         torch.cuda.synchronize()
         t0 = time.time()
-        att.attack(data, target)
+        adv, succ = att.attack(data, target)
         torch.cuda.synchronize()
-        return att, time.time() - t0
+        return att, time.time() - t0, {"adv": adv, "success": np.float64(succ)}
 
     run(max(8, args.warmup), True)
     run(max(8, args.warmup), False)
@@ -959,16 +995,18 @@ def main_cwknn(args):
     sharding.barrier()
     if sampler:
         sampler.begin()
-    att2, wall2 = run(2 * iters, True)
+    att2, wall2, out = run(n_graph, True)
     if sampler:
         sampler.end()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **out)
     sharding.barrier()
     launches0 = _lib.launch_count()
-    att_e, _ = run(iters, False)
+    att_e, _, _ = run(iters, False)
     launches = (_lib.launch_count() - launches0) // iters
     graph_ms = sharding.max_over_ranks(att2.replay_ms / max(att2.replays, 1))
     eager_ms = sharding.max_over_ranks(att_e.loop_ms / iters)
-    e2e_ms = sharding.max_over_ranks(wall2 * 1e3 / (2 * iters))
+    e2e_ms = sharding.max_over_ranks(wall2 * 1e3 / n_graph)
     clocks = sampler.stop() if sampler else {}
     if world > 1:
         torch.distributed.barrier()
@@ -985,22 +1023,22 @@ def main_cwknn(args):
                        "l2": "working set (victim activations, 388 x 1024 x 1024 floats per layer) exceeds the 126 MB L2"},
             "clocks": clocks,
             "e2e": {"value": world * B / (e2e_ms * 1e-3), "unit": "cloud-iterations/s", "ms_per_step": e2e_ms,
-                    "h2d_bytes_per_step": int(data.numel() * 4 / (2 * iters)), "d2h_bytes_per_step": int(B * K * 3 * 4 / (2 * iters))},
+                    "h2d_bytes_per_step": int(data.numel() * 4 / n_graph), "d2h_bytes_per_step": int(B * K * 3 * 4 / n_graph)},
             "gpu_launches": int(launches),
             "gpu_launches_note": "hitgeom kernel launches per iteration, counted on the eager run (a graph replay re-runs the same kernels without passing the counter)"}
     if world == 1 and not args.no_cpu_baseline:
         try:  # the reference's torch program on THIS GPU
-            n_ref = 10
+            n_ref = args.steps
             cwknn_port_run(B, K, 3, dev)
-            per_iter = cwknn_port_run(B, K, n_ref, dev) / n_ref
+            per_iter = cwknn_port_run(B, K, n_ref, dev)[0] / n_ref
             line["reference_torch_path_on_this_gpu"] = {"value": B / per_iter, "unit": "cloud-iterations/s", "ms_per_step": per_iter * 1e3,
                                                         "what": "oracle/cwknn_port.py + torch_port.py (the reference's tensor program) on cuda:0, batch %d" % B}
         except Exception as e:
             line["reference_torch_path_on_this_gpu"] = {"value": None, "what": f"failed: {e}"}
         try:
             torch.set_num_threads(os.cpu_count() or 1)
-            Bc, it = 16, 5
-            dt = cwknn_port_run(Bc, K, it, "cpu")
+            Bc, it = 16, args.steps
+            dt, _ = cwknn_port_run(Bc, K, it, "cpu")
             line["cpu_baseline"] = {"value": Bc * it / dt, "unit": "cloud-iterations/s", "cores": os.cpu_count(), "kind": "port",
                                     "sample": f"batch of {Bc} clouds x {K} points, {it} iterations"}
         except Exception as e:

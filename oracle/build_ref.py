@@ -1,5 +1,5 @@
 """Compile the UNMODIFIED reference `pointnet2_ops._ext` (the nine CUDA kernels of SURVEY.md section 2.2)
-for sm_100 into `oracle/_ref/`, straight from the sources where they lie under /root/reference.
+for sm_100 into `oracle/_ref/`, straight from the sources where they lie under $HITADV_REFERENCE.
 
 TEST INFRASTRUCTURE ONLY.  The resulting `oracle/_ref/_ext_ref.so` is the GPU-side oracle for the
 pointnet2_ops rows (a12-a17): `tests/test_gpu_pointnet2_ref.py` compares the hitgeom kernels against it
@@ -9,13 +9,13 @@ reference code enters history) but it does travel to the GPU box with the gpurun
 The only thing changed w.r.t. the reference's own build (`pointnet2_ops_lib/setup.py:19`) is the arch
 list, which upstream pins to sm_37..sm_75 (SURVEY.md R15).  No reference source is copied or edited.
 
-Runs only where /root/reference exists (the build container); on the GPU box the prebuilt .so is used.
+Runs only where $HITADV_REFERENCE names a reference checkout; elsewhere a prebuilt .so is used if present.
 """
 import glob
 import os
 import sys
 
-REF_SRC = "/root/reference/pointnet2_ops_lib/pointnet2_ops/_ext-src"
+REF_SRC = os.path.join(os.environ.get("HITADV_REFERENCE", "/nonexistent"), "pointnet2_ops_lib/pointnet2_ops/_ext-src")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 

@@ -1,8 +1,8 @@
-"""Stage the UNMODIFIED reference Python tree for the GPU box: copy every `*.py` under /root/reference into
+"""Stage the UNMODIFIED reference Python tree: copy every `*.py` under $HITADV_REFERENCE (a TRLou/HiT-ADV checkout) into
 `oracle/_ref/pytree/`, byte for byte.
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box; `oracle/_ref/` is git-ignored (no reference
-source enters the history) but travels with the gpurun snapshot, exactly like `oracle/_ref/_ext_ref.so`.  The staged
+TEST INFRASTRUCTURE ONLY.  `oracle/_ref/` is git-ignored (no reference source enters the history); copy it along to a
+GPU machine that has no reference checkout, like `oracle/_ref/_ext_ref.so`.  The staged
 tree lets `tests/test_gpu_unmodified_callers.py` run the reference's own attack classes (CW/kNN.py, CW/UKNN.py,
 ShapeAttack/HiT_ADV.py) and its evaluation block (util/other_utils.py eval_ASR) ON A B200 over hitgeom's seams
 (`hitgeom.install()` + `patch_reference()`), files unchanged.  Nothing in the product imports it.
@@ -10,12 +10,12 @@ ShapeAttack/HiT_ADV.py) and its evaluation block (util/other_utils.py eval_ASR) 
 import os
 import shutil
 
-REF = "/root/reference"
+REF = os.environ.get("HITADV_REFERENCE", "")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "pytree")
 
 
 def stage():
-    if not os.path.isdir(REF):
+    if not REF or not os.path.isdir(REF):
         return OUT if os.path.isdir(OUT) else None
     n = 0
     for root, dirs, files in os.walk(REF):

@@ -1,7 +1,6 @@
-"""Load the UNMODIFIED reference (TRLou/HiT-ADV) from /root/reference for golden-vector generation.
+"""Load the UNMODIFIED reference from $HITADV_REFERENCE (a checkout of TRLou/HiT-ADV) for golden-vector generation.
 
-Only `make_golden.py` imports this, and only in the build container: `/root/reference` does not exist on
-the GPU box, so nothing under `tests/test_*.py`, `bench.py` or `__graft_entry__.py` may import it.
+Only the `make_golden*.py` scripts import this: the reference is not part of the repository, so nothing under `tests/test_*.py`, `bench.py` or `__graft_entry__.py` may import it.
 
 What is patched (harness-side only, the reference files are read-only and untouched):
   * stub modules for the reference's absent third-party imports (`pytorch3d`, `mayavi`, `open3d`,
@@ -10,11 +9,12 @@ What is patched (harness-side only, the reference files are read-only and untouc
     `.cuda()` (`util/dist_utils.py:36,76,115,171`), run on this CPU-only box -- SURVEY.md R5.
 """
 import importlib
+import os
 import importlib.util
 import sys
 import types
 
-REF = "/root/reference"
+REF = os.environ.get("HITADV_REFERENCE", "")
 
 
 def _stub(name, **attrs):

@@ -125,13 +125,14 @@ def loss_class_cases(ref):
                 key = f"knn_k{k}_{layout}_{wtag}"
                 out[key] = loss
                 out[key + "_grad"] = a.grad
-    # internals of KNNDist for k=5 (dist_utils.py:148-166) so the oracle's intermediate tensors are pinned too
+    # internals of KNNDist for k=5 (dist_utils.py:148-166) so the oracle's intermediate tensors are pinned too; the
+    # [B,K,K] matrix itself is not stored (no test reads it, and it alone would take the file past 1 MB)
     pc = adv.transpose(2, 1)
     inner = -2.0 * torch.matmul(pc.transpose(2, 1), pc)
     xx = torch.sum(pc ** 2, dim=1, keepdim=True)
     dist = xx + inner + xx.transpose(2, 1)
     neg_value, idx = (-dist).topk(k=6, dim=-1)
-    out.update(knn_dist_matrix=dist, knn_topk_vals=-neg_value, knn_topk_idx=idx)
+    out.update(knn_topk_vals=-neg_value, knn_topk_idx=idx)
     a = adv.clone().requires_grad_()
     loss = du.ChamferkNNDist()(a, ori, weights=w, batch_avg=True)
     loss.backward()

@@ -1,7 +1,7 @@
 """The reference's OWN callers, files unchanged, executed on the B200 over hitgeom's seams.
 
-`oracle/stage_ref.py` copies the reference's Python tree byte for byte into the git-ignored, gpurun-shipped
-`oracle/_ref/pytree/` (the GPU box has no /root/reference).  A subprocess then puts that tree on sys.path, calls
+`oracle/stage_ref.py` copies the reference's Python tree ($HITADV_REFERENCE, a checkout of TRLou/HiT-ADV; not part of
+this repository) byte for byte into the git-ignored `oracle/_ref/pytree/`; without it the test skips.  A subprocess then puts that tree on sys.path, calls
 `hitgeom.install()` (pointnet2_ops._ext and pytorch3d.ops resolve to hitgeom), imports the reference modules, calls
 `hitgeom.patch_reference()` and runs, on CUDA:
 
@@ -18,6 +18,7 @@ the staged files' and that the seams really are hitgeom's (no silent fall-throug
 import os
 import subprocess
 import sys
+import tempfile
 import textwrap
 
 import pytest
@@ -144,9 +145,10 @@ SCRIPT = textwrap.dedent('''
 ''')
 
 
-@pytest.mark.skipif(not os.path.isdir(TREE), reason="oracle/_ref/pytree not staged (python oracle/stage_ref.py in the build container)")
+@pytest.mark.skipif(not os.path.isdir(TREE), reason="needs the unmodified TRLou/HiT-ADV Python tree in oracle/_ref/pytree: "
+                                                    "HITADV_REFERENCE=<checkout> python oracle/stage_ref.py")
 def test_unmodified_reference_callers_run_on_cuda_over_hitgeom():
     out = subprocess.run([sys.executable, "-c", SCRIPT % {"root": ROOT, "tree": TREE}], capture_output=True, text=True,
-                         timeout=900, cwd="/tmp")
+                         timeout=900, cwd=tempfile.gettempdir())
     assert out.returncode == 0 and "CALLERS_OK" in out.stdout, (out.stdout[-2000:], out.stderr[-4000:])
     print(out.stdout[-600:])
