@@ -48,6 +48,8 @@ HG_API int hg_tune(const char *key, int value) {
     g_hg_tune_small_fused_off = value;
     return HG_OK;
   }
+  // "prune" (0 = all-pairs kernels only, 1 = automatic), "prune_min_n" (size threshold, 0 = default), "prune_count"
+  if (hg_prune_tune(key, value)) return HG_OK;
   hg_set_error("hg_tune: unknown key '%s'", key);
   return HG_E_BADARG;
 }

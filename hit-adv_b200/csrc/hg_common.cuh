@@ -204,6 +204,25 @@ __device__ __forceinline__ int hg_csr_next(const int *__restrict__ list, int p0,
 bool hg_knn_tc_supported(int K, int C, int k1);
 int hg_knn_tc_run(const float *pc, const float *xx, int B, int K, int C, int k1, float *vals, int *idx, cudaStream_t stream);
 
+// ---- spatially pruned exact passes for large clouds (hg_prune.cu) ---------------------------------------------------
+#define HG_PRUNE_MAX_N 16384  // the ordering build sorts one cloud in shared memory with 14-bit point indices
+// One cloud batch in kd-tree order: points (x, y, z, squared norm), original index of every sorted point, per-leaf
+// boxes (lo, hi) of 32 points, per-cloud (bound on max |p|^2, 1 if the cloud must take the all-pairs kernels).
+struct HgPruneOrder {
+  float4 *pts;   // [B,N]
+  int *perm;     // [B,N]
+  float4 *box;   // [B,ceil(N/32),2]
+  float4 *info;  // [B]
+  int N;
+};
+int hg_prune_tune(const char *key, int value);  // 1 if the key is one of the pruned path's
+bool hg_prune_applies(int N);               // the size threshold and hg_tune("prune") as they stand
+size_t hg_prune_order_bytes(int B, int N);  // 0 when the path does not apply to N
+int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream);
+int hg_prune_nn_search(const HgPruneOrder &q, const HgPruneOrder &c, int B, float *mins, int *args, cudaStream_t stream);
+int hg_prune_knn_search(const HgPruneOrder &o, int B, int k1, const float *thr0, float *vals, int *idx, int *idx_state,
+                        cudaStream_t stream);
+
 // ---- 3-D streaming kNN (hg_knn3.cu) ---------------------------------------------------------------------------
 #define HG_KNN_FORM_EXPANDED 0  // dist = (xx_j + (-2 zz)) + xx_i   (KNNDist / DGCNN)
 #define HG_KNN_FORM_DIRECT 1    // dist = fma(dz,dz, fma(dy,dy, dx*dx))   (pytorch3d knn_points)

@@ -548,10 +548,11 @@ static bool knn3_pad_candidate(int K, int k1) { return k1 >= 12 && hg_knn_tc_sup
 HG_API size_t hg_knn_self_workspace_bytes(int B, int K, int C, int k1) {
   if (B <= 0 || K <= 0 || C <= 0) return 0;
   if (C == 3) {
-    size_t w = hg_knn3_seed_workspace_bytes(B, K);
+    size_t w = 0;
     if (knn3_pad_candidate(K, k1))  // padded copy + squared norms for the tensor-core kernel
-      w += hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
-    return w;
+      w = hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
+    const size_t order = hg_prune_order_bytes(B, K);  // kd-tree ordering of the pruned path, in the same place
+    return hg_knn3_seed_workspace_bytes(B, K) + (w > order ? w : order);
   }
   size_t per = (size_t)K * K * sizeof(float);
   size_t nb = kGenericScratchBytes / per;
@@ -581,6 +582,8 @@ HG_API int hg_knn_self_temporal_f32(const float *pc, int B, int K, int C, int k1
     // 192: 326 / 313; 2048 points: 32 clouds 196 / 244, 96: 485 / 464); KNNDist's short lists (and its temporal state) stay 3-D
     const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, K);
     const size_t pad_ws = hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
+    if (hg_prune_applies(K))  // large clouds: pruned search, whatever the list length
+      return hg_knn3_self_seeded_i32(pc, B, K, k1, vals, idx, workspace, workspace_bytes, stream, idx_state, state_valid);
     if (!idx_state && knn3_pad_candidate(K, k1) && g_hg_tune_knn_tc_off != 1 && workspace &&
         workspace_bytes >= seed_ws + pad_ws &&
         ((4LL * B * ((K + 127) / 128) >= hg_sm_count() && (long long)B * ((K + 127) / 128) <= 8LL * hg_sm_count()) ||

@@ -42,6 +42,16 @@ __device__ __forceinline__ float knn_dist_exact(float a0, float a1, float a2, fl
   }
 }
 
+// exact distance for the threshold seeds: a NaN distance (a non-finite coordinate) never enters a list, so it counts as
+// +inf here.  Left as NaN it would break the min/max insertion networks below (fminf / fmaxf drop it and the level
+// duplicates its entry, leaving a bound under the true k-th value) and the max of the temporal seeds (a bound resting
+// on k1 - 1 real candidates).
+__device__ __forceinline__ float knn_seed_dist(float a0, float a1, float a2, float a3, float c0, float c1, float c2,
+                                               float cw) {
+  const float d = knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, c0, c1, c2, cw);
+  return d == d ? d : CUDART_INF_F;
+}
+
 // The main loop never needs the distance itself, only whether it is below the query's threshold -- and that test
 // can be folded into the last addition.  EXPANDED: d = fl(s + a3) with s = fl(cw + nzz); with the addend
 // af = rd(a3 - thr) the sign bit of fl(s + af) is set iff s < ru(thr - a3) (a sum of two floats never rounds to
@@ -131,7 +141,10 @@ __global__ void __launch_bounds__(kThreads) knn3_kernel(const float *__restrict_
                                                         const float *__restrict__ thr0 /*[B,Nq] or null*/,
                                                         const float *__restrict__ sbound /*FOLD4: [B] stride 8,
                                                         upper bound on max |candidate|^2*/,
-                                                        int *__restrict__ idx_state /*second copy of idx or null*/) {
+                                                        int *__restrict__ idx_state /*second copy of idx or null*/,
+                                                        const float4 *__restrict__ only /*null, or per-cloud info of
+                                                        a pruned-path ordering: flagged clouds only*/) {
+  if (only != nullptr && only[blockIdx.y].y == 0.f) return;
   constexpr int kTilePairs = 32 * GP;
   constexpr int kTileC = 2 * kTilePairs;
   __shared__ float4 cand[2 * kTilePairs];  // two float4 per candidate pair
@@ -573,7 +586,7 @@ __global__ void __launch_bounds__(256) knn_seed_small_kernel(const float *__rest
     const int t0 = max(0, min(s - win / 2, N - win)), t1 = min(N, t0 + win);
     for (int t = t0; t < t1; ++t) {
       const float4 r = spts[t];
-      float d = knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, r.x, r.y, r.z, r.w);
+      float d = knn_seed_dist(a0, a1, a2, a3, r.x, r.y, r.z, r.w);
 #pragma unroll
       for (int u = 0; u < KM; ++u) {  // v stays sorted ascending: each level keeps the smaller, passes the larger on
         const float l = fminf(v[u], d);
@@ -595,15 +608,16 @@ static int g_force_qt = 0, g_force_gp = 0;
 
 template <int FORM, int QT, int KM, typename IdxT>
 int launch_qt(const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, IdxT *idx,
-              const float *thr0, const float *sbound, cudaStream_t stream, int *idx_state = nullptr) {
+              const float *thr0, const float *sbound, cudaStream_t stream, int *idx_state = nullptr,
+              const float4 *only = nullptr) {
   dim3 grid((Nq + QT * kThreads - 1) / (QT * kThreads), B);
   const bool prof = hg_prof_begin(HG_PROF_KNN, stream);
   // 8 candidates per hit bit (512-candidate tiles) for long candidate lists, 4 (256) for short ones, where the
   // cheaper group re-evaluation in the drain outweighs the extra mask updates (measured cross-over ~2-4k)
   if (g_force_gp ? g_force_gp == 2 : Nr < 2048)
-    knn3_kernel<FORM, QT, KM, 2, IdxT><<<grid, kThreads, 0, stream>>>(q, r, Nq, Nr, k1, vals, idx, thr0, sbound, idx_state);
+    knn3_kernel<FORM, QT, KM, 2, IdxT><<<grid, kThreads, 0, stream>>>(q, r, Nq, Nr, k1, vals, idx, thr0, sbound, idx_state, only);
   else
-    knn3_kernel<FORM, QT, KM, 4, IdxT><<<grid, kThreads, 0, stream>>>(q, r, Nq, Nr, k1, vals, idx, thr0, sbound, idx_state);
+    knn3_kernel<FORM, QT, KM, 4, IdxT><<<grid, kThreads, 0, stream>>>(q, r, Nq, Nr, k1, vals, idx, thr0, sbound, idx_state, only);
   hg_prof_end(HG_PROF_KNN, stream, prof);
   HG_CHECK_LAUNCH("knn3_kernel");
   return HG_OK;
@@ -611,7 +625,8 @@ int launch_qt(const float *q, const float *r, int B, int Nq, int Nr, int k1, flo
 
 template <int FORM, typename IdxT>
 int launch_form(const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, IdxT *idx,
-                const float *thr0, const float *sbound, cudaStream_t stream, int *idx_state = nullptr) {
+                const float *thr0, const float *sbound, cudaStream_t stream, int *idx_state = nullptr,
+                const float4 *only = nullptr) {
   if (k1 < 1 || k1 > 64) {
     hg_set_error("knn: k=%d outside [1,64]", k1);
     return HG_E_UNSUPPORTED;
@@ -625,16 +640,16 @@ int launch_form(const float *q, const float *r, int B, int Nq, int Nr, int k1, f
   const bool short_list = Nr < 2048;
   if (g_force_qt) {
     const int qt = g_force_qt;
-    if (k1 <= 6 && qt == 4) return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (k1 <= 6 && qt == 2) return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (k1 <= 6 && qt == 1) return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+    if (k1 <= 6 && qt == 4) return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+    if (k1 <= 6 && qt == 2) return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+    if (k1 <= 6 && qt == 1) return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
     if (k1 > 6 && k1 <= 20 && qt == 2)
-      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
     if (k1 > 6 && k1 <= 20 && qt == 1)
-      return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
     if (k1 > 20 && k1 <= 32 && qt == 1)
-      return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (k1 > 32 && qt == 1) return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+    if (k1 > 32 && qt == 1) return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
     hg_set_error("knn: forced QT=%d has no instantiation for k=%d", qt, k1);
     return HG_E_UNSUPPORTED;
   }
@@ -642,19 +657,19 @@ int launch_form(const float *q, const float *r, int B, int Nq, int Nr, int k1, f
     // (four queries per lane need twice the CTAs to pay: 32 x 8192: 654 us with two against 695, 16 x 16384: 1080 / 1128;
     // 64 x 8192 and up: four win -- tools/debug/knn_small_shapes.py big)
     if (!short_list && Nq >= 3 * kThreads && ctas(4) >= 2 * want)
-      return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
     if (Nq > kThreads && ctas(2) >= want)
-      return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
-    return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+    return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
   }
   if (k1 <= 20) {
     if (!short_list && Nq > kThreads && ctas(2) >= want)
-      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
-    return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+    return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
   }
-  if (k1 <= 32) return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+  if (k1 <= 32) return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
   // 33..64 neighbours (HiT-ADV's default curv_loss_knn = 32 asks knn_points for 33): a 64-entry register list
-  return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state);
+  return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
 }
 
 // ---- threshold seeding for self-kNN ---------------------------------------------------------------------------
@@ -788,8 +803,8 @@ __global__ void __launch_bounds__(128) knn_seed_kernel(const float4 *__restrict_
     seen += max(te - t, 0);
     for (; t + 1 < te; t += 2) {  // two candidates in flight; insertion without branches (values only)
       const float4 r0 = pts[t], r1 = pts[t + 1];
-      float d0 = knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
-      float d1 = knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, r1.x, r1.y, r1.z, r1.w);
+      float d0 = knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
+      float d1 = knn_seed_dist(a0, a1, a2, a3, r1.x, r1.y, r1.z, r1.w);
 #pragma unroll
       for (int u = 0; u < KM; ++u) {  // v stays sorted ascending: each level keeps the smaller, passes the larger on
         const float lo0 = fminf(v[u], d0);
@@ -805,7 +820,7 @@ __global__ void __launch_bounds__(128) knn_seed_kernel(const float4 *__restrict_
     }
     if (t < te) {
       const float4 r0 = pts[t];
-      float d0 = knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
+      float d0 = knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
 #pragma unroll
       for (int u = 0; u < KM; ++u) {
         const float lo0 = fminf(v[u], d0);
@@ -870,7 +885,7 @@ __global__ void __launch_bounds__(256) knn_seed_prev_kernel(const float *__restr
           ok = false;
         } else {
           const float cx = __ldg(p + (size_t)j * 3), cy = __ldg(p + (size_t)j * 3 + 1), cz = __ldg(p + (size_t)j * 3 + 2);
-          bound = fmaxf(bound, knn_dist_exact<HG_KNN_FORM_EXPANDED>(a0, a1, a2, a3, cx, cy, cz, hg_sumsq3_seq(cx, cy, cz)));
+          bound = fmaxf(bound, knn_seed_dist(a0, a1, a2, a3, cx, cy, cz, hg_sumsq3_seq(cx, cy, cz)));
         }
       }
     }
@@ -1045,6 +1060,28 @@ HG_API void hg_knn_tune_small(int small_max_n) { g_small_max_n = small_max_n; }
 // seeds when state_valid, and overwritten with this call's indices (a second copy of idx).
 int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, void *workspace,
                             size_t workspace_bytes, cudaStream_t stream, int *idx_state, int state_valid) {
+  const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, N);
+  if (hg_prune_applies(N) && workspace != nullptr && workspace_bytes >= seed_ws + hg_prune_order_bytes(B, N)) {
+    // large clouds: kd-tree ordering and pruned search (hg_prune.cu), seeded from each query's own leaf or, with
+    // temporal seeds, from the previous call's neighbours; clouds the ordering flags (non-finite coordinates) then
+    // take the all-pairs kernel with the reference arithmetic
+    float *sb = (float *)((char *)workspace + hg_align((size_t)B * N * sizeof(int)));
+    float *thr = (float *)((char *)sb + hg_align((size_t)B * 8 * sizeof(float)));
+    const float *thr0 = nullptr;
+    if (idx_state && state_valid) {
+      int rc = launch_seed_prev(pc, B, N, k1, idx_state, thr, sb, stream);
+      if (rc) return rc;
+      thr0 = thr;
+    }
+    HgPruneOrder o;
+    const bool prof = hg_prof_begin(HG_PROF_KNN, stream);
+    int rc = hg_prune_build(pc, B, N, false, (char *)workspace + seed_ws, &o, stream);
+    if (!rc) rc = hg_prune_knn_search(o, B, k1, thr0, vals, idx, idx_state, stream);
+    hg_prof_end(HG_PROF_KNN, stream, prof);
+    if (rc) return rc;
+    return launch_form<HG_KNN_FORM_EXPANDED, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, nullptr, stream, idx_state,
+                                                  o.info);
+  }
   if (k1 > 32 || workspace == nullptr || workspace_bytes < hg_knn3_seed_workspace_bytes(B, N))
     return launch_form<HG_KNN_FORM_EXPANDED, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, nullptr, stream, idx_state);
   float *sb_slot = (float *)((char *)workspace + hg_align((size_t)B * N * sizeof(int)));  // `params`: [B] stride 8

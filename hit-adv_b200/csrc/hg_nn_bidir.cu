@@ -46,7 +46,13 @@ struct NnParams {
   unsigned *rowsec;             // [B,N2]  ord(smallest tracked value outside the winning lane's columns)
   const float *eps2;            // [B]     2 * (bound on |tracked - reference value|) for this pair of clouds
   int *amb;                     // [1 + B*(N1+N2)]  counter, then the entries the finish kernel could not settle
+  // null, or the per-cloud info of the two pruned-path orderings: only the clouds they flag are computed here
+  const float4 *only_a, *only_b;
 };
+
+__device__ __forceinline__ bool nn_skip(const NnParams &p, int b) {
+  return p.only_a != nullptr && p.only_a[b].y == 0.f && p.only_b[b].y == 0.f;
+}
 
 // exact P for the finish kernel; identical operation sequence to the packed main loop
 __device__ __forceinline__ float nn_p_exact(float x0, float x1, float x2, float y0, float y1, float y2) {
@@ -70,6 +76,7 @@ __global__ void __launch_bounds__(WARPS * 32, (T == 8 ? 16 : 12) / WARPS) nn_bid
   int *scid = reinterpret_cast<int *>(sprev + T * WARPS * 32);                     // [T][WARPS*32]
 
   const int b = blockIdx.z;
+  if (nn_skip(p, b)) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int cgroup = blockIdx.y * WARPS + warp;  // global column group (32*T columns)
   const int cbase = cgroup * 32 * T + lane * T;
@@ -223,6 +230,7 @@ __global__ void __launch_bounds__(256) nn_bidir_d3_finish_kernel(NnParams p, int
        g += (long long)gridDim.x * blockDim.x) {
     const int b = (int)(g / (p.N1 + p.N2));
     const int e = (int)(g % (p.N1 + p.N2));
+    if (nn_skip(p, b)) continue;
     const float *gx = p.gts + (size_t)b * p.N2 * 3;
     const float *gy = p.preds + (size_t)b * p.N1 * 3;
     if (e < p.N1) {  // column j: nearest row inside the recorded batch of kColBatch rows
@@ -290,6 +298,7 @@ __global__ void __launch_bounds__(256) nn_bidir_d3_finish_small_kernel(NnParams 
   extern __shared__ float fsm[];
   const int b = blockIdx.x, tid = threadIdx.x;
   const int N1 = p.N1, N2 = p.N2;
+  if (nn_skip(p, b)) return;
   const float *gx = p.gts + (size_t)b * N2 * 3;
   const float *gy = p.preds + (size_t)b * N1 * 3;
   if ((int)blockIdx.y < ncolcta) {
@@ -958,11 +967,16 @@ HG_API void hg_nn_bidir_tune(int T, int RB) {
   g_force_RB = RB;
 }
 
+// merged (value, cell) keys, runner-up values, per-cloud error bound, ambiguity list
+static size_t nn_d3_bytes(int B, int N2, int N1) {
+  return hg_align((size_t)B * N1 * 8) + hg_align((size_t)B * N2 * 8) + hg_align((size_t)B * N1 * 4) +
+         hg_align((size_t)B * N2 * 4) + hg_align((size_t)B * 4) + hg_align(((size_t)B * (N1 + N2) + 1) * 4);
+}
+
 HG_API size_t hg_nn_bidir_workspace_bytes(int B, int N2, int N1, int D) {
   if (B <= 0 || N1 <= 0 || N2 <= 0 || D <= 0) return 0;
-  if (D == 3)  // merged (value, cell) keys, runner-up values, per-cloud error bound, ambiguity list
-    return hg_align((size_t)B * N1 * 8) + hg_align((size_t)B * N2 * 8) + hg_align((size_t)B * N1 * 4) +
-           hg_align((size_t)B * N2 * 4) + hg_align((size_t)B * 4) + hg_align(((size_t)B * (N1 + N2) + 1) * 4);
+  if (D == 3)  // + the kd-tree orderings of both clouds when the pruned path applies
+    return nn_d3_bytes(B, N2, N1) + hg_prune_order_bytes(B, N2) + hg_prune_order_bytes(B, N1);
   return hg_align((size_t)B * N2 * N1 * sizeof(float));
 }
 
@@ -1007,8 +1021,26 @@ HG_API int hg_nn_bidir_f32(const float *gts, const float *preds, int B, int N2, 
   p.eps2 = eps2;
   w += hg_align((size_t)B * 4);
   p.amb = (int *)w;
+  p.only_a = p.only_b = nullptr;
+  // large clouds: kd-tree orderings and pruned 1-NN passes in both directions (hg_prune.cu); the all-pairs kernels below
+  // then run on the clouds the ordering build flagged (non-finite coordinates) only
+  const bool prune = hg_prune_applies(N1) && hg_prune_applies(N2) &&
+                     workspace_bytes >= nn_d3_bytes(B, N2, N1) + hg_prune_order_bytes(B, N2) + hg_prune_order_bytes(B, N1);
+  if (prune) {
+    char *ow = (char *)workspace + nn_d3_bytes(B, N2, N1);
+    HgPruneOrder og, op;
+    const bool prof = hg_prof_begin(HG_PROF_NN_BIDIR, stream);
+    int rc = hg_prune_build(gts, B, N2, true, ow, &og, stream);
+    if (!rc) rc = hg_prune_build(preds, B, N1, true, ow + hg_prune_order_bytes(B, N2), &op, stream);
+    if (!rc) rc = hg_prune_nn_search(op, og, B, min1, arg1, stream);  // column j (preds): nearest row (gts)
+    if (!rc) rc = hg_prune_nn_search(og, op, B, min2, arg2, stream);  // row i (gts): nearest column (preds)
+    hg_prof_end(HG_PROF_NN_BIDIR, stream, prof);
+    if (rc) return rc;
+    p.only_a = og.info;
+    p.only_b = op.info;
+  }
   // the approximate tracker (4 FMA-pipe operations per pair, exact recovery in the finish kernels) when switched on
-  const bool approx = !g_hg_tune_nn_exact && (double)B * (N1 + N2) < 2.0e9;
+  const bool approx = !prune && !g_hg_tune_nn_exact && (double)B * (N1 + N2) < 2.0e9;
   HG_CUDA(cudaMemsetAsync(workspace, 0xff, (size_t)((char *)eps2 - (char *)workspace), stream));
   if (approx) {
     HG_CUDA(cudaMemsetAsync(p.amb, 0, sizeof(int), stream));

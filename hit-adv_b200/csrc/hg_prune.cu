@@ -1,0 +1,553 @@
+// hg_prune.cu -- exact, spatially pruned nearest-neighbour (Chamfer, both directions) and self-kNN passes for large
+// clouds.
+//
+// The all-pairs kernels (hg_nn_bidir.cu, hg_knn3.cu) evaluate every (query, candidate) pair; at 16384 points a query's
+// few nearest neighbours lie within ~1 % of the cloud.  Here every cloud is first put in kd-tree order (leaves of 32
+// points with tight axis-aligned boxes), then a warp owns one leaf of 32 queries and visits candidate leaves in
+// tree order starting from the nearest one (own leaf for self-kNN), skipping a whole leaf when no lane can find
+// anything in it:
+//     lowerbound(D^2(query or query box, leaf box)) > thr + slack,    slack = 1.5e-6 (S + thr) >= 24 u (S + thr),
+// D^2 computed with rounding toward -inf, thr the lane's current exact threshold (1-NN: best value so far; kNN: the
+// k-th listed value nudged up one ulp, or a seed), S = (|q| + max|c|)^2.  The reference's FP32 value undershoots the
+// real squared distance by at most ~9 u S (DESIGN 5.1, 5.2), so a skipped leaf holds no candidate whose reference
+// value is <= thr: ties at the threshold are always visited.  Visited leaves go through the packed arithmetic of the
+// all-pairs kernels (Chamfer: P = (rx + ry) + zz', zz' = fma(x2',y2, fma(x1',y1, x0'*y0)), x' = -2x, which gives the
+// same bits with the roles of the two points swapped; kNN: the 4-operation folded sign-bit filter and an exact drain).
+// Leaves are not visited in index order, so every selection compares (value, original index) lexicographically:
+// results equal the all-pairs kernels' bit for bit (first index among equal values).
+//
+// A cloud with a non-finite coordinate or a squared norm >= 1e36 is flagged by the ordering build; the search skips
+// it and the caller runs the all-pairs kernels on the flagged clouds only (documented NaN behaviour unchanged).
+#include <string.h>
+
+#include "hg_common.cuh"
+
+namespace {
+
+constexpr int kLeaf = 32;
+constexpr int kIdxBits = 14;  // sort keys: 18 bits of quantised coordinate, 14 bits of point index
+constexpr unsigned kIdxMask = (1u << kIdxBits) - 1u;
+constexpr unsigned kPadKey = 0xffffffffu;
+constexpr float kQuantMax = 262142.f;  // 2^18 - 2: a real key never equals kPadKey
+constexpr int kBuildThreads = 1024;
+constexpr int kMaxSegs = HG_PRUNE_MAX_N / 64;  // segments of the last split level
+constexpr int kSearchWarps = 4;
+constexpr float kSlack = 1.5e-6f;  // >= 24 u, u = 2^-24
+
+__device__ unsigned long long g_prune_tiles[4];  // nn: visited, total leaf pairs; knn: visited, total
+
+__device__ __forceinline__ float gap_rd(float alo, float ahi, float blo, float bhi) {
+  return fmaxf(fmaxf(__fsub_rd(blo, ahi), __fsub_rd(alo, bhi)), 0.f);
+}
+// lower bound on the squared distance between two boxes (a point is a box with lo == hi)
+__device__ __forceinline__ float box_d2_rd(float4 alo, float4 ahi, float4 blo, float4 bhi) {
+  const float gx = gap_rd(alo.x, ahi.x, blo.x, bhi.x), gy = gap_rd(alo.y, ahi.y, blo.y, bhi.y),
+              gz = gap_rd(alo.z, ahi.z, blo.z, bhi.z);
+  return __fadd_rd(__fadd_rd(__fmul_rd(gx, gx), __fmul_rd(gy, gy)), __fmul_rd(gz, gz));
+}
+__device__ __forceinline__ bool may_hold(float lb, float thr, float S) { return !(lb > thr + kSlack * (S + thr)); }
+
+// ---- ordering build: one CTA per cloud, kd splits (median of the longest axis) by a segmented bitonic sort ----------
+// key[i] = (quantised coordinate on the segment's split axis) << 14 | point index; padding to a power of two carries
+// kPadKey and stays at the end of the array at every level.  Correctness never depends on the quality of a split:
+// the leaf boxes are recomputed from the points.
+template <bool CHAMFER_NORM>
+__global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float *__restrict__ pc, int N, int Np,
+                                                                    HgPruneOrder o) {
+  extern __shared__ unsigned key[];  // [Np]
+  __shared__ unsigned smin[3][kMaxSegs], smax[3][kMaxSegs];
+  __shared__ float slo[kMaxSegs], sscale[kMaxSegs];
+  __shared__ int saxis[kMaxSegs];
+  __shared__ unsigned s_bad, s_norm;
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  const float *p = pc + (size_t)b * N * 3;
+  if (tid == 0) {
+    s_bad = 0u;
+    s_norm = 0u;
+  }
+  __syncthreads();
+  float mn = 0.f;
+  bool bad = false;
+  for (int i = tid; i < Np; i += kBuildThreads) {
+    key[i] = i < N ? (unsigned)i : kPadKey;
+    if (i < N) {
+      const float x = p[(size_t)i * 3], y = p[(size_t)i * 3 + 1], z = p[(size_t)i * 3 + 2];
+      bad |= !(isfinite(x) && isfinite(y) && isfinite(z));
+      mn = fmaxf(mn, fmaf(z, z, fmaf(y, y, x * x)));
+    }
+  }
+  mn = hg_warp_max_f32(mn);
+  bad = __any_sync(0xffffffffu, bad);
+  if (lane == 0) {
+    atomicMax(&s_norm, __float_as_uint(mn));
+    if (bad) s_bad = 1u;
+  }
+  __syncthreads();
+  const float norm = __uint_as_float(s_norm);
+  const bool flagged = s_bad != 0u || !(norm < 1e36f);
+  if (tid == 0) o.info[b] = make_float4(norm * 1.0001f, flagged ? 1.f : 0.f, 0.f, 0.f);
+  if (flagged) return;
+
+  for (int s = Np; s > kLeaf; s >>= 1) {
+    const int nseg = Np / s;
+    for (int t = tid; t < nseg; t += kBuildThreads)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        smin[c][t] = 0xffffffffu;
+        smax[c][t] = 0u;
+      }
+    __syncthreads();
+    for (int i = tid; i < Np; i += kBuildThreads) {  // s >= 64: the 32 entries of a warp lie in one segment
+      const unsigned e = key[i];
+      const bool real = e != kPadKey;
+      const int id = (int)(e & kIdxMask);
+      const int seg = i / s;
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const unsigned u = real ? hg_ord(p[(size_t)id * 3 + c]) : 0u;
+        const unsigned lo = __reduce_min_sync(0xffffffffu, real ? u : 0xffffffffu);
+        const unsigned hi = __reduce_max_sync(0xffffffffu, u);
+        if (lane == 0) {
+          atomicMin(&smin[c][seg], lo);
+          atomicMax(&smax[c][seg], hi);
+        }
+      }
+    }
+    __syncthreads();
+    for (int t = tid; t < nseg; t += kBuildThreads) {
+      float lo[3], ext[3];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        lo[c] = hg_unord(smin[c][t]);
+        ext[c] = hg_unord(smax[c][t]) - lo[c];  // NaN for a segment of padding only
+      }
+      int ax = 0;
+      if (ext[1] > ext[ax]) ax = 1;
+      if (ext[2] > ext[ax]) ax = 2;
+      saxis[t] = ax;
+      slo[t] = lo[ax];
+      sscale[t] = ext[ax] > 0.f ? kQuantMax / ext[ax] : 0.f;
+    }
+    __syncthreads();
+    for (int i = tid; i < Np; i += kBuildThreads) {
+      const unsigned e = key[i];
+      if (e == kPadKey) continue;
+      const int seg = i / s, id = (int)(e & kIdxMask);
+      const float f = (p[(size_t)id * 3 + saxis[seg]] - slo[seg]) * sscale[seg];
+      key[i] = ((unsigned)fminf(fmaxf(f, 0.f), kQuantMax) << kIdxBits) | (unsigned)id;
+    }
+    __syncthreads();
+    // bitonic sort of every segment of s entries, all segments ascending
+    for (int k = 2; k <= s; k <<= 1)
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        for (int t = tid; t < Np / 2; t += kBuildThreads) {
+          const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1)), c = a + j;
+          const bool asc = k == s || (a & k) == 0;
+          const unsigned x = key[a], y = key[c];
+          if ((x > y) == asc) {
+            key[a] = y;
+            key[c] = x;
+          }
+        }
+        __syncthreads();
+      }
+  }
+
+  for (int i = tid; i < N; i += kBuildThreads) {
+    const int id = (int)(key[i] & kIdxMask);
+    const float x = p[(size_t)id * 3], y = p[(size_t)id * 3 + 1], z = p[(size_t)id * 3 + 2];
+    const float w = CHAMFER_NORM ? hg_dot3_fma(x, y, z, x, y, z) : hg_sumsq3_seq(x, y, z);
+    o.pts[(size_t)b * N + i] = make_float4(x, y, z, w);
+    o.perm[(size_t)b * N + i] = id;
+  }
+  const int nleaf = (N + kLeaf - 1) / kLeaf;
+  for (int L = tid >> 5; L < nleaf; L += kBuildThreads / 32) {
+    const int i = L * kLeaf + lane;
+    float v[3] = {0.f, 0.f, 0.f};
+    if (i < N) {
+      const int id = (int)(key[i] & kIdxMask);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) v[c] = p[(size_t)id * 3 + c];
+    }
+    float lo[3], hi[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      lo[c] = hg_warp_min_f32(i < N ? v[c] : CUDART_INF_F);
+      hi[c] = hg_warp_max_f32(i < N ? v[c] : -CUDART_INF_F);
+    }
+    if (lane == 0) {
+      o.box[((size_t)b * nleaf + L) * 2] = make_float4(lo[0], lo[1], lo[2], 0.f);
+      o.box[((size_t)b * nleaf + L) * 2 + 1] = make_float4(hi[0], hi[1], hi[2], 0.f);
+    }
+  }
+}
+
+struct PruneSearch {
+  HgPruneOrder q, c;
+  int self;  // candidates are the query cloud (self-kNN): the visit starts at the query's own leaf
+  int k1;
+  float *vals;        // kNN [B,Nq,k1] (may be null), 1-NN [B,Nq]
+  int *idx;           // same shape
+  int *idx_state;     // kNN: second copy of idx or null
+  const float *thr0;  // kNN: [B,Nq] exact upper bounds by original index, or null
+  unsigned long long *count;  // null, or {visited leaf pairs, all leaf pairs}
+};
+
+// Sorted list with the lexicographic (value, index) order, held in registers (static indexing only).
+template <int KM>
+struct LexTopK {
+  float v[KM];
+  int id[KM];
+  __device__ __forceinline__ void init() {
+#pragma unroll
+    for (int t = 0; t < KM; ++t) {
+      v[t] = CUDART_INF_F;
+      id[t] = 0;
+    }
+  }
+  __device__ __forceinline__ void push(float d, int j) {
+    if (d < v[KM - 1] || (d == v[KM - 1] && j < id[KM - 1])) {
+      v[KM - 1] = d;
+      id[KM - 1] = j;
+#pragma unroll
+      for (int t = KM - 1; t > 0; --t) {
+        if (v[t] < v[t - 1] || (v[t] == v[t - 1] && id[t] < id[t - 1])) {
+          const float tv = v[t];
+          v[t] = v[t - 1];
+          v[t - 1] = tv;
+          const int ti = id[t];
+          id[t] = id[t - 1];
+          id[t - 1] = ti;
+        }
+      }
+    }
+  }
+  __device__ __forceinline__ float kth(int k1) const {
+    float r = v[0];
+#pragma unroll
+    for (int t = 1; t < KM; ++t)
+      if (t == k1 - 1) r = v[t];
+    return r;
+  }
+};
+
+__device__ __forceinline__ float nudge_up(float v) { return v < CUDART_INF_F ? nextafterf(v, CUDART_INF_F) : v; }
+
+// KM == 1: 1-NN with the Chamfer arithmetic; KM > 1: kNN list with the KNNDist arithmetic and the folded filter.
+template <int KM>
+__global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSearch a) {
+  __shared__ float4 tile[kSearchWarps][kLeaf];  // 16 candidate pairs: (c0_j,c0_j1,c1_j,c1_j1), (c2_j,c2_j1,w_j,w_j1)
+  __shared__ int tperm[kSearchWarps][kLeaf];
+  constexpr bool kNN1 = KM == 1;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, b = blockIdx.y;
+  const int Nq = a.q.N, Nc = a.c.N;
+  const int nlq = (Nq + kLeaf - 1) / kLeaf, nlc = (Nc + kLeaf - 1) / kLeaf;
+  const int Lq = blockIdx.x * kSearchWarps + warp;
+  if (Lq >= nlq) return;
+  const float4 qinfo = a.q.info[b], cinfo = a.c.info[b];
+  if (qinfo.y != 0.f || cinfo.y != 0.f) return;  // all-pairs kernels take this cloud
+
+  const int pos = Lq * kLeaf + lane;
+  const bool valid = pos < Nq;
+  const float4 qp = valid ? a.q.pts[(size_t)b * Nq + pos] : make_float4(0.f, 0.f, 0.f, 0.f);
+  const int qid = valid ? a.q.perm[(size_t)b * Nq + pos] : 0;
+  const float a0 = -2.0f * qp.x, a1 = -2.0f * qp.y, a2 = -2.0f * qp.z, rq = qp.w;
+  const float cmax = sqrtf(cinfo.x);
+  const float S = (sqrtf(rq) + cmax) * (sqrtf(rq) + cmax) * 1.0001f;
+  const float Sw = hg_warp_max_f32(valid ? S : 0.f);
+  const float4 *qbox = a.q.box + (size_t)b * nlq * 2;
+  const float4 *cbox = a.c.box + (size_t)b * nlc * 2;
+  const float4 *cpts = a.c.pts + (size_t)b * Nc;
+  const int *cperm = a.c.perm + (size_t)b * Nc;
+  const float4 qlo = qbox[2 * Lq], qhi = qbox[2 * Lq + 1];
+  const float4 qpt = make_float4(qp.x, qp.y, qp.z, 0.f);
+  float *tf = reinterpret_cast<float *>(tile[warp]);
+
+  auto stage = [&](int L) {
+    const int cpos = L * kLeaf + lane;
+    const float4 c = cpos < Nc ? cpts[cpos] : make_float4(0.f, 0.f, 0.f, CUDART_INF_F);
+    const int cid = cpos < Nc ? cperm[cpos] : 0x7fffffff;
+    __syncwarp();
+    const int pp = lane >> 1, h = lane & 1;
+    tf[8 * pp + h] = c.x;
+    tf[8 * pp + 2 + h] = c.y;
+    tf[8 * pp + 4 + h] = c.z;
+    tf[8 * pp + 6 + h] = c.w;
+    tperm[warp][lane] = cid;
+    __syncwarp();
+  };
+
+  // first leaf: the query's own (self) or the one whose centre is nearest to the query leaf's centre
+  int Ls = Lq;
+  if (!a.self) {
+    float bd = CUDART_INF_F;
+    int bi = 0;
+    const float cx = 0.5f * (qlo.x + qhi.x), cy = 0.5f * (qlo.y + qhi.y), cz = 0.5f * (qlo.z + qhi.z);
+    for (int L = lane; L < nlc; L += 32) {
+      const float4 lo = cbox[2 * L], hi = cbox[2 * L + 1];
+      const float dx = 0.5f * (lo.x + hi.x) - cx, dy = 0.5f * (lo.y + hi.y) - cy, dz = 0.5f * (lo.z + hi.z) - cz;
+      const float d = dx * dx + dy * dy + dz * dz;
+      if (d < bd) {
+        bd = d;
+        bi = L;
+      }
+    }
+    const float wm = hg_warp_min_f32(bd);
+    Ls = __reduce_min_sync(0xffffffffu, bd == wm ? bi : 0x7fffffff);
+    if (Ls == 0x7fffffff) Ls = 0;
+  }
+
+  float best = CUDART_INF_F;  // 1-NN
+  int bid = 0x7fffffff;
+  LexTopK<kNN1 ? 1 : KM> top;
+  float seed = CUDART_INF_F, thr = CUDART_INF_F;
+  if (!kNN1) {
+    if (a.thr0 != nullptr) {
+      seed = valid ? a.thr0[(size_t)b * Nq + qid] : CUDART_INF_F;
+    } else if (KM <= kLeaf) {
+      // seed: the k1-th smallest exact distance over the own leaf (real candidates: an exact upper bound)
+      stage(Ls);
+      top.init();
+      for (int c = 0; c < kLeaf; ++c) {
+        const int pp = c >> 1, h = c & 1;
+        const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
+        float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
+#pragma unroll
+        for (int u = 0; u < (kNN1 ? 1 : KM); ++u) {  // value-only insertion network
+          const float lo = fminf(top.v[u], d);
+          d = fmaxf(top.v[u], d);
+          top.v[u] = lo;
+        }
+      }
+      seed = valid ? nudge_up(top.kth(a.k1)) : CUDART_INF_F;
+    }
+    top.init();
+    thr = seed;
+  }
+  if (!valid) thr = -CUDART_INF_F;  // padding lanes never need a leaf
+
+  int P2 = 1;
+  while (P2 < nlc) P2 <<= 1;
+  unsigned long long visited = 0;
+  for (int d0 = 0; d0 < P2; d0 += 32) {
+    // warp-uniform test of 32 leaves against the largest current threshold of the warp, box against box
+    const float tw = hg_warp_max_f32(thr);
+    const int Lt = Ls ^ (d0 + lane);
+    bool pass = false;
+    if (Lt < nlc) pass = may_hold(box_d2_rd(qlo, qhi, cbox[2 * Lt], cbox[2 * Lt + 1]), tw, Sw);
+    unsigned m = __ballot_sync(0xffffffffu, pass);
+    while (m) {
+      const int bit = __ffs(m) - 1;
+      m &= m - 1u;
+      const int L = Ls ^ (d0 + bit);
+      // re-test against every lane's current threshold, point against box
+      const float4 clo = cbox[2 * L], chi = cbox[2 * L + 1];
+      const bool need = may_hold(box_d2_rd(qpt, qpt, clo, chi), thr, S);
+      if (!__any_sync(0xffffffffu, need)) continue;
+      ++visited;
+      stage(L);
+      if (kNN1) {
+        float mv = CUDART_INF_F;
+#pragma unroll 4
+        for (int pp = 0; pp < kLeaf / 2; ++pp) {
+          const float4 A = tile[warp][2 * pp], Bv = tile[warp][2 * pp + 1];
+          float2 t = __fmul2_rn(make_float2(a0, a0), make_float2(A.x, A.y));
+          t = __ffma2_rn(make_float2(a1, a1), make_float2(A.z, A.w), t);
+          t = __ffma2_rn(make_float2(a2, a2), make_float2(Bv.x, Bv.y), t);
+          const float2 P = __fadd2_rn(__fadd2_rn(make_float2(rq, rq), make_float2(Bv.z, Bv.w)), t);
+          mv = fminf(fminf(mv, P.x), P.y);
+        }
+        if (valid && mv <= best) {  // rare: find the first original index attaining mv in this leaf
+          int id = 0x7fffffff;
+          for (int c = 0; c < kLeaf; ++c) {
+            const int pp = c >> 1, h = c & 1;
+            const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
+            const float v = __fadd_rn(__fadd_rn(rq, cw), __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0))));
+            if (v == mv) id = min(id, tperm[warp][c]);
+          }
+          if (mv < best || id < bid) {
+            best = mv;
+            bid = id;
+          }
+          thr = best;
+        }
+      } else {
+        // folded 4-operation filter (hg_knn3.cu filter_addend / filter_value, FOLD4): sign bit = maybe below thr
+        const float af = __fsub_rd(rq, __fadd_ru(thr, kSlack * (S + thr)));
+        unsigned o = 0u;
+#pragma unroll 4
+        for (int pp = 0; pp < kLeaf / 2; ++pp) {
+          const float4 A = tile[warp][2 * pp], Bv = tile[warp][2 * pp + 1];
+          float2 t = __fadd2_rn(make_float2(Bv.z, Bv.w), make_float2(af, af));
+          t = __ffma2_rn(make_float2(a2, a2), make_float2(Bv.x, Bv.y), t);
+          t = __ffma2_rn(make_float2(a1, a1), make_float2(A.z, A.w), t);
+          t = __ffma2_rn(make_float2(a0, a0), make_float2(A.x, A.y), t);
+          o |= __float_as_uint(t.x) | __float_as_uint(t.y);
+        }
+        const bool hit = valid && (o >> 31) != 0u;
+        if (__any_sync(0xffffffffu, hit) && hit) {  // drain: which candidates, then exact values and insertion
+          unsigned sub = 0u;
+#pragma unroll 4
+          for (int pp = 0; pp < kLeaf / 2; ++pp) {
+            const float4 A = tile[warp][2 * pp], Bv = tile[warp][2 * pp + 1];
+            float2 t = __fadd2_rn(make_float2(Bv.z, Bv.w), make_float2(af, af));
+            t = __ffma2_rn(make_float2(a2, a2), make_float2(Bv.x, Bv.y), t);
+            t = __ffma2_rn(make_float2(a1, a1), make_float2(A.z, A.w), t);
+            t = __ffma2_rn(make_float2(a0, a0), make_float2(A.x, A.y), t);
+            sub |= ((__float_as_uint(t.x) >> 31) << (2 * pp)) | ((__float_as_uint(t.y) >> 31) << (2 * pp + 1));
+          }
+          while (sub) {
+            const int c = __ffs(sub) - 1;
+            sub &= sub - 1u;
+            const int pp = c >> 1, h = c & 1;
+            const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
+            // knn_dist_exact<EXPANDED>: (xx_j + nzz) + xx_i
+            const float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
+            top.push(d, tperm[warp][c]);
+          }
+          thr = fminf(seed, nudge_up(top.kth(a.k1)));
+        }
+      }
+    }
+  }
+  if (a.count != nullptr && lane == 0) {
+    atomicAdd(a.count, visited);
+    atomicAdd(a.count + 1, (unsigned long long)nlc);
+  }
+  if (!valid) return;
+  if (kNN1) {
+    a.vals[(size_t)b * Nq + qid] = best;
+    a.idx[(size_t)b * Nq + qid] = bid == 0x7fffffff ? 0 : bid;
+  } else {
+    const size_t o = ((size_t)b * Nq + qid) * a.k1;
+#pragma unroll
+    for (int s = 0; s < (kNN1 ? 1 : KM); ++s) {
+      if (s < a.k1) {
+        if (a.vals) a.vals[o + s] = top.v[s];
+        a.idx[o + s] = top.id[s];
+        if (a.idx_state) a.idx_state[o + s] = top.id[s];
+      }
+    }
+  }
+}
+
+template <int KM>
+int launch_search(const PruneSearch &a, int B, cudaStream_t stream) {
+  const int nlq = (a.q.N + kLeaf - 1) / kLeaf;
+  dim3 grid((nlq + kSearchWarps - 1) / kSearchWarps, B);
+  prune_search_kernel<KM><<<grid, kSearchWarps * 32, 0, stream>>>(a);
+  HG_CHECK_LAUNCH("prune_search_kernel");
+  return HG_OK;
+}
+
+int g_prune_mode = 1;     // hg_tune("prune", v): 0 = all-pairs kernels only, 1 = automatic
+int g_prune_min_n = 0;    // hg_tune("prune_min_n", n): smallest cloud that takes the pruned path (0 = default)
+int g_prune_count = 0;    // hg_tune("prune_count", 1): count visited leaf pairs (hg_prune_counters)
+
+unsigned long long *counters() {
+  if (!g_prune_count) return nullptr;
+  void *ptr = nullptr;
+  if (cudaGetSymbolAddress(&ptr, g_prune_tiles) != cudaSuccess) return nullptr;
+  return (unsigned long long *)ptr;
+}
+
+}  // namespace
+
+// Default size threshold: see DESIGN 5.1 / 5.2 (sweep with tools/prune_ab.py).
+constexpr int kPruneDefaultMinN = 8192;
+
+int hg_prune_tune(const char *key, int value) {
+  if (!strcmp(key, "prune")) {
+    g_prune_mode = value;
+    return 1;
+  }
+  if (!strcmp(key, "prune_min_n")) {
+    g_prune_min_n = value;
+    return 1;
+  }
+  if (!strcmp(key, "prune_count")) {
+    g_prune_count = value;
+    return 1;
+  }
+  return 0;
+}
+
+bool hg_prune_applies(int N) {
+  const int min_n = g_prune_min_n > 0 ? g_prune_min_n : kPruneDefaultMinN;
+  return g_prune_mode != 0 && N >= min_n && N >= 2 * kLeaf && N <= HG_PRUNE_MAX_N;
+}
+
+size_t hg_prune_order_bytes(int B, int N) {
+  if (B <= 0 || !hg_prune_applies(N)) return 0;
+  const size_t nleaf = (size_t)(N + kLeaf - 1) / kLeaf;
+  return hg_align((size_t)B * N * sizeof(float4)) + hg_align((size_t)B * N * sizeof(int)) +
+         hg_align((size_t)B * nleaf * 2 * sizeof(float4)) + hg_align((size_t)B * sizeof(float4));
+}
+
+int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream) {
+  const size_t nleaf = (size_t)(N + kLeaf - 1) / kLeaf;
+  char *w = (char *)ws;
+  o->N = N;
+  o->pts = (float4 *)w;
+  w += hg_align((size_t)B * N * sizeof(float4));
+  o->perm = (int *)w;
+  w += hg_align((size_t)B * N * sizeof(int));
+  o->box = (float4 *)w;
+  w += hg_align((size_t)B * nleaf * 2 * sizeof(float4));
+  o->info = (float4 *)w;
+  int Np = 2 * kLeaf;
+  while (Np < N) Np <<= 1;
+  const size_t smem = (size_t)Np * sizeof(unsigned);
+  static HgPerDeviceOnce once[2];
+  auto kernel = chamfer_norm ? prune_order_kernel<true> : prune_order_kernel<false>;
+  if (once[chamfer_norm ? 1 : 0].first())
+    HG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 HG_PRUNE_MAX_N * (int)sizeof(unsigned)));
+  kernel<<<B, kBuildThreads, smem, stream>>>(pc, N, Np, *o);
+  HG_CHECK_LAUNCH("prune_order_kernel");
+  return HG_OK;
+}
+
+int hg_prune_nn_search(const HgPruneOrder &q, const HgPruneOrder &c, int B, float *mins, int *args,
+                       cudaStream_t stream) {
+  PruneSearch a;
+  a.q = q;
+  a.c = c;
+  a.self = 0;
+  a.k1 = 1;
+  a.vals = mins;
+  a.idx = args;
+  a.idx_state = nullptr;
+  a.thr0 = nullptr;
+  a.count = counters();
+  return launch_search<1>(a, B, stream);
+}
+
+int hg_prune_knn_search(const HgPruneOrder &o, int B, int k1, const float *thr0, float *vals, int *idx, int *idx_state,
+                        cudaStream_t stream) {
+  PruneSearch a;
+  a.q = o;
+  a.c = o;
+  a.self = 1;
+  a.k1 = k1;
+  a.vals = vals;
+  a.idx = idx;
+  a.idx_state = idx_state;
+  a.thr0 = thr0;
+  a.count = counters();
+  if (a.count) a.count += 2;
+  if (k1 <= 6) return launch_search<6>(a, B, stream);
+  if (k1 <= 20) return launch_search<20>(a, B, stream);
+  if (k1 <= 32) return launch_search<32>(a, B, stream);
+  return launch_search<64>(a, B, stream);
+}
+
+// Visited and total leaf pairs since the last call, {nn, nn total, knn, knn total}; synchronises the device.
+HG_API int hg_prune_counters(unsigned long long *out4) {
+  HG_REQUIRE(out4, HG_E_BADARG, "prune_counters: null pointer");
+  HG_CUDA(cudaDeviceSynchronize());
+  HG_CUDA(cudaMemcpyFromSymbol(out4, g_prune_tiles, sizeof(unsigned long long) * 4));
+  const unsigned long long zero[4] = {0, 0, 0, 0};
+  HG_CUDA(cudaMemcpyToSymbol(g_prune_tiles, zero, sizeof(zero)));
+  return HG_OK;
+}

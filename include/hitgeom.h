@@ -63,6 +63,9 @@ int hg_probe_fp32_peak(float *tflops, float *device_scratch, hgStream stream);
  * (same results; the tests run both); "knn_win" = Z-order window of the small-cloud kNN seeds (0 = default);
  * "fps_threads" = 128 | 256 threads per cloud in furthest point sampling for clouds up to 2048 points (0 = default). */
 int hg_tune(const char *key, int value);
+/* Leaf pairs the pruned passes visited and could have visited since the last call: {Chamfer visited, Chamfer total,
+ * kNN visited, kNN total}, counted while hg_tune("prune_count", 1) is on.  Synchronises the device. */
+int hg_prune_counters(unsigned long long *out4);
 unsigned long long hg_launch_count(void); /* kernels launched by this library since it was loaded */
 void hg_prof_enable(int on);
 int hg_prof_read(int tag, float *total_ms, int *launches);
