@@ -218,7 +218,10 @@ struct HgPruneOrder {
 int hg_prune_tune(const char *key, int value);  // 1 if the key is one of the pruned path's
 bool hg_prune_applies(int N);               // the size threshold and hg_tune("prune") as they stand
 size_t hg_prune_order_bytes(int B, int N);  // 0 when the path does not apply to N
-int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream);
+// state (null, or an ordering state of hg_order_state_bytes(B, N) bytes): refit the state's permutation and rebuild only
+// the clouds whose refit fails (hg_prune.cu); o->perm then points into the state
+int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream,
+                   void *state = nullptr);
 int hg_prune_nn_search(const HgPruneOrder &q, const HgPruneOrder &c, int B, float *mins, int *args, cudaStream_t stream);
 int hg_prune_knn_search(const HgPruneOrder &o, int B, int k1, const float *thr0, float *vals, int *idx, int *idx_state,
                         cudaStream_t stream);
@@ -232,4 +235,5 @@ int hg_knn3_launch_i64(int form, const float *q, const float *r, int B, int Nq, 
                        long long *idx, cudaStream_t stream);
 size_t hg_knn3_seed_workspace_bytes(int B, int N);
 int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, void *workspace,
-                            size_t workspace_bytes, cudaStream_t stream, int *idx_state = nullptr, int state_valid = 0);
+                            size_t workspace_bytes, cudaStream_t stream, int *idx_state = nullptr, int state_valid = 0,
+                            void *order = nullptr);

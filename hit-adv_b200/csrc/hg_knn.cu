@@ -570,8 +570,17 @@ HG_API int hg_knn_self_f32(const float *pc, int B, int K, int C, int k1, float *
 HG_API int hg_knn_self_temporal_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, int *idx_state,
                                     int state_valid, void *workspace, size_t workspace_bytes, hgStream stream_) {
   HG_NVTX_RANGE("hg_knn_self_temporal_f32");
+  return hg_knn_self_temporal_order_f32(pc, B, K, C, k1, vals, idx, idx_state, state_valid, nullptr, workspace,
+                                        workspace_bytes, stream_);
+}
+
+HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx,
+                                          int *idx_state, int state_valid, void *order, void *workspace,
+                                          size_t workspace_bytes, hgStream stream_) {
+  HG_NVTX_RANGE("hg_knn_self_temporal_order_f32");
   cudaStream_t stream = hg_stream(stream_);
   HG_REQUIRE(pc && idx, HG_E_BADARG, "knn_self: null pointer");
+  HG_REQUIRE(((uintptr_t)order & 15) == 0, HG_E_BADARG, "knn_self: the ordering state must be 16-byte aligned");
   HG_REQUIRE(B > 0 && K > 0 && C > 0, HG_E_BADARG, "knn_self: sizes must be positive");
   HG_REQUIRE(k1 >= 1 && k1 <= (C == 3 ? 64 : 32) && k1 <= K, HG_E_BADARG,
              "knn_self: need 1 <= k <= min(%d, K); got k=%d K=%d", C == 3 ? 64 : 32, k1, K);
@@ -583,7 +592,8 @@ HG_API int hg_knn_self_temporal_f32(const float *pc, int B, int K, int C, int k1
     const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, K);
     const size_t pad_ws = hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
     if (hg_prune_applies(K))  // large clouds: pruned search, whatever the list length
-      return hg_knn3_self_seeded_i32(pc, B, K, k1, vals, idx, workspace, workspace_bytes, stream, idx_state, state_valid);
+      return hg_knn3_self_seeded_i32(pc, B, K, k1, vals, idx, workspace, workspace_bytes, stream, idx_state, state_valid,
+                                     order);
     if (!idx_state && knn3_pad_candidate(K, k1) && g_hg_tune_knn_tc_off != 1 && workspace &&
         workspace_bytes >= seed_ws + pad_ws &&
         ((4LL * B * ((K + 127) / 128) >= hg_sm_count() && (long long)B * ((K + 127) / 128) <= 8LL * hg_sm_count()) ||

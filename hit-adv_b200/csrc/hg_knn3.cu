@@ -1058,8 +1058,9 @@ HG_API void hg_knn_tune_small(int small_max_n) { g_small_max_n = small_max_n; }
 // self-kNN (expanded form) with seeded thresholds; falls back to the unseeded launch when there is no workspace.
 // idx_state (optional, [B,N,k1]): the neighbour indices of the previous call on a nearby cloud -- read as temporal
 // seeds when state_valid, and overwritten with this call's indices (a second copy of idx).
+// order (optional): an ordering state for the pruned path (hg_order_state_bytes), refit instead of rebuilt.
 int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, void *workspace,
-                            size_t workspace_bytes, cudaStream_t stream, int *idx_state, int state_valid) {
+                            size_t workspace_bytes, cudaStream_t stream, int *idx_state, int state_valid, void *order) {
   const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, N);
   if (hg_prune_applies(N) && workspace != nullptr && workspace_bytes >= seed_ws + hg_prune_order_bytes(B, N)) {
     // large clouds: kd-tree ordering and pruned search (hg_prune.cu), seeded from each query's own leaf or, with
@@ -1068,14 +1069,14 @@ int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, 
     float *sb = (float *)((char *)workspace + hg_align((size_t)B * N * sizeof(int)));
     float *thr = (float *)((char *)sb + hg_align((size_t)B * 8 * sizeof(float)));
     const float *thr0 = nullptr;
-    if (idx_state && state_valid) {
+    if (idx_state && state_valid && k1 <= 32) {  // (the seed kernel bounds at most 32 previous neighbours)
       int rc = launch_seed_prev(pc, B, N, k1, idx_state, thr, sb, stream);
       if (rc) return rc;
       thr0 = thr;
     }
     HgPruneOrder o;
     const bool prof = hg_prof_begin(HG_PROF_KNN, stream);
-    int rc = hg_prune_build(pc, B, N, false, (char *)workspace + seed_ws, &o, stream);
+    int rc = hg_prune_build(pc, B, N, false, (char *)workspace + seed_ws, &o, stream, order);
     if (!rc) rc = hg_prune_knn_search(o, B, k1, thr0, vals, idx, idx_state, stream);
     hg_prof_end(HG_PROF_KNN, stream, prof);
     if (rc) return rc;

@@ -983,8 +983,20 @@ HG_API size_t hg_nn_bidir_workspace_bytes(int B, int N2, int N1, int D) {
 HG_API int hg_nn_bidir_f32(const float *gts, const float *preds, int B, int N2, int N1, int D, float *min1, int *arg1,
                            float *min2, int *arg2, void *workspace, size_t workspace_bytes, hgStream stream_) {
   HG_NVTX_RANGE("hg_nn_bidir_f32");
+  return hg_nn_bidir_temporal_f32(gts, preds, B, N2, N1, D, min1, arg1, min2, arg2, nullptr, nullptr, workspace,
+                                  workspace_bytes, stream_);
+}
+
+HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B, int N2, int N1, int D, float *min1,
+                                    int *arg1, float *min2, int *arg2, void *gts_order, void *preds_order,
+                                    void *workspace, size_t workspace_bytes, hgStream stream_) {
+  HG_NVTX_RANGE("hg_nn_bidir_temporal_f32");
   cudaStream_t stream = hg_stream(stream_);
   HG_REQUIRE(gts && preds && min1 && arg1 && min2 && arg2, HG_E_BADARG, "nn_bidir: null pointer");
+  HG_REQUIRE(((uintptr_t)gts_order & 15) == 0 && ((uintptr_t)preds_order & 15) == 0, HG_E_BADARG,
+             "nn_bidir: ordering states must be 16-byte aligned");
+  HG_REQUIRE(gts_order == nullptr || gts_order != preds_order, HG_E_BADARG,
+             "nn_bidir: gts and preds need ordering states of their own");
   HG_REQUIRE(B > 0 && N1 > 0 && N2 > 0 && D > 0, HG_E_BADARG, "nn_bidir: sizes must be positive (B=%d N2=%d N1=%d D=%d)",
              B, N2, N1, D);
   HG_REQUIRE(B <= 65535, HG_E_UNSUPPORTED, "nn_bidir: B=%d > 65535 clouds per call", B);
@@ -1030,8 +1042,8 @@ HG_API int hg_nn_bidir_f32(const float *gts, const float *preds, int B, int N2, 
     char *ow = (char *)workspace + nn_d3_bytes(B, N2, N1);
     HgPruneOrder og, op;
     const bool prof = hg_prof_begin(HG_PROF_NN_BIDIR, stream);
-    int rc = hg_prune_build(gts, B, N2, true, ow, &og, stream);
-    if (!rc) rc = hg_prune_build(preds, B, N1, true, ow + hg_prune_order_bytes(B, N2), &op, stream);
+    int rc = hg_prune_build(gts, B, N2, true, ow, &og, stream, gts_order);
+    if (!rc) rc = hg_prune_build(preds, B, N1, true, ow + hg_prune_order_bytes(B, N2), &op, stream, preds_order);
     if (!rc) rc = hg_prune_nn_search(op, og, B, min1, arg1, stream);  // column j (preds): nearest row (gts)
     if (!rc) rc = hg_prune_nn_search(og, op, B, min2, arg2, stream);  // row i (gts): nearest column (preds)
     hg_prof_end(HG_PROF_NN_BIDIR, stream, prof);

@@ -47,19 +47,58 @@ __device__ __forceinline__ float box_d2_rd(float4 alo, float4 ahi, float4 blo, f
 }
 __device__ __forceinline__ bool may_hold(float lb, float thr, float S) { return !(lb > thr + kSlack * (S + thr)); }
 
+__device__ unsigned long long g_order_counts[3];  // orderings: refit and kept, rebuilt from a state, built without one
+
+// Leaf L's box from the warp's 32 points (v, real when `in`), written to o.box; returns h + the leaf's
+// (ext_x + ext_y + ext_z), accumulated on lane 0.  The build and the refit both go through here, so H_built and the
+// refit's H are the same bits for the same permutation and points.
+__device__ __forceinline__ float leaf_box(const HgPruneOrder &o, int b, int nleaf, int L, int lane, bool in,
+                                          const float (&v)[3], float h) {
+  float lo[3], hi[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    lo[c] = hg_warp_min_f32(in ? v[c] : CUDART_INF_F);
+    hi[c] = hg_warp_max_f32(in ? v[c] : -CUDART_INF_F);
+  }
+  if (lane == 0) {
+    o.box[((size_t)b * nleaf + L) * 2] = make_float4(lo[0], lo[1], lo[2], 0.f);
+    o.box[((size_t)b * nleaf + L) * 2 + 1] = make_float4(hi[0], hi[1], hi[2], 0.f);
+    h += ((hi[0] - lo[0]) + (hi[1] - lo[1])) + (hi[2] - lo[2]);
+  }
+  return h;
+}
+// sum of the per-warp leaf sums (lane 0 of every warp) in warp order; the result is valid on thread 0
+__device__ __forceinline__ float block_sum_leaves(float h, float *s_h) {
+  const int tid = threadIdx.x;
+  if ((tid & 31) == 0) s_h[tid >> 5] = h;
+  __syncthreads();
+  float H = 0.f;
+  if (tid == 0)
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) H += s_h[w];
+  return H;
+}
+
 // ---- ordering build: one CTA per cloud, kd splits (median of the longest axis) by a segmented bitonic sort ----------
 // key[i] = (quantised coordinate on the segment's split axis) << 14 | point index; padding to a power of two carries
 // kPadKey and stays at the end of the array at every level.  Correctness never depends on the quality of a split:
 // the leaf boxes are recomputed from the points.
+//
+// With an ordering state (hdr != null: o.perm points into the state, hdr is its per-cloud header) the kernel runs after
+// prune_refit_kernel and rebuilds only the clouds the refit marked (info.z != 0); it then also stores the leaf-box
+// quality H of the new permutation in the header.  count (null, or g_order_counts): clouds ordered without a state.
 template <bool CHAMFER_NORM>
 __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float *__restrict__ pc, int N, int Np,
-                                                                    HgPruneOrder o) {
+                                                                    HgPruneOrder o, float4 *hdr,
+                                                                    unsigned long long *count) {
   extern __shared__ unsigned key[];  // [Np]
   __shared__ unsigned smin[3][kMaxSegs], smax[3][kMaxSegs];
   __shared__ float slo[kMaxSegs], sscale[kMaxSegs];
   __shared__ int saxis[kMaxSegs];
   __shared__ unsigned s_bad, s_norm;
+  __shared__ float s_h[kBuildThreads / 32];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  if (hdr != nullptr && o.info[b].z == 0.f) return;  // the refit kept this cloud's ordering
+  if (count != nullptr && hdr == nullptr && tid == 0) atomicAdd(count + 2, 1ull);
   const float *p = pc + (size_t)b * N * 3;
   if (tid == 0) {
     s_bad = 0u;
@@ -161,6 +200,7 @@ __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float 
     o.perm[(size_t)b * N + i] = id;
   }
   const int nleaf = (N + kLeaf - 1) / kLeaf;
+  float h = 0.f;
   for (int L = tid >> 5; L < nleaf; L += kBuildThreads / 32) {
     const int i = L * kLeaf + lane;
     float v[3] = {0.f, 0.f, 0.f};
@@ -169,16 +209,96 @@ __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float 
 #pragma unroll
       for (int c = 0; c < 3; ++c) v[c] = p[(size_t)id * 3 + c];
     }
-    float lo[3], hi[3];
+    h = leaf_box(o, b, nleaf, L, lane, i < N, v, h);
+  }
+  if (hdr != nullptr) {
+    const float H = block_sum_leaves(h, s_h);
+    if (tid == 0) hdr[b] = make_float4(H, 0.f, 0.f, 0.f);
+  }
+}
+
+// ---- ordering state: refit of the previous call's permutation ---------------------------------------------------------
+// One CTA per cloud.  Validates the state's permutation (every entry in [0, N), each index once: a bitmap in shared
+// memory), recomputes the per-cloud info exactly as the build does (the max and the any-non-finite test do not depend
+// on the order), gathers the points through the permutation (pts in the form's norm arithmetic and leaf boxes, bit for
+// bit what prune_order_kernel writes for the same permutation) and measures H = sum over leaves of the box's
+// (ext_x + ext_y + ext_z).  The cloud is marked for the rebuild (info.z = 1) when the permutation is invalid or
+// !(H <= (1 + tol) H_built): a NaN or garbage header fails the comparison too.  STAGE: the cloud is staged in shared
+// memory (12 B per point) for the gather instead of being read again from global memory (L2).
+template <bool CHAMFER_NORM, bool STAGE>
+__global__ void __launch_bounds__(kBuildThreads) prune_refit_kernel(const float *__restrict__ pc, int N, HgPruneOrder o,
+                                                                    const float4 *__restrict__ hdr, float tol,
+                                                                    unsigned long long *count) {
+  extern __shared__ float spts[];  // STAGE: [N * 3]
+  __shared__ unsigned bits[HG_PRUNE_MAX_N / 32];
+  __shared__ unsigned s_bad, s_norm, s_invalid;
+  __shared__ float s_h[kBuildThreads / 32];
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  const float *p = pc + (size_t)b * N * 3;
+  const int *perm = o.perm + (size_t)b * N;
+  for (int t = tid; t < (N + 31) / 32; t += kBuildThreads) bits[t] = 0u;
+  if (tid == 0) {
+    s_bad = 0u;
+    s_norm = 0u;
+    s_invalid = 0u;
+  }
+  __syncthreads();
+  float mn = 0.f;
+  bool bad = false, invalid = false;
+  for (int i = tid; i < N; i += kBuildThreads) {
+    const float x = p[(size_t)i * 3], y = p[(size_t)i * 3 + 1], z = p[(size_t)i * 3 + 2];
+    bad |= !(isfinite(x) && isfinite(y) && isfinite(z));
+    mn = fmaxf(mn, fmaf(z, z, fmaf(y, y, x * x)));
+    if (STAGE) {
+      spts[i * 3] = x;
+      spts[i * 3 + 1] = y;
+      spts[i * 3 + 2] = z;
+    }
+    const int id = perm[i];
+    if ((unsigned)id >= (unsigned)N) {
+      invalid = true;
+    } else {
+      const unsigned bit = 1u << (id & 31);
+      invalid |= (atomicOr(&bits[id >> 5], bit) & bit) != 0u;  // N entries in range, none twice: a permutation
+    }
+  }
+  mn = hg_warp_max_f32(mn);
+  bad = __any_sync(0xffffffffu, bad);
+  invalid = __any_sync(0xffffffffu, invalid);
+  if (lane == 0) {
+    atomicMax(&s_norm, __float_as_uint(mn));
+    if (bad) s_bad = 1u;
+    if (invalid) s_invalid = 1u;
+  }
+  __syncthreads();
+  const float norm = __uint_as_float(s_norm);
+  const bool flagged = s_bad != 0u || !(norm < 1e36f);
+  if (flagged || s_invalid != 0u) {  // flagged: the all-pairs kernels take the cloud, nothing else to write
+    if (tid == 0) {
+      o.info[b] = make_float4(norm * 1.0001f, flagged ? 1.f : 0.f, flagged ? 0.f : 1.f, 0.f);
+      if (count != nullptr) atomicAdd(count + (flagged ? 0 : 1), 1ull);
+    }
+    return;
+  }
+  const int nleaf = (N + kLeaf - 1) / kLeaf;
+  float h = 0.f;
+  for (int L = tid >> 5; L < nleaf; L += kBuildThreads / 32) {  // the build's thread-to-point map, one pass
+    const int i = L * kLeaf + lane;
+    float v[3] = {0.f, 0.f, 0.f};
+    if (i < N) {
+      const int id = perm[i];
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      lo[c] = hg_warp_min_f32(i < N ? v[c] : CUDART_INF_F);
-      hi[c] = hg_warp_max_f32(i < N ? v[c] : -CUDART_INF_F);
+      for (int c = 0; c < 3; ++c) v[c] = STAGE ? spts[id * 3 + c] : p[(size_t)id * 3 + c];
+      const float w = CHAMFER_NORM ? hg_dot3_fma(v[0], v[1], v[2], v[0], v[1], v[2]) : hg_sumsq3_seq(v[0], v[1], v[2]);
+      o.pts[(size_t)b * N + i] = make_float4(v[0], v[1], v[2], w);
     }
-    if (lane == 0) {
-      o.box[((size_t)b * nleaf + L) * 2] = make_float4(lo[0], lo[1], lo[2], 0.f);
-      o.box[((size_t)b * nleaf + L) * 2 + 1] = make_float4(hi[0], hi[1], hi[2], 0.f);
-    }
+    h = leaf_box(o, b, nleaf, L, lane, i < N, v, h);
+  }
+  const float H = block_sum_leaves(h, s_h);
+  if (tid == 0) {
+    const bool rebuild = !(H <= (1.f + tol) * hdr[b].x);
+    o.info[b] = make_float4(norm * 1.0001f, 0.f, rebuild ? 1.f : 0.f, 0.f);
+    if (count != nullptr) atomicAdd(count + (rebuild ? 1 : 0), 1ull);
   }
 }
 
@@ -442,7 +562,9 @@ int launch_search(const PruneSearch &a, int B, cudaStream_t stream) {
 
 int g_prune_mode = 1;     // hg_tune("prune", v): 0 = all-pairs kernels only, 1 = automatic
 int g_prune_min_n = 0;    // hg_tune("prune_min_n", n): smallest cloud that takes the pruned path (0 = default)
-int g_prune_count = 0;    // hg_tune("prune_count", 1): count visited leaf pairs (hg_prune_counters)
+int g_prune_count = 0;    // hg_tune("prune_count", 1): count visited leaf pairs and orderings (hg_prune_*counters)
+int g_refit_tol = 0;      // hg_tune("prune_refit_tol", permille): rebuild threshold of the refit (0 = default)
+int g_refit_stage = 0;    // hg_tune("prune_refit_stage", v): 0 = default, 1 = stage the cloud in shared memory, 2 = not
 
 unsigned long long *counters() {
   if (!g_prune_count) return nullptr;
@@ -450,11 +572,25 @@ unsigned long long *counters() {
   if (cudaGetSymbolAddress(&ptr, g_prune_tiles) != cudaSuccess) return nullptr;
   return (unsigned long long *)ptr;
 }
+unsigned long long *order_counters() {
+  if (!g_prune_count) return nullptr;
+  void *ptr = nullptr;
+  if (cudaGetSymbolAddress(&ptr, g_order_counts) != cudaSuccess) return nullptr;
+  return (unsigned long long *)ptr;
+}
+
+// the state's header (one float4 per cloud) follows the permutations
+float4 *state_header(void *state, int B, int N) {
+  return (float4 *)((char *)state + hg_align((size_t)B * N * sizeof(int)));
+}
 
 }  // namespace
 
 // Default size threshold: see DESIGN 5.1 / 5.2 (sweep with tools/prune_ab.py).
 constexpr int kPruneDefaultMinN = 8192;
+// Default refit tolerance tau [permille] and gather source: see DESIGN 5.5 (sweep with tools/order_state_ab.py).
+constexpr int kRefitDefaultTolPermille = 100;
+constexpr bool kRefitDefaultStage = true;
 
 int hg_prune_tune(const char *key, int value) {
   if (!strcmp(key, "prune")) {
@@ -467,6 +603,14 @@ int hg_prune_tune(const char *key, int value) {
   }
   if (!strcmp(key, "prune_count")) {
     g_prune_count = value;
+    return 1;
+  }
+  if (!strcmp(key, "prune_refit_tol")) {
+    g_refit_tol = value;
+    return 1;
+  }
+  if (!strcmp(key, "prune_refit_stage")) {
+    g_refit_stage = value;
     return 1;
   }
   return 0;
@@ -484,26 +628,50 @@ size_t hg_prune_order_bytes(int B, int N) {
          hg_align((size_t)B * nleaf * 2 * sizeof(float4)) + hg_align((size_t)B * sizeof(float4));
 }
 
-int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream) {
+HG_API size_t hg_order_state_bytes(int B, int N) {
+  if (B <= 0 || N <= 0) return 0;
+  return hg_align((size_t)B * N * sizeof(int)) + hg_align((size_t)B * sizeof(float4));
+}
+
+int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream,
+                   void *state) {
   const size_t nleaf = (size_t)(N + kLeaf - 1) / kLeaf;
   char *w = (char *)ws;
   o->N = N;
   o->pts = (float4 *)w;
   w += hg_align((size_t)B * N * sizeof(float4));
-  o->perm = (int *)w;
+  o->perm = state ? (int *)state : (int *)w;  // with a state, the permutation lives there (the workspace slot is unused)
   w += hg_align((size_t)B * N * sizeof(int));
   o->box = (float4 *)w;
   w += hg_align((size_t)B * nleaf * 2 * sizeof(float4));
   o->info = (float4 *)w;
   int Np = 2 * kLeaf;
   while (Np < N) Np <<= 1;
+  float4 *hdr = state ? state_header(state, B, N) : nullptr;
+  if (state) {
+    const bool stage = g_refit_stage == 0 ? kRefitDefaultStage : g_refit_stage == 1;
+    const float tol = (g_refit_tol > 0 ? g_refit_tol : kRefitDefaultTolPermille) * 1e-3f;
+    const size_t rsmem = stage ? (size_t)N * 3 * sizeof(float) : 0;
+    static HgPerDeviceOnce ronce[2];
+    auto refit = chamfer_norm ? (stage ? prune_refit_kernel<true, true> : prune_refit_kernel<true, false>)
+                              : (stage ? prune_refit_kernel<false, true> : prune_refit_kernel<false, false>);
+    if (stage && ronce[chamfer_norm ? 1 : 0].first()) {
+      HG_CUDA(cudaFuncSetAttribute(prune_refit_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   HG_PRUNE_MAX_N * 3 * (int)sizeof(float)));
+      HG_CUDA(cudaFuncSetAttribute(prune_refit_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   HG_PRUNE_MAX_N * 3 * (int)sizeof(float)));
+    }
+    refit<<<B, kBuildThreads, rsmem, stream>>>(pc, N, *o, hdr, tol, order_counters());
+    HG_CHECK_LAUNCH("prune_refit_kernel");
+  }
   const size_t smem = (size_t)Np * sizeof(unsigned);
   static HgPerDeviceOnce once[2];
   auto kernel = chamfer_norm ? prune_order_kernel<true> : prune_order_kernel<false>;
   if (once[chamfer_norm ? 1 : 0].first())
     HG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  HG_PRUNE_MAX_N * (int)sizeof(unsigned)));
-  kernel<<<B, kBuildThreads, smem, stream>>>(pc, N, Np, *o);
+  // with a state: the clouds the refit marked only (the others exit at entry), so no host decision is needed
+  kernel<<<B, kBuildThreads, smem, stream>>>(pc, N, Np, *o, hdr, order_counters());
   HG_CHECK_LAUNCH("prune_order_kernel");
   return HG_OK;
 }
@@ -549,5 +717,16 @@ HG_API int hg_prune_counters(unsigned long long *out4) {
   HG_CUDA(cudaMemcpyFromSymbol(out4, g_prune_tiles, sizeof(unsigned long long) * 4));
   const unsigned long long zero[4] = {0, 0, 0, 0};
   HG_CUDA(cudaMemcpyToSymbol(g_prune_tiles, zero, sizeof(zero)));
+  return HG_OK;
+}
+
+// Orderings since the last call, {refit and kept, rebuilt from a state, built without a state}, counted per cloud while
+// hg_tune("prune_count", 1) is on; synchronises the device.
+HG_API int hg_prune_order_counters(unsigned long long *out3) {
+  HG_REQUIRE(out3, HG_E_BADARG, "prune_order_counters: null pointer");
+  HG_CUDA(cudaDeviceSynchronize());
+  HG_CUDA(cudaMemcpyFromSymbol(out3, g_order_counts, sizeof(unsigned long long) * 3));
+  const unsigned long long zero[3] = {0, 0, 0};
+  HG_CUDA(cudaMemcpyToSymbol(g_order_counts, zero, sizeof(zero)));
   return HG_OK;
 }

@@ -24,12 +24,15 @@ _SIGNATURES = {
                            ctypes.POINTER(ctypes.c_longlong)]),
     "hg_nn_bidir_workspace_bytes": (Z, [I, I, I, I]),
     "hg_nn_bidir_f32": (I, [P, P, I, I, I, I, P, P, P, P, P, Z, P]),
+    "hg_order_state_bytes": (Z, [I, I]),
+    "hg_nn_bidir_temporal_f32": (I, [P, P, I, I, I, I, P, P, P, P, P, P, P, Z, P]),
     "hg_nn_bidir_tune": (None, [I, I]),
     "hg_knn_tune": (None, [I, I]),
     "hg_knn_force_shape": (None, [I, I]),
     "hg_knn_tune_small": (None, [I]),
     "hg_tune": (I, [ctypes.c_char_p, I]),
     "hg_prune_counters": (I, [ctypes.POINTER(ctypes.c_ulonglong)]),
+    "hg_prune_order_counters": (I, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "hg_launch_count": (ctypes.c_ulonglong, []),
     "hg_prof_enable": (None, [I]),
     "hg_prof_read": (I, [I, ctypes.POINTER(F), ctypes.POINTER(I)]),
@@ -40,6 +43,7 @@ _SIGNATURES = {
     "hg_knn_self_workspace_bytes": (Z, [I, I, I, I]),
     "hg_knn_self_f32": (I, [P, I, I, I, I, P, P, P, Z, P]),
     "hg_knn_self_temporal_f32": (I, [P, I, I, I, I, P, P, P, I, P, Z, P]),
+    "hg_knn_self_temporal_order_f32": (I, [P, I, I, I, I, P, P, P, I, P, P, Z, P]),
     "hg_knn_outlier_fwd_f32": (I, [P, I, I, I, F, P, P, P, P, P]),
     "hg_knn_outlier_bwd_workspace_bytes": (Z, [I, I, I]),
     "hg_knn_outlier_bwd_f32": (I, [P, P, P, P, I, I, I, I, P, P, Z, P]),

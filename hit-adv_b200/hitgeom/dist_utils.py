@@ -41,6 +41,38 @@ class L2Dist(nn.Module):
         return _finish(dist, weights, batch_avg)
 
 
+def _order(store, role, t):
+    """The ordering state of cloud `t` [B,N,3] in role 'ori' / 'adv' (one per shape and device), allocated on first use
+    (zero-filled: the first call builds).  None where the ordering does not apply (not a 3-D CUDA cloud)."""
+    if not (t.is_cuda and t.dim() == 3 and t.shape[2] == 3):
+        return None
+    key = (role, tuple(t.shape), t.device)
+    s = store.get(key)
+    if s is None:
+        s = store[key] = F.order_state(t.shape[0], t.shape[1], t.device)
+    return s
+
+
+class _TemporalOrders:
+    """`temporal_seeds(True)` for the set distances (an addition): keep the kd-tree ordering of `adv` and `ori` between
+    calls, so that clouds of 8192..16384 points refit the previous call's ordering instead of rebuilding it
+    (hg_nn_bidir_temporal_f32).  Meant for attack loops, where `ori` stays put and `adv` moves by a learning-rate step
+    per call; the loss and its gradient are the same bits either way.  The states are per (role, batch shape, device) and
+    belong to this module: a module must not run on two streams at once.  [B,3,K] inputs (HiT-ADV's channel-first call)
+    are not 3-D point clouds and take no state."""
+
+    def temporal_seeds(self, on=True):
+        self.temporal = bool(on)
+        self._orders = {}
+        return self
+
+    def _losses(self, fn, adv_pc, ori_pc):
+        po, go = _order(self._orders, "adv", adv_pc), _order(self._orders, "ori", ori_pc)
+        if po is not None and go is not None:
+            return fn(adv_pc, ori_pc, po, go)
+        return fn(adv_pc, ori_pc)
+
+
 def _select(loss1, loss2, method):
     if method == 'adv2ori':
         return loss1
@@ -49,26 +81,38 @@ def _select(loss1, loss2, method):
     return (loss1 + loss2) / 2.
 
 
-class ChamferDist(nn.Module):
+class ChamferDist(_TemporalOrders, nn.Module):
+    """Same constructor as the reference; `temporal_seeds(True)`: see _TemporalOrders."""
+
     def __init__(self, method='adv2ori'):
         super(ChamferDist, self).__init__()
         self.method = method
 
     def forward(self, adv_pc, ori_pc, weights=None, batch_avg=True):
         B = adv_pc.shape[0]
-        loss1, loss2 = chamfer(adv_pc, ori_pc)  # [B], adv2ori, ori2adv
+        # (getattr: install.patch_reference() binds this forward to the REFERENCE's class, which has no temporal state)
+        if getattr(self, "temporal", False):
+            loss1, loss2 = self._losses(F.chamfer_losses, adv_pc, ori_pc)
+        else:
+            loss1, loss2 = chamfer(adv_pc, ori_pc)  # [B], adv2ori, ori2adv
         loss = _select(loss1, loss2, self.method)
         return _finish(loss, _weights(weights, B, loss.device), batch_avg)
 
 
-class HausdorffDist(nn.Module):
+class HausdorffDist(_TemporalOrders, nn.Module):
+    """Same constructor as the reference; `temporal_seeds(True)`: see _TemporalOrders."""
+
     def __init__(self, method='adv2ori'):
         super(HausdorffDist, self).__init__()
         self.method = method
 
     def forward(self, adv_pc, ori_pc, weights=None, batch_avg=True):
         B = adv_pc.shape[0]
-        loss1, loss2 = hausdorff(adv_pc, ori_pc)
+        # (getattr: install.patch_reference() binds this forward to the REFERENCE's class, which has no temporal state)
+        if getattr(self, "temporal", False):
+            loss1, loss2 = self._losses(F.hausdorff_losses, adv_pc, ori_pc)
+        else:
+            loss1, loss2 = hausdorff(adv_pc, ori_pc)
         loss = _select(loss1, loss2, self.method)
         return _finish(loss, _weights(weights, B, loss.device), batch_avg)
 
@@ -77,8 +121,9 @@ class KNNDist(nn.Module):
     """Same constructor as the reference.  `temporal_seeds(True)` (an addition) keeps the neighbour indices of the
     previous call as state and hands them to the next call as seeds: inside an attack loop (CW/kNN.py:77-111) the cloud
     moves by a learning-rate step per iteration, so they bound every k-th distance almost tightly and replace the
-    spatial pre-pass.  The loss and its gradient are the same bits either way; the state is per (batch shape, device)
-    and replay-safe (the kernel updates it in place)."""
+    spatial pre-pass.  Clouds of 8192..16384 points also keep their kd-tree ordering state (hg_knn_self_temporal_order_f32,
+    see _TemporalOrders).  The loss and its gradient are the same bits either way; the states are per (batch shape,
+    device) and replay-safe (the kernels update them in place)."""
 
     def __init__(self, k=5, alpha=1.05):
         super(KNNDist, self).__init__()
@@ -86,10 +131,12 @@ class KNNDist(nn.Module):
         self.alpha = alpha
         self.temporal = False
         self._state = {}
+        self._orders = {}
 
     def temporal_seeds(self, on=True):
         self.temporal = bool(on)
         self._state.clear()
+        self._orders = {}
         return self
 
     def forward(self, pc, weights=None, batch_avg=True):
@@ -97,7 +144,7 @@ class KNNDist(nn.Module):
         B = pc.shape[0]
         if pc.shape[1] == 3:
             pc = pc.transpose(2, 1)  # kernels are point-major
-        state, valid = None, False
+        state, valid, order = None, False, None
         # (getattr: install.patch_reference() binds this forward to the REFERENCE's KNNDist class, whose __init__ knows
         # nothing of the temporal state)
         if getattr(self, "temporal", False) and pc.is_cuda and pc.shape[2] == 3:
@@ -106,7 +153,8 @@ class KNNDist(nn.Module):
             if not valid:
                 self._state[key] = torch.empty((pc.shape[0], pc.shape[1], self.k + 1), dtype=torch.int32, device=pc.device)
             state = self._state[key]
-        loss = F.knn_outlier_loss(pc, self.k, self.alpha, state, valid)  # [B]
+            order = _order(self._orders, "adv", pc)
+        loss = F.knn_outlier_loss(pc, self.k, self.alpha, state, valid, order)  # [B]
         return _finish(loss, _weights(weights, B, loss.device), batch_avg)
 
 
@@ -119,8 +167,12 @@ class ChamferkNNDist(nn.Module):
         self.w2 = knn_weight
 
     def temporal_seeds(self, on=True):
-        """See KNNDist.temporal_seeds."""
+        """Both terms: see KNNDist.temporal_seeds and ChamferDist.temporal_seeds.  The two terms share one ordering
+        state of `adv`: forward runs them one after the other on the current stream, so the kNN term refits the
+        ordering the Chamfer term has just refit or rebuilt."""
+        self.chamfer_dist.temporal_seeds(on)
         self.knn_dist.temporal_seeds(on)
+        self.knn_dist._orders = self.chamfer_dist._orders
         return self
 
     def forward(self, adv_pc, ori_pc, weights=None, batch_avg=True):

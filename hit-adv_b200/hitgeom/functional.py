@@ -2,6 +2,8 @@
 and the `torch.autograd.Function`s whose backward reuses the saved nearest-neighbour indices.
 
 No arithmetic on point data happens in Python/PyTorch here; torch only allocates outputs and workspaces."""
+import ctypes
+
 import torch
 
 from . import _lib
@@ -32,11 +34,28 @@ def _on_tensor_device(fn):
 # ------------------------------------------------------------------------------------------------------------
 # set distance (util/set_distance.py)
 # ------------------------------------------------------------------------------------------------------------
+def order_state(B, N, device):
+    """A kd-tree ordering state for a batch of B clouds of N points (hg_order_state_bytes): uint8, zero-filled, so the
+    first call that uses it builds.  Hand it to `nn_bidir` / `knn_self` for the same cloud on later calls, which then
+    refit the stored ordering instead of rebuilding it; the results do not depend on its contents."""
+    return torch.zeros(max(int(lib().hg_order_state_bytes(int(B), int(N))), 16), dtype=torch.uint8, device=device)
+
+
+def _check_order(order, B, N, dev, name):
+    if order is None:
+        return
+    require(order, name, dtype=torch.uint8)
+    if order.device != dev or order.numel() < lib().hg_order_state_bytes(B, N):
+        raise RuntimeError(f"{name} must be an order_state({B}, {N}) tensor on {dev}")
+
+
 @_on_tensor_device
-def nn_bidir(gts, preds):
+def nn_bidir(gts, preds, gts_order=None, preds_order=None):
     """Fused `batch_pairwise_dist(gts, preds)` + `torch.min(P,1)` + `torch.min(P,2)` (set_distance.py:15-48).
 
-    gts [B,N2,D], preds [B,N1,D] -> (min1 [B,N1], arg1 [B,N1] int32, min2 [B,N2], arg2 [B,N2] int32)."""
+    gts [B,N2,D], preds [B,N1,D] -> (min1 [B,N1], arg1 [B,N1] int32, min2 [B,N2], arg2 [B,N2] int32).
+    `gts_order` / `preds_order` (optional, `order_state(B, N2 | N1, device)`): ordering states of the two clouds
+    (hg_nn_bidir_temporal_f32); the results do not depend on them."""
     require(gts, "gts", ndim=3)
     require(preds, "preds", ndim=3)
     B, N2, D = gts.shape
@@ -50,8 +69,15 @@ def nn_bidir(gts, preds):
     arg2 = torch.empty((B, N2), dtype=torch.int32, device=dev)
     nbytes = lib().hg_nn_bidir_workspace_bytes(B, N2, N1, D)
     ws = workspace(nbytes, dev)
-    check(lib().hg_nn_bidir_f32(ptr(gts), ptr(preds), B, N2, N1, D, ptr(min1), ptr(arg1), ptr(min2), ptr(arg2),
-                                ptr(ws), ws.numel(), stream_ptr()), "hg_nn_bidir_f32")
+    if gts_order is None and preds_order is None:
+        check(lib().hg_nn_bidir_f32(ptr(gts), ptr(preds), B, N2, N1, D, ptr(min1), ptr(arg1), ptr(min2), ptr(arg2),
+                                    ptr(ws), ws.numel(), stream_ptr()), "hg_nn_bidir_f32")
+        return min1, arg1, min2, arg2
+    _check_order(gts_order, B, N2, dev, "gts_order")
+    _check_order(preds_order, B, N1, dev, "preds_order")
+    check(lib().hg_nn_bidir_temporal_f32(ptr(gts), ptr(preds), B, N2, N1, D, ptr(min1), ptr(arg1), ptr(min2), ptr(arg2),
+                                         ptr(gts_order), ptr(preds_order), ptr(ws), ws.numel(), stream_ptr()),
+          "hg_nn_bidir_temporal_f32")
     return min1, arg1, min2, arg2
 
 
@@ -113,29 +139,30 @@ class shared_distance_pass:
         return False
 
     @staticmethod
-    def lookup(preds, gts, preds_c, gts_c):
+    def lookup(preds, gts, preds_c, gts_c, preds_order=None, gts_order=None):
         if shared_distance_pass._depth == 0:
-            return nn_bidir(gts_c, preds_c)
+            return nn_bidir(gts_c, preds_c, gts_order, preds_order)
         key = (preds_c.data_ptr(), preds._version, gts_c.data_ptr(), gts._version, tuple(preds_c.shape),
                tuple(gts_c.shape), stream_ptr())
         for k, _, res in shared_distance_pass._entries:
             if k == key:
                 return res
-        res = nn_bidir(gts_c, preds_c)
+        res = nn_bidir(gts_c, preds_c, gts_order, preds_order)
         # the entry keeps its inputs alive, so their addresses cannot be recycled for other tensors meanwhile
         shared_distance_pass._entries.append((key, (preds, gts, preds_c, gts_c), res))
         return res
 
 
 class SetDistanceFn(torch.autograd.Function):
-    """(preds, gts) -> (loss1 [B], loss2 [B]) for Chamfer (mode 0) / Hausdorff (mode 1)."""
+    """(preds, gts) -> (loss1 [B], loss2 [B]) for Chamfer (mode 0) / Hausdorff (mode 1); optional ordering states of
+    the two clouds (`order_state`)."""
 
     @staticmethod
     @_on_tensor_device
-    def forward(ctx, preds, gts, mode):
+    def forward(ctx, preds, gts, mode, preds_order=None, gts_order=None):
         preds_c = preds.detach().contiguous()
         gts_c = gts.detach().contiguous()
-        min1, arg1, min2, arg2 = shared_distance_pass.lookup(preds, gts, preds_c, gts_c)
+        min1, arg1, min2, arg2 = shared_distance_pass.lookup(preds, gts, preds_c, gts_c, preds_order, gts_order)
         loss1, loss2, hd1, hd2 = set_loss(min1, min2, mode)
         ctx.mode = mode
         # save_for_backward (not a plain attribute): preds_c / gts_c alias the caller's storage when it is contiguous,
@@ -153,11 +180,12 @@ class SetDistanceFn(torch.autograd.Function):
         dev = preds_c.device
         need_p, need_g = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
         if g1 is None and g2 is None:
-            return (torch.zeros_like(preds_c) if need_p else None), (torch.zeros_like(gts_c) if need_g else None), None
+            return ((torch.zeros_like(preds_c) if need_p else None), (torch.zeros_like(gts_c) if need_g else None), None,
+                    None, None)
         g1 = None if g1 is None else g1.to(torch.float32).contiguous()
         g2 = None if g2 is None else g2.to(torch.float32).contiguous()
         grad_preds, grad_gts = set_loss_bwd(gts_c, preds_c, arg1, arg2, hd1, hd2, g1, g2, ctx.mode, need_g)
-        return (grad_preds if need_p else None), (grad_gts if need_g else None), None
+        return (grad_preds if need_p else None), (grad_gts if need_g else None), None, None, None
 
 
 def _as_points(t, name):
@@ -172,26 +200,28 @@ def _as_points(t, name):
     return t
 
 
-def chamfer_losses(preds, gts):
+def chamfer_losses(preds, gts, preds_order=None, gts_order=None):
     """`ChamferDistance.forward(preds, gts)` (set_distance.py:40-50) -> (loss1 [B], loss2 [B])."""
-    return SetDistanceFn.apply(_as_points(preds, "preds"), _as_points(gts, "gts"), MODE_CHAMFER)
+    return SetDistanceFn.apply(_as_points(preds, "preds"), _as_points(gts, "gts"), MODE_CHAMFER, preds_order, gts_order)
 
 
-def hausdorff_losses(preds, gts):
+def hausdorff_losses(preds, gts, preds_order=None, gts_order=None):
     """`HausdorffDistance.forward(preds, gts)` (set_distance.py:58-70)."""
-    return SetDistanceFn.apply(_as_points(preds, "preds"), _as_points(gts, "gts"), MODE_HAUSDORFF)
+    return SetDistanceFn.apply(_as_points(preds, "preds"), _as_points(gts, "gts"), MODE_HAUSDORFF, preds_order,
+                               gts_order)
 
 
 # ------------------------------------------------------------------------------------------------------------
 # kNN (util/dist_utils.py KNNDist, model/dgcnn_cls.py knn, pytorch3d.ops.knn_points)
 # ------------------------------------------------------------------------------------------------------------
 @_on_tensor_device
-def knn_self(pc, k1, want_vals=True, state=None, state_valid=False):
+def knn_self(pc, k1, want_vals=True, state=None, state_valid=False, order=None):
     """k1 smallest per row of dist[i,j] = (xx_j + (-2 zz_ij)) + xx_i.  pc [B,K,C] point-major.
 
     Returns (vals [B,K,k1] ascending or None, idx [B,K,k1] int32).  `state` (optional int32 [B,K,k1], caller-owned):
     the indices of an earlier call on a nearby cloud, used as temporal seeds when `state_valid`, and overwritten with
-    this call's indices (hg_knn_self_temporal_f32); the results do not depend on it."""
+    this call's indices (hg_knn_self_temporal_f32); `order` (optional, `order_state(B, K, device)`): the cloud's
+    ordering state (hg_knn_self_temporal_order_f32).  The results depend on neither."""
     require(pc, "pc", ndim=3)
     B, K, C = pc.shape
     dev = pc.device
@@ -202,8 +232,15 @@ def knn_self(pc, k1, want_vals=True, state=None, state_valid=False):
         require(state, "state", dtype=torch.int32, ndim=3)
         if tuple(state.shape) != (B, K, k1) or state.device != dev:
             raise RuntimeError(f"state must be an int32 [{B},{K},{k1}] tensor on {dev}")
-    check(lib().hg_knn_self_temporal_f32(ptr(pc), B, K, C, k1, ptr(vals), ptr(idx), ptr(state), 1 if state_valid else 0,
-                                         ptr(ws), ws.numel(), stream_ptr()), "hg_knn_self_temporal_f32")
+    if order is None:
+        check(lib().hg_knn_self_temporal_f32(ptr(pc), B, K, C, k1, ptr(vals), ptr(idx), ptr(state),
+                                             1 if state_valid else 0, ptr(ws), ws.numel(), stream_ptr()),
+              "hg_knn_self_temporal_f32")
+        return vals, idx
+    _check_order(order, B, K, dev, "order")
+    check(lib().hg_knn_self_temporal_order_f32(ptr(pc), B, K, C, k1, ptr(vals), ptr(idx), ptr(state),
+                                               1 if state_valid else 0, ptr(order), ptr(ws), ws.numel(), stream_ptr()),
+          "hg_knn_self_temporal_order_f32")
     return vals, idx
 
 
@@ -212,11 +249,11 @@ class KnnOutlierFn(torch.autograd.Function):
 
     @staticmethod
     @_on_tensor_device
-    def forward(ctx, pc, k, alpha, state=None, state_valid=False):
+    def forward(ctx, pc, k, alpha, state=None, state_valid=False, order=None):
         pc_c = pc.detach().contiguous()
         B, K, C = pc_c.shape
         dev = pc_c.device
-        vals, idx = knn_self(pc_c, k + 1, state=state, state_valid=state_valid)
+        vals, idx = knn_self(pc_c, k + 1, state=state, state_valid=state_valid, order=order)
         value = torch.empty((B, K), dtype=torch.float32, device=dev)
         mask = torch.empty((B, K), dtype=torch.float32, device=dev)
         loss = torch.empty(B, dtype=torch.float32, device=dev)
@@ -237,11 +274,11 @@ class KnnOutlierFn(torch.autograd.Function):
         ws = workspace(lib().hg_knn_outlier_bwd_workspace_bytes(B, K, ctx.k1), pc_c.device)
         check(lib().hg_knn_outlier_bwd_f32(ptr(pc_c), ptr(idx), ptr(mask), ptr(g), B, K, C, ctx.k1, ptr(grad), ptr(ws),
                                            ws.numel(), stream_ptr()), "hg_knn_outlier_bwd_f32")
-        return grad, None, None, None, None
+        return grad, None, None, None, None, None
 
 
-def knn_outlier_loss(pc, k, alpha, state=None, state_valid=False):
-    return KnnOutlierFn.apply(_as_points(pc, "pc"), int(k), float(alpha), state, bool(state_valid))
+def knn_outlier_loss(pc, k, alpha, state=None, state_valid=False, order=None):
+    return KnnOutlierFn.apply(_as_points(pc, "pc"), int(k), float(alpha), state, bool(state_valid), order)
 
 
 @_on_tensor_device
@@ -410,6 +447,14 @@ def tune_nn_bidir(T=0, RB=0):
 def force_knn_shape(qt=0, gp=0):
     """Test-only override of the streaming kNN kernel's instantiation (queries per lane, pairs per filter bit)."""
     lib().hg_knn_force_shape(int(qt), int(gp))
+
+
+def prune_order_counters():
+    """Ordering builds of the pruned path since the last call, per cloud, while hg_tune("prune_count", 1) is on:
+    (refit and kept, rebuilt from a state, built without a state).  Synchronises the device."""
+    out = (ctypes.c_ulonglong * 3)()
+    check(lib().hg_prune_order_counters(out), "hg_prune_order_counters")
+    return tuple(int(v) for v in out)
 
 
 def tune_knn_small(small_max_n=0):

@@ -61,11 +61,18 @@ int hg_probe_fp32_peak(float *tflops, float *device_scratch, hgStream stream);
  * instead of the default 5-operation exact tracker (same results; see hg_nn_bidir.cu for why it is not the default);
  * "small_fused" = 1 sends clouds that fit in shared memory down the general finish / kNN-backward kernels as well
  * (same results; the tests run both); "knn_win" = Z-order window of the small-cloud kNN seeds (0 = default);
- * "fps_threads" = 128 | 256 threads per cloud in furthest point sampling for clouds up to 2048 points (0 = default). */
+ * "fps_threads" = 128 | 256 threads per cloud in furthest point sampling for clouds up to 2048 points (0 = default);
+ * "prune" = 0 switches the pruned passes off, "prune_min_n" moves their size threshold, "prune_count" = 1 counts visited
+ * leaf pairs and orderings; "prune_refit_tol" = rebuild tolerance of an ordering state's refit [permille] (0 = default),
+ * "prune_refit_stage" = 1 stages the cloud in shared memory for the refit's gather, 2 reads it from global memory
+ * (0 = default). */
 int hg_tune(const char *key, int value);
 /* Leaf pairs the pruned passes visited and could have visited since the last call: {Chamfer visited, Chamfer total,
  * kNN visited, kNN total}, counted while hg_tune("prune_count", 1) is on.  Synchronises the device. */
 int hg_prune_counters(unsigned long long *out4);
+/* Ordering builds since the last call, counted per cloud while hg_tune("prune_count", 1) is on: {refit and kept, rebuilt
+ * from a state (invalid permutation or degraded leaf boxes), built without a state}.  Synchronises the device. */
+int hg_prune_order_counters(unsigned long long *out3);
 unsigned long long hg_launch_count(void); /* kernels launched by this library since it was loaded */
 void hg_prof_enable(int on);
 int hg_prof_read(int tag, float *total_ms, int *launches);
@@ -93,6 +100,25 @@ void hg_knn_tune_small(int small_max_n);
 size_t hg_nn_bidir_workspace_bytes(int B, int N2, int N1, int D);
 int hg_nn_bidir_f32(const float *gts, const float *preds, int B, int N2, int N1, int D, float *min1, int *arg1,
                     float *min2, int *arg2, void *workspace, size_t workspace_bytes, hgStream stream);
+
+/* Ordering state for attack loops (CW/kNN.py:77-111 evaluates the losses 2500 times on the same `ori` and on an `adv`
+ * that moves by a learning-rate step per iteration).  Clouds of 8192..16384 points take spatially pruned passes that
+ * first put every cloud in kd-tree order; a state keeps one cloud batch's permutation (int32 [B,N]) and, per cloud, the
+ * quality of the leaf boxes it had when it was built.  A call with a state refits instead of rebuilding: it gathers the
+ * points through the stored permutation and recomputes norms and leaf boxes (a pass over memory), and rebuilds, on the
+ * device and only for those clouds, the orderings whose permutation is invalid or whose boxes have grown by more than a
+ * tolerance.  The state holds nothing specific to a call, so the Chamfer call and the self-kNN call on the same cloud can
+ * share one.  Everything read from the state is validated on the device: garbage or stale contents (an uninitialised
+ * buffer included) cost speed, never correctness -- results are bit-identical to the stateless calls.  The state is
+ * read and written by the call, on its stream: one state must not be used by calls on two streams at the same time.
+ * It is ignored and left untouched when the pruned path does not apply (D != 3, N outside the size range,
+ * hg_tune("prune", 0)).  The size does not depend on hg_tune, so a caller can allocate once. */
+size_t hg_order_state_bytes(int B, int N);
+/* hg_nn_bidir_f32 with ordering states for gts [B,N2,3] and preds [B,N1,3]: two distinct buffers, 16-byte aligned;
+ * either may be NULL (that cloud is then ordered in the workspace, as hg_nn_bidir_f32 does).  Same workspace. */
+int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B, int N2, int N1, int D, float *min1, int *arg1,
+                             float *min2, int *arg2, void *gts_order, void *preds_order, void *workspace,
+                             size_t workspace_bytes, hgStream stream);
 
 /* util/set_distance.py:15-32 `batch_pairwise_dist(x [B,Nx,D], y [B,Ny,D])` -> P [B,Nx,Ny], materialised.
  * Debug / API-completeness entry point: the loss path above never stores P. */
@@ -130,6 +156,11 @@ int hg_knn_self_f32(const float *pc, int B, int K, int C, int k1, float *vals, i
  * idx_state holds this call's indices (a copy of idx; idx_state may alias idx). */
 int hg_knn_self_temporal_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, int *idx_state,
                              int state_valid, void *workspace, size_t workspace_bytes, hgStream stream);
+/* hg_knn_self_temporal_f32 with an ordering state for pc (see hg_order_state_bytes; NULL = ordered in the workspace):
+ * a state the Chamfer call on the same cloud just refit or rebuilt is refit again here.  Same workspace. */
+int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, int *idx_state,
+                                   int state_valid, void *order, void *workspace, size_t workspace_bytes,
+                                   hgStream stream);
 
 /* util/dist_utils.py:157-172: value = mean of the k = k1-1 non-first neighbours, threshold mean+alpha*std
  * (unbiased), mask, loss[b] = weights[b] * mean(value*mask).  weights may be NULL (ones). */
