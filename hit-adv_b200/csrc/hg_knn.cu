@@ -190,7 +190,12 @@ __global__ void __launch_bounds__(256) knn_dist_generic_kernel(const float *__re
 //   3. k1 rounds of "smallest (value, index) strictly after the previous pick" run over the candidates only.
 // The first version ran step 3 over the whole row (k1 x K/32 steps per lane).  If the candidates overflow the buffer
 // (heavy ties), the row falls back to exactly that.
-constexpr int kSelCap = 128;  // candidates per row kept in shared memory (4 per lane)
+// Long lists (kLong: 33 <= k1 <= 64) bound with the TWO smallest strided elements of every lane instead: the k1-th
+// smallest of those 64 distinct elements (one 64-wide bitonic sort, two per lane) is again an upper bound, and the
+// candidate buffer is twice as large.
+constexpr int kSelCap = 128;      // candidates per row kept in shared memory (4 per lane)
+constexpr int kSelCapLong = 256;  // the same for long lists (8 per lane)
+__host__ __device__ constexpr int knn_sel_cap(bool long_list) { return long_list ? kSelCapLong : kSelCap; }
 
 __device__ __forceinline__ void knn_select_rounds(const float *__restrict__ v, const int *__restrict__ id, int n,
                                                   int k1, int lane, float *__restrict__ vals, int *__restrict__ idx,
@@ -220,35 +225,73 @@ __device__ __forceinline__ void knn_select_rounds(const float *__restrict__ v, c
   }
 }
 
+template <bool kLong>
 __global__ void __launch_bounds__(128) knn_select_rows_kernel(const float *__restrict__ dist, int nrows, int K,
                                                               int k1, float *__restrict__ vals,
                                                               int *__restrict__ idx) {
-  extern __shared__ float rowbuf[];  // [4 warps][K] rows, then [4][kSelCap] candidate values, [4][kSelCap] indices
+  constexpr int kCap = knn_sel_cap(kLong);
+  extern __shared__ float rowbuf[];  // [4 warps][K] rows, then [4][kCap] candidate values, [4][kCap] indices
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float *row = rowbuf + (size_t)warp * K;
-  float *cv = rowbuf + (size_t)4 * K + (size_t)warp * kSelCap;
-  int *ci = reinterpret_cast<int *>(rowbuf + (size_t)4 * K + (size_t)4 * kSelCap) + (size_t)warp * kSelCap;
+  float *cv = rowbuf + (size_t)4 * K + (size_t)warp * kCap;
+  int *ci = reinterpret_cast<int *>(rowbuf + (size_t)4 * K + (size_t)4 * kCap) + (size_t)warp * kCap;
   for (int r = blockIdx.x * 4 + warp; r < nrows; r += gridDim.x * 4) {
     __syncwarp();
-    float lmin = CUDART_INF_F;
+    float lmin = CUDART_INF_F, lmin2 = CUDART_INF_F;  // (lmin2: the second smallest, long lists only)
     for (int j = lane; j < K; j += 32) {
       const float x = dist[(size_t)r * K + j];
       row[j] = x;
-      lmin = fminf(lmin, x);
-    }
-    // bitonic sort of the 32 lane minima across the warp (ascending by lane)
-    float s = lmin;
-#pragma unroll
-    for (int size = 2; size <= 32; size <<= 1) {
-#pragma unroll
-      for (int stride = size >> 1; stride > 0; stride >>= 1) {
-        const float o = __shfl_xor_sync(0xffffffffu, s, stride);
-        const bool up = ((lane & size) == 0);         // ascending block
-        const bool lower = ((lane & stride) == 0);    // this lane keeps the smaller of the pair in an ascending block
-        s = (up == lower) ? fminf(s, o) : fmaxf(s, o);
+      if (kLong) {  // (a NaN compares false and is skipped, as fminf skips it)
+        if (x < lmin) {
+          lmin2 = lmin;
+          lmin = x;
+        } else if (x < lmin2) {
+          lmin2 = x;
+        }
+      } else {
+        lmin = fminf(lmin, x);
       }
     }
-    const float tau = __shfl_sync(0xffffffffu, s, k1 - 1);
+    float tau;
+    if (kLong) {
+      // bitonic sort of the 64 values (element e = lane + 32 r held as s[r]), ascending; stride 32 pairs a lane's own
+      // two values, and the size-32 blocks run ascending for r = 0, descending for r = 1
+      float s[2] = {lmin, lmin2};
+#pragma unroll
+      for (int size = 2; size <= 64; size <<= 1) {
+#pragma unroll
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+          if (stride == 32) {
+            const float lo = fminf(s[0], s[1]), hi = fmaxf(s[0], s[1]);
+            s[0] = lo;
+            s[1] = hi;
+            continue;
+          }
+          const bool lower = ((lane & stride) == 0);
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            const float o = __shfl_xor_sync(0xffffffffu, s[h], stride);
+            const bool up = size == 64 ? true : size == 32 ? h == 0 : ((lane & size) == 0);
+            s[h] = (up == lower) ? fminf(s[h], o) : fmaxf(s[h], o);
+          }
+        }
+      }
+      tau = __shfl_sync(0xffffffffu, s[1], k1 - 33);  // element k1 - 1 >= 32
+    } else {
+      // bitonic sort of the 32 lane minima across the warp (ascending by lane)
+      float s = lmin;
+#pragma unroll
+      for (int size = 2; size <= 32; size <<= 1) {
+#pragma unroll
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+          const float o = __shfl_xor_sync(0xffffffffu, s, stride);
+          const bool up = ((lane & size) == 0);         // ascending block
+          const bool lower = ((lane & stride) == 0);    // this lane keeps the smaller of the pair in an ascending block
+          s = (up == lower) ? fminf(s, o) : fmaxf(s, o);
+        }
+      }
+      tau = __shfl_sync(0xffffffffu, s, k1 - 1);
+    }
     __syncwarp();
     int cnt = 0;
     for (int j0 = 0; j0 < K; j0 += 32) {
@@ -257,14 +300,14 @@ __global__ void __launch_bounds__(128) knn_select_rows_kernel(const float *__res
       const bool keep = (j < K) && (x <= tau);
       const unsigned m = __ballot_sync(0xffffffffu, keep);
       const int pos = cnt + __popc(m & ((1u << lane) - 1u));
-      if (keep && pos < kSelCap) {
+      if (keep && pos < kCap) {
         cv[pos] = x;
         ci[pos] = j;
       }
       cnt += __popc(m);
     }
     __syncwarp();
-    if (cnt <= kSelCap)
+    if (cnt <= kCap)
       knn_select_rounds(cv, ci, cnt, k1, lane, vals, idx, (size_t)r * k1);
     else
       knn_select_rounds(row, nullptr, K, k1, lane, vals, idx, (size_t)r * k1);
@@ -543,7 +586,7 @@ constexpr size_t kGenericScratchBytes = (size_t)256 << 20;
 }  // namespace
 
 // 3-D self-kNN shapes that may take the tensor-core kernel on a padded copy (the dispatch also looks at the batch size)
-static bool knn3_pad_candidate(int K, int k1) { return k1 >= 12 && hg_knn_tc_supported(K, kPadC, k1); }
+static bool knn3_pad_candidate(int K, int k1) { return k1 >= 12 && k1 <= 32 && hg_knn_tc_supported(K, kPadC, k1); }
 
 HG_API size_t hg_knn_self_workspace_bytes(int B, int K, int C, int k1) {
   if (B <= 0 || K <= 0 || C <= 0) return 0;
@@ -582,8 +625,7 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   HG_REQUIRE(pc && idx, HG_E_BADARG, "knn_self: null pointer");
   HG_REQUIRE(((uintptr_t)order & 15) == 0, HG_E_BADARG, "knn_self: the ordering state must be 16-byte aligned");
   HG_REQUIRE(B > 0 && K > 0 && C > 0, HG_E_BADARG, "knn_self: sizes must be positive");
-  HG_REQUIRE(k1 >= 1 && k1 <= (C == 3 ? 64 : 32) && k1 <= K, HG_E_BADARG,
-             "knn_self: need 1 <= k <= min(%d, K); got k=%d K=%d", C == 3 ? 64 : 32, k1, K);
+  HG_REQUIRE(k1 >= 1 && k1 <= 64 && k1 <= K, HG_E_BADARG, "knn_self: need 1 <= k <= min(64, K); got k=%d K=%d", k1, K);
   HG_REQUIRE(B <= 65535, HG_E_UNSUPPORTED, "knn_self: B=%d > 65535 clouds per call", B);
   if (C == 3) {
     // long lists on enough clouds to fill the machine: the tensor-core kernel on a 32-channel copy beats the 3-D
@@ -619,23 +661,28 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   // else (and hg_tune("knn_tc", 1)) takes the FP32 distance tile + row select below
   // (small batches leave the serial chain of a CTA exposed -- measured at K = 1024, C = 64: 16 clouds 85 us against
   // 143 us, 8 clouds 82 against 95, 4 clouds 79 against 65 -- so fewer CTAs than a quarter of the SMs stay on the FP32
-  // path unless hg_tune("knn_tc", 2) forces the tensor-core kernel)
-  const bool tc_fills = 4LL * B * ((K + 127) / 128) >= hg_sm_count() || g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5;
+  // path unless hg_tune("knn_tc", 2) forces the tensor-core kernel; long lists, k1 > 32, need half the SMs -- measured at
+  // 2048 x 64, k = 40: 4 clouds 143 us FP32 against 153 tensor-core, 8 clouds 283 against 157, 32 clouds 1121 against 393)
+  const long long tc_ctas = (long long)B * ((K + 127) / 128);
+  const bool tc_fills = (k1 > 32 ? 2 : 4) * tc_ctas >= hg_sm_count() || g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5;
   if (g_hg_tune_knn_tc_off != 1 && tc_fills && hg_knn_tc_supported(K, C, k1) && (reinterpret_cast<uintptr_t>(pc) & 15) == 0)
     return hg_knn_tc_run(pc, xx, B, K, C, k1, vals, idx, stream);
   const size_t per = (size_t)K * K * sizeof(float);
   int nb = (int)(kGenericScratchBytes / per);
   if (nb < 1) nb = 1;
-  const size_t sel_smem = ((size_t)4 * K + (size_t)8 * kSelCap) * sizeof(float);
+  const bool long_list = k1 > 32;
+  const size_t sel_smem = ((size_t)4 * K + (size_t)8 * knn_sel_cap(long_list)) * sizeof(float);
   if (sel_smem > 48 * 1024)
-    HG_CUDA(cudaFuncSetAttribute(knn_select_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sel_smem));
+    HG_CUDA(cudaFuncSetAttribute(long_list ? knn_select_rows_kernel<true> : knn_select_rows_kernel<false>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sel_smem));
   for (int b0 = 0; b0 < B; b0 += nb) {
     const int cb = (B - b0 < nb) ? (B - b0) : nb;
     dim3 grid((K + kGTN - 1) / kGTN, (K + kGTM - 1) / kGTM, cb);
     knn_dist_generic_kernel<<<grid, 256, 0, stream>>>(pc + (size_t)b0 * K * C, xx + (size_t)b0 * K, K, C, dist);
     HG_CHECK_LAUNCH("knn_dist_generic_kernel");
     const int nrows = cb * K;
-    knn_select_rows_kernel<<<grid_for((long long)nrows * 32, 128), 128, sel_smem, stream>>>(
+    (long_list ? knn_select_rows_kernel<true> : knn_select_rows_kernel<false>)<<<grid_for((long long)nrows * 32, 128),
+                                                                                 128, sel_smem, stream>>>(
         dist, nrows, K, k1, vals ? vals + (size_t)b0 * K * k1 : nullptr, idx + (size_t)b0 * K * k1);
     HG_CHECK_LAUNCH("knn_select_rows_kernel");
   }

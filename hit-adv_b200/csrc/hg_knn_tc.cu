@@ -392,6 +392,258 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
 }
 
+__device__ __forceinline__ void tc_ld16(uint32_t taddr, float (&v)[16]) {
+  uint32_t r[16];
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, "
+      "[%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
+
+// ---- long lists (33 <= k1 <= 64; DGCNN with k = 40): the same filter and exact evaluation, register budget reworked ----
+// A 64-entry (value, index) list takes 128 registers, and knn_tc_fused_kernel<64, 32> already uses 251, so this kernel
+// differs from it in three ways (the short-list instantiations stay as they are):
+//   * the own row is always re-read from the A panels (as C = 96/128 already do): -C registers at C <= 64;
+//   * the threshold sweep and the evaluation sweep are two separate loops, and the list is initialised between them,
+//     so the 64 class minima and the 128 list registers are never live together;
+//   * the TMEM accumulator is read 16 columns at a time instead of 32.
+// The first threshold is the k1-th smallest of 64 column-class minima (class = column mod 64; K >= 256, so tile 0 alone
+// already gives every class a real column): k1 <= 64 distinct columns have an approximate distance <= tau, so the
+// admission test  approx_j <= (k1-th exact so far) + 2 eps  is the short-list kernel's, and so are values and indices.
+template <int C>
+__global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
+    knn_tc_long_kernel(const __grid_constant__ CUtensorMap map, int K, int k1, int two_pass,
+                       const float *__restrict__ xx, float *__restrict__ vals, int *__restrict__ idx) {
+  constexpr int KM = 64;
+  constexpr int NP = C / kTcPanelK;
+  constexpr int kABytes = kTcRows * 128, kBBytes = kTcTile * 128;
+  extern __shared__ __align__(1024) unsigned char smraw[];
+  unsigned char *sA = smraw, *sB = smraw + NP * kABytes;
+  float *sxx = reinterpret_cast<float *>(sB + NP * kBBytes);
+  __shared__ __align__(8) uint64_t bar_a, bar_b, bar_mma;
+  __shared__ uint32_t tmem_base_s;
+  __shared__ float wmax[4];
+
+  const int b = blockIdx.y, row0 = blockIdx.x * kTcRows;
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const int ntiles = (K + kTcTile - 1) / kTcTile;
+
+  if (tid == 0) {
+    hg_mbar_init(&bar_a, 1);
+    hg_mbar_init(&bar_b, 1);
+    hg_mbar_init(&bar_mma, 1);
+    hg_mbar_init_fence();
+  }
+  if (warp == 0) {
+    __syncwarp();
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(hg_smem_addr(&tmem_base_s))
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  float xmax = 0.f;
+  for (int j = tid; j < ntiles * kTcTile; j += 128) {
+    const float v = j < K ? xx[(size_t)b * K + j] : CUDART_INF_F;
+    sxx[j] = v;
+    if (j < K) xmax = fmaxf(xmax, v);
+  }
+  xmax = hg_warp_max_f32(xmax);
+  if ((tid & 31) == 0) wmax[warp] = xmax;
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = tmem_base_s;
+  xmax = fmaxf(fmaxf(wmax[0], wmax[1]), fmaxf(wmax[2], wmax[3]));
+
+  if (tid == 0) {
+    hg_mbar_expect_tx(&bar_a, NP * kABytes);
+    for (int p = 0; p < NP; ++p) tc_tma_load_3d(sA + p * kABytes, &map, &bar_a, p * kTcPanelK, row0, b);
+  }
+
+  const int i = row0 + tid;
+  const bool live = i < K;
+  const float xi = live ? sxx[i] : 0.f;
+  const float eps = 1.1f * 0.00390625f * sqrtf(xi * xmax) + 1e-5f * (xi + xmax);
+  const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
+  const unsigned sw = (unsigned)(tid & 7);
+  unsigned phase_b = 0, phase_m = 0;
+
+  // tile t into the B panels, 128 x 256 accumulator into TMEM; every thread waits for both itself
+  auto load_mma = [&](int t, bool first) {
+    if (tid == 0) {
+      hg_mbar_expect_tx(&bar_b, NP * kBBytes);
+      for (int p = 0; p < NP; ++p) {
+        tc_tma_load_3d(sB + p * kBBytes, &map, &bar_b, p * kTcPanelK, t * kTcTile, b);
+        tc_tma_load_3d(sB + p * kBBytes + kABytes, &map, &bar_b, p * kTcPanelK, t * kTcTile + 128, b);
+      }
+      if (first) tc_mbar_wait(&bar_a, 0);
+      tc_mbar_wait(&bar_b, phase_b);
+      tc_fence_after();
+      constexpr uint32_t idesc = tc_idesc(kTcRows, kTcTile);
+#pragma unroll
+      for (int p = 0; p < NP; ++p)
+#pragma unroll
+        for (int ks = 0; ks < 4; ++ks)
+          tc_mma_tf32(tmem, tc_smem_desc(sA + p * kABytes, ks * 32), tc_smem_desc(sB + p * kBBytes, ks * 32), idesc,
+                      (p | ks) ? 1u : 0u);
+      tc_commit(&bar_mma);
+    }
+    if (first) tc_mbar_wait(&bar_a, 0);
+    tc_mbar_wait(&bar_b, phase_b);
+    phase_b ^= 1;
+    tc_mbar_wait(&bar_mma, phase_m);
+    phase_m ^= 1;
+    __syncwarp();
+    tc_fence_after();
+  };
+  auto release = [&]() {
+    tc_fence_before();
+    __syncthreads();  // the accumulator and the B panels are free again
+    tc_fence_after();
+  };
+
+  // ---- threshold sweep: all tiles (two_pass) or tile 0 only ----
+  float thr;
+  {
+    float m[64];
+#pragma unroll
+    for (int c = 0; c < 64; ++c) m[c] = CUDART_INF_F;
+    const int nscan = two_pass ? ntiles : 1;
+    for (int t = 0; t < nscan; ++t) {
+      load_mma(t, t == 0);
+#pragma unroll 1
+      for (int q2 = 0; q2 < kTcTile / 64; ++q2)
+#pragma unroll
+        for (int h = 0; h < 4; ++h) {  // columns q2 * 64 + h * 16 + c: class h * 16 + c
+          float acc[16];
+          tc_ld16(trow + (uint32_t)(q2 * 64 + h * 16), acc);
+          const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q2 * 64 + h * 16);
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            const float4 xj = sx4[c4];
+            float *mm = m + h * 16 + 4 * c4;
+            mm[0] = fminf(mm[0], fmaf(-2.0f, acc[4 * c4], xi + xj.x));
+            mm[1] = fminf(mm[1], fmaf(-2.0f, acc[4 * c4 + 1], xi + xj.y));
+            mm[2] = fminf(mm[2], fmaf(-2.0f, acc[4 * c4 + 2], xi + xj.z));
+            mm[3] = fminf(mm[3], fmaf(-2.0f, acc[4 * c4 + 3], xi + xj.w));
+          }
+        }
+      if (two_pass) release();
+    }
+#pragma unroll
+    for (int size = 2; size <= 64; size <<= 1)
+#pragma unroll
+      for (int stride = size >> 1; stride > 0; stride >>= 1)
+#pragma unroll
+        for (int a = 0; a < 64; ++a) {
+          const int p2 = a ^ stride;
+          if (p2 > a) {
+            const bool up = (a & size) == 0;
+            const float lo = fminf(m[a], m[p2]), hi = fmaxf(m[a], m[p2]);
+            m[a] = up ? lo : hi;
+            m[p2] = up ? hi : lo;
+          }
+        }
+    float tau = -CUDART_INF_F;  // m[k1 - 1], as a masked maximum (see TcList::kth)
+#pragma unroll
+    for (int c = 0; c < 64; ++c)
+      if (c < k1) tau = fmaxf(tau, m[c]);
+    thr = tau + 2.0f * eps;
+  }
+
+  // ---- evaluation sweep (the single-sweep variant evaluates tile 0 from the accumulator it has just scanned) ----
+  TcList<KM> top;
+  top.init();
+  for (int t = 0; t < ntiles; ++t) {
+    if (two_pass || t > 0) load_mma(t, false);
+    unsigned hm[kTcTile / 32];
+#pragma unroll
+    for (int q = 0; q < kTcTile / 32; ++q) {
+      unsigned hits = 0u;
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        float acc[16];
+        tc_ld16(trow + (uint32_t)(q * 32 + h * 16), acc);
+        const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q * 32 + h * 16);
+#pragma unroll
+        for (int c4 = 0; c4 < 4; ++c4) {
+          const float4 xj = sx4[c4];
+          const int s = h * 16 + 4 * c4;
+          hits |= (fmaf(-2.0f, acc[4 * c4], xi + xj.x) <= thr ? 1u : 0u) << s;
+          hits |= (fmaf(-2.0f, acc[4 * c4 + 1], xi + xj.y) <= thr ? 1u : 0u) << (s + 1);
+          hits |= (fmaf(-2.0f, acc[4 * c4 + 2], xi + xj.z) <= thr ? 1u : 0u) << (s + 2);
+          hits |= (fmaf(-2.0f, acc[4 * c4 + 3], xi + xj.w) <= thr ? 1u : 0u) << (s + 3);
+        }
+      }
+      hm[q] = live ? hits : 0u;
+    }
+    auto next_hit = [&]() -> int {  // lowest set bit of the 256-bit mask, cleared; -1 when none is left
+      unsigned w = 0u;
+      int base = -1;
+#pragma unroll
+      for (int q = kTcTile / 32 - 1; q >= 0; --q)
+        if (hm[q]) {
+          w = hm[q];
+          base = q;
+        }
+#pragma unroll
+      for (int q = 0; q < kTcTile / 32; ++q)
+        if (q == base) hm[q] = w & (w - 1u);
+      return base < 0 ? -1 : base * 32 + __ffs(w) - 1;
+    };
+    while (true) {
+      const int jr0 = next_hit();
+      if (!__any_sync(0xffffffffu, jr0 >= 0)) break;
+      if (jr0 >= 0) {
+        const int jr1 = next_hit();
+        const int jrb = jr1 >= 0 ? jr1 : jr0;
+        // the reference's sequential FMA chain for columns jr0, jrb (see exact2 in knn_tc_fused_kernel)
+        float acc0 = 0.f, acc1 = 0.f;
+        const unsigned sw0 = (unsigned)(jr0 & 7), sw1 = (unsigned)(jrb & 7);
+#pragma unroll
+        for (int p = 0; p < NP; ++p) {
+          const unsigned char *r0 = sB + p * kBBytes + jr0 * 128, *r1 = sB + p * kBBytes + jrb * 128;
+          const unsigned char *rowi = sA + p * kABytes + tid * 128;
+#pragma unroll
+          for (int c = 0; c < 8; ++c) {
+            const float4 v0 = *reinterpret_cast<const float4 *>(r0 + ((c ^ sw0) << 4));
+            const float4 v1 = *reinterpret_cast<const float4 *>(r1 + ((c ^ sw1) << 4));
+            const float4 a = *reinterpret_cast<const float4 *>(rowi + ((c ^ sw) << 4));
+            acc0 = __fmaf_rn(a.x, v0.x, acc0);
+            acc1 = __fmaf_rn(a.x, v1.x, acc1);
+            acc0 = __fmaf_rn(a.y, v0.y, acc0);
+            acc1 = __fmaf_rn(a.y, v1.y, acc1);
+            acc0 = __fmaf_rn(a.z, v0.z, acc0);
+            acc1 = __fmaf_rn(a.z, v1.z, acc1);
+            acc0 = __fmaf_rn(a.w, v0.w, acc0);
+            acc1 = __fmaf_rn(a.w, v1.w, acc1);
+          }
+        }
+        const float d0 = __fadd_rn(__fadd_rn(__fadd_rn(sxx[t * kTcTile + jr0], __fmul_rn(-2.0f, acc0)), xi), 0.0f);
+        const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(sxx[t * kTcTile + jrb], __fmul_rn(-2.0f, acc1)), xi), 0.0f);
+        if (d0 < top.v[KM - 1]) top.push(d0, t * kTcTile + jr0);
+        if (jr1 >= 0 && d1 < top.v[KM - 1]) top.push(d1, t * kTcTile + jr1);
+      }
+    }
+    thr = fminf(thr, (k1 == KM ? top.v[KM - 1] : top.kth(k1)) + 2.0f * eps);
+    release();
+  }
+  if (live) {
+    const size_t o = ((size_t)b * K + i) * k1;
+#pragma unroll
+    for (int s = 0; s < KM; ++s)
+      if (s < k1) {
+        if (vals) vals[o + s] = top.v[s];
+        idx[o + s] = top.id[s];
+      }
+  }
+  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -418,6 +670,7 @@ int run_tc(const float *pc, const float *xx, int B, int K, int k1, float *vals, 
   if (once.first()) {
     HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 20>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
     HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
+    HG_CUDA((cudaFuncSetAttribute(knn_tc_long_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
   }
   CUtensorMap map;
   const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)K, (cuuint64_t)B};
@@ -434,17 +687,20 @@ int run_tc(const float *pc, const float *xx, int B, int K, int k1, float *vals, 
   const int two_pass = g_hg_tune_knn_tc_off == 5 ? 0 : 1;
   if (k1 <= 20)
     knn_tc_fused_kernel<C, 20><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
-  else
+  else if (k1 <= 32)
     knn_tc_fused_kernel<C, 32><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
+  else
+    knn_tc_long_kernel<C><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
   HG_CHECK_LAUNCH("knn_tc_fused_kernel");
   return HG_OK;
 }
 
 }  // namespace
 
-// Shapes the tensor-core path takes: C a multiple of 32 up to 128 (DGCNN: 64, 64, 128), clouds of 256..4096 points.
+// Shapes the tensor-core path takes: C a multiple of 32 up to 128 (DGCNN: 64, 64, 128), clouds of 256..4096 points,
+// lists of up to 64 neighbours.
 bool hg_knn_tc_supported(int K, int C, int k1) {
-  return (C == 32 || C == 64 || C == 96 || C == 128) && K >= 256 && K <= 4096 && k1 <= 32;
+  return (C == 32 || C == 64 || C == 96 || C == 128) && K >= 256 && K <= 4096 && k1 <= 64;
 }
 
 // xx [B,K] are the reference squared norms (knn_sumsq_kernel).  B <= 65535 (checked by the caller).

@@ -218,7 +218,7 @@ def hausdorff_losses(preds, gts, preds_order=None, gts_order=None):
 def knn_self(pc, k1, want_vals=True, state=None, state_valid=False, order=None):
     """k1 smallest per row of dist[i,j] = (xx_j + (-2 zz_ij)) + xx_i.  pc [B,K,C] point-major.
 
-    Returns (vals [B,K,k1] ascending or None, idx [B,K,k1] int32).  `state` (optional int32 [B,K,k1], caller-owned):
+    1 <= k1 <= min(64, K) for every C.  Returns (vals [B,K,k1] ascending or None, idx [B,K,k1] int32).  `state` (optional int32 [B,K,k1], caller-owned):
     the indices of an earlier call on a nearby cloud, used as temporal seeds when `state_valid`, and overwritten with
     this call's indices (hg_knn_self_temporal_f32); `order` (optional, `order_state(B, K, device)`): the cloud's
     ordering state (hg_knn_self_temporal_order_f32).  The results depend on neither."""

@@ -71,7 +71,8 @@ def query_ball_point(radius, nsample, xyz, new_xyz):
 
 
 def knn(x, k):
-    """DGCNN kNN: x [B,C,N] -> idx [B,N,k] int64, the k largest of -||x_i - x_j||^2 (self included)."""
+    """DGCNN kNN: x [B,C,N] -> idx [B,N,k] int64, the k largest of -||x_i - x_j||^2 (self included); 1 <= k <= 64
+    for every C (DGCNN's k = 20 and k = 40 included)."""
     pc = x.detach().transpose(2, 1).contiguous()  # kernels are point-major
     _, idx = F.knn_self(pc, int(k), want_vals=False)
     return idx.long()

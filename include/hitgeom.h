@@ -142,7 +142,7 @@ int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *arg1, c
  * util/dist_utils.py:148-156 (KNNDist) and model/dgcnn_cls.py:8-12 (DGCNN knn): the k1 smallest entries per
  * row of dist[i,j] = (xx_j + (-2*zz_ij)) + xx_i (DGCNN's pairwise_distance is exactly -dist).
  *   pc [B,K,C] point-major; vals [B,K,k1] ascending (may be NULL), idx [B,K,k1], lowest index first on ties.
- *   1 <= k1 <= 64 for C == 3 (32 otherwise), k1 <= K.
+ *   1 <= k1 <= 64 for every C, k1 <= K (DGCNN's k = 40 on its feature layers included).
  * ------------------------------------------------------------------------------------------------------- */
 size_t hg_knn_self_workspace_bytes(int B, int K, int C, int k1);
 int hg_knn_self_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, void *workspace,
