@@ -205,7 +205,7 @@ bool hg_knn_tc_supported(int K, int C, int k1);
 int hg_knn_tc_run(const float *pc, const float *xx, int B, int K, int C, int k1, float *vals, int *idx, cudaStream_t stream);
 
 // ---- spatially pruned exact passes for large clouds (hg_prune.cu) ---------------------------------------------------
-#define HG_PRUNE_MAX_N 16384  // the ordering build sorts one cloud in shared memory with 14-bit point indices
+#define HG_PRUNE_MAX_N 16384  // the ordering build holds one cloud in shared memory and keys with 14-bit point indices
 // One cloud batch in kd-tree order: points (x, y, z, squared norm), original index of every sorted point, per-leaf
 // boxes (lo, hi) of 32 points, per-cloud (bound on max |p|^2, 1 if the cloud must take the all-pairs kernels).
 struct HgPruneOrder {

@@ -30,7 +30,6 @@ constexpr unsigned kIdxMask = (1u << kIdxBits) - 1u;
 constexpr unsigned kPadKey = 0xffffffffu;
 constexpr float kQuantMax = 262142.f;  // 2^18 - 2: a real key never equals kPadKey
 constexpr int kBuildThreads = 1024;
-constexpr int kMaxSegs = HG_PRUNE_MAX_N / 64;  // segments of the last split level
 constexpr int kSearchWarps = 4;
 constexpr float kSlack = 1.5e-6f;  // >= 24 u, u = 2^-24
 
@@ -78,25 +77,131 @@ __device__ __forceinline__ float block_sum_leaves(float h, float *s_h) {
   return H;
 }
 
-// ---- ordering build: one CTA per cloud, kd splits (median of the longest axis) by a segmented bitonic sort ----------
-// key[i] = (quantised coordinate on the segment's split axis) << 14 | point index; padding to a power of two carries
-// kPadKey and stays at the end of the array at every level.  Correctness never depends on the quality of a split:
-// the leaf boxes are recomputed from the points.
+// ---- ordering build: one CTA per cloud, kd splits (median of the longest axis) by selection -----------------------
+// The tree: the positions [0, Np) (Np = N padded to a power of two, padding at positions >= N) are split level by level
+// into segments of s = Np, Np/2, ..., 64 entries.  A segment's key of a point is (quantised coordinate on the
+// segment's longest axis) << 14 | point index, so keys are distinct, and the left child of a segment is exactly its
+// s/2 smallest keys (all of its real points when it holds s/2 or fewer; padding sorts after every real key).  The box,
+// the axis, the scale and so the next level's keys depend only on which points a segment holds, so the order of the
+// points inside a segment matters only at the last level, where each 64-entry segment is sorted by its key and that
+// order is the permutation.  Correctness never depends on the quality of a split: the leaf boxes are recomputed from
+// the points.
+//
+// Warp w of the first nw = Np / (32 E) warps holds the positions [w 32E, (w + 1) 32E), entry (h, lane) at w 32E + 32h +
+// lane.  Levels whose segments span several warps run CTA-wide: the segment's rank-(s/2 - 1) key by an MSD radix
+// select (8-bit digits, a shared-memory histogram per segment, one warp per segment scans it), then one in-place
+// partition (ballots and popc within a warp, the counts of the segment's earlier warps).  From 32E entries down, a
+// warp finishes its own entries in registers: per level, each group's box from warp reductions, its keys, and a
+// bitonic sort of the group with shuffles (the last one is the 64-entry sort that fixes the leaf order).
 //
 // With an ordering state (hdr != null: o.perm points into the state, hdr is its per-cloud header) the kernel runs after
 // prune_refit_kernel and rebuilds only the clouds the refit marked (info.z != 0); it then also stores the leaf-box
 // quality H of the new permutation in the header.  count (null, or g_order_counts): clouds ordered without a state.
-template <bool CHAMFER_NORM>
-__global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float *__restrict__ pc, int N, int Np,
-                                                                    HgPruneOrder o, float4 *hdr,
-                                                                    unsigned long long *count) {
-  extern __shared__ unsigned key[];  // [Np]
-  __shared__ unsigned smin[3][kMaxSegs], smax[3][kMaxSegs];
-  __shared__ float slo[kMaxSegs], sscale[kMaxSegs];
-  __shared__ int saxis[kMaxSegs];
+constexpr int kCtaSegs = kBuildThreads / 32 / 2;  // segments of the CTA-wide levels: at most half the warps
+
+struct SegSplit {
+  int ax;
+  float lo, scale;
+};
+// split of a segment from its box (ordered-int min / max per coordinate): the axis of the largest extent (strict >),
+// its low end and the quantisation scale
+__device__ __forceinline__ SegSplit seg_split(const unsigned (&mn)[3], const unsigned (&mx)[3]) {
+  SegSplit sp = {0, hg_unord(mn[0]), 0.f};
+  float ext = hg_unord(mx[0]) - sp.lo;
+#pragma unroll
+  for (int c = 1; c < 3; ++c) {
+    const float lo = hg_unord(mn[c]), e = hg_unord(mx[c]) - lo;
+    if (e > ext) {
+      sp.ax = c;
+      sp.lo = lo;
+      ext = e;
+    }
+  }
+  sp.scale = ext > 0.f ? kQuantMax / ext : 0.f;
+  return sp;
+}
+__device__ __forceinline__ unsigned split_key(const float *p, unsigned id, SegSplit sp) {
+  const float f = (p[(size_t)id * 3 + sp.ax] - sp.lo) * sp.scale;
+  return ((unsigned)fminf(fmaxf(f, 0.f), kQuantMax) << kIdxBits) | id;
+}
+__device__ __forceinline__ void box_add(const float *p, unsigned id, unsigned (&mn)[3], unsigned (&mx)[3]) {
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const unsigned u = hg_ord(p[(size_t)id * 3 + c]);
+    mn[c] = min(mn[c], u);
+    mx[c] = max(mx[c], u);
+  }
+}
+
+// Ascending bitonic sort of every group of G consecutive register rows (32 G entries, entry (h, lane) is element
+// 32 (h % G) + lane of group h / G), in registers with shuffles.
+template <int E, int G>
+__device__ __forceinline__ void warp_sort_groups(unsigned (&k)[E], int lane) {
+#pragma unroll
+  for (int kk = 2; kk <= 32 * G; kk <<= 1) {
+#pragma unroll
+    for (int j = kk >> 1; j > 0; j >>= 1) {
+      if (j >= 32) {
+        const int jh = j >> 5;
+#pragma unroll
+        for (int h = 0; h < E; ++h) {
+          if ((h & jh) == 0) {
+            const bool asc = (((h % G) << 5) & kk) == 0;
+            const unsigned lo = min(k[h], k[h | jh]), hi = max(k[h], k[h | jh]);
+            k[h] = asc ? lo : hi;
+            k[h | jh] = asc ? hi : lo;
+          }
+        }
+      } else {
+        const bool lower = (lane & j) == 0;
+#pragma unroll
+        for (int h = 0; h < E; ++h) {
+          const unsigned y = __shfl_xor_sync(0xffffffffu, k[h], j);
+          const bool asc = ((((h % G) << 5) | lane) & kk) == 0;
+          k[h] = lower == asc ? min(k[h], y) : max(k[h], y);
+        }
+      }
+    }
+  }
+}
+
+// The warp-local levels from groups of G rows down to 2 rows (64 entries): per group of 32 G entries the box (padding
+// is kPadKey), the keys, then the sort of every group.
+template <int E, int G>
+__device__ __forceinline__ void warp_levels(const float *p, unsigned (&v)[E], int lane) {
+#pragma unroll
+  for (int g = 0; g < E; g += G) {
+    unsigned lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};
+#pragma unroll
+    for (int h = g; h < g + G; ++h)
+      if (v[h] != kPadKey) box_add(p, v[h] & kIdxMask, lo, hi);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      lo[c] = __reduce_min_sync(0xffffffffu, lo[c]);
+      hi[c] = __reduce_max_sync(0xffffffffu, hi[c]);
+    }
+    const SegSplit sp = seg_split(lo, hi);
+#pragma unroll
+    for (int h = g; h < g + G; ++h)
+      if (v[h] != kPadKey) v[h] = split_key(p, v[h] & kIdxMask, sp);
+  }
+  warp_sort_groups<E, G>(v, lane);
+  if constexpr (G > 2) warp_levels<E, G / 2>(p, v, lane);
+}
+
+// E = entries per lane (Np / 1024 from 2048 points up, else 2)
+template <bool CHAMFER_NORM, int E>
+__global__ void __launch_bounds__(kBuildThreads, 1) prune_order_kernel(const float *__restrict__ pc, int N, int Np,
+                                                                       HgPruneOrder o, float4 *hdr,
+                                                                       unsigned long long *count) {
+  extern __shared__ unsigned sid[];  // [Np] point indices in tree order
+  __shared__ unsigned smin[3][kCtaSegs], smax[3][kCtaSegs];
+  __shared__ SegSplit ssplit[kCtaSegs];
+  __shared__ unsigned hist[kCtaSegs][256], spref[kCtaSegs], srank[kCtaSegs], swl[kBuildThreads / 32];
   __shared__ unsigned s_bad, s_norm;
   __shared__ float s_h[kBuildThreads / 32];
-  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  constexpr int C = 32 * E;  // entries per warp
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (hdr != nullptr && o.info[b].z == 0.f) return;  // the refit kept this cloud's ordering
   if (count != nullptr && hdr == nullptr && tid == 0) atomicAdd(count + 2, 1ull);
   const float *p = pc + (size_t)b * N * 3;
@@ -104,16 +209,15 @@ __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float 
     s_bad = 0u;
     s_norm = 0u;
   }
+  for (int t = tid; t < kCtaSegs * 256; t += kBuildThreads) (&hist[0][0])[t] = 0u;
   __syncthreads();
   float mn = 0.f;
   bool bad = false;
-  for (int i = tid; i < Np; i += kBuildThreads) {
-    key[i] = i < N ? (unsigned)i : kPadKey;
-    if (i < N) {
-      const float x = p[(size_t)i * 3], y = p[(size_t)i * 3 + 1], z = p[(size_t)i * 3 + 2];
-      bad |= !(isfinite(x) && isfinite(y) && isfinite(z));
-      mn = fmaxf(mn, fmaf(z, z, fmaf(y, y, x * x)));
-    }
+  for (int i = tid; i < N; i += kBuildThreads) {
+    sid[i] = (unsigned)i;
+    const float x = p[(size_t)i * 3], y = p[(size_t)i * 3 + 1], z = p[(size_t)i * 3 + 2];
+    bad |= !(isfinite(x) && isfinite(y) && isfinite(z));
+    mn = fmaxf(mn, fmaf(z, z, fmaf(y, y, x * x)));
   }
   mn = hg_warp_max_f32(mn);
   bad = __any_sync(0xffffffffu, bad);
@@ -127,73 +231,139 @@ __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float 
   if (tid == 0) o.info[b] = make_float4(norm * 1.0001f, flagged ? 1.f : 0.f, 0.f, 0.f);
   if (flagged) return;
 
-  for (int s = Np; s > kLeaf; s >>= 1) {
-    const int nseg = Np / s;
-    for (int t = tid; t < nseg; t += kBuildThreads)
+  const bool active = warp < Np / C;
+  const int wbase = warp * C;
+  unsigned v[E];  // the warp's entries: point indices, then this level's keys
+  // CTA-wide levels: segments of 2C .. Np entries
+  for (int s = Np; s > C; s >>= 1) {
+    const int nseg = Np / s, seg = wbase / s, sbase = seg * s;
+    if (tid < nseg)
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        smin[c][t] = 0xffffffffu;
-        smax[c][t] = 0u;
+        smin[c][tid] = 0xffffffffu;
+        smax[c][tid] = 0u;
       }
     __syncthreads();
-    for (int i = tid; i < Np; i += kBuildThreads) {  // s >= 64: the 32 entries of a warp lie in one segment
-      const unsigned e = key[i];
-      const bool real = e != kPadKey;
-      const int id = (int)(e & kIdxMask);
-      const int seg = i / s;
+    if (active) {
+      unsigned lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};
+#pragma unroll
+      for (int h = 0; h < E; ++h) {
+        const int pos = wbase + 32 * h + lane;
+        if (pos < N) {
+          v[h] = sid[pos];
+          box_add(p, v[h], lo, hi);
+        }
+      }
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        const unsigned u = real ? hg_ord(p[(size_t)id * 3 + c]) : 0u;
-        const unsigned lo = __reduce_min_sync(0xffffffffu, real ? u : 0xffffffffu);
-        const unsigned hi = __reduce_max_sync(0xffffffffu, u);
+        lo[c] = __reduce_min_sync(0xffffffffu, lo[c]);
+        hi[c] = __reduce_max_sync(0xffffffffu, hi[c]);
         if (lane == 0) {
-          atomicMin(&smin[c][seg], lo);
-          atomicMax(&smax[c][seg], hi);
+          atomicMin(&smin[c][seg], lo[c]);
+          atomicMax(&smax[c][seg], hi[c]);
         }
       }
     }
     __syncthreads();
-    for (int t = tid; t < nseg; t += kBuildThreads) {
-      float lo[3], ext[3];
+    if (tid < nseg) {
+      unsigned lo[3], hi[3];
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        lo[c] = hg_unord(smin[c][t]);
-        ext[c] = hg_unord(smax[c][t]) - lo[c];  // NaN for a segment of padding only
+        lo[c] = smin[c][tid];
+        hi[c] = smax[c][tid];
       }
-      int ax = 0;
-      if (ext[1] > ext[ax]) ax = 1;
-      if (ext[2] > ext[ax]) ax = 2;
-      saxis[t] = ax;
-      slo[t] = lo[ax];
-      sscale[t] = ext[ax] > 0.f ? kQuantMax / ext[ax] : 0.f;
+      ssplit[tid] = seg_split(lo, hi);
+      spref[tid] = 0u;
+      srank[tid] = s / 2 - 1;
     }
     __syncthreads();
-    for (int i = tid; i < Np; i += kBuildThreads) {
-      const unsigned e = key[i];
-      if (e == kPadKey) continue;
-      const int seg = i / s, id = (int)(e & kIdxMask);
-      const float f = (p[(size_t)id * 3 + saxis[seg]] - slo[seg]) * sscale[seg];
-      key[i] = ((unsigned)fminf(fmaxf(f, 0.f), kQuantMax) << kIdxBits) | (unsigned)id;
+    // a segment with s/2 real points or fewer keeps them where they are (all in its left half)
+    const bool split = active && N - sbase > s / 2;
+    if (split) {
+      const SegSplit sp = ssplit[seg];
+#pragma unroll
+      for (int h = 0; h < E; ++h)
+        if (wbase + 32 * h + lane < N) v[h] = split_key(p, v[h], sp);
     }
-    __syncthreads();
-    // bitonic sort of every segment of s entries, all segments ascending
-    for (int k = 2; k <= s; k <<= 1)
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        for (int t = tid; t < Np / 2; t += kBuildThreads) {
-          const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1)), c = a + j;
-          const bool asc = k == s || (a & k) == 0;
-          const unsigned x = key[a], y = key[c];
-          if ((x > y) == asc) {
-            key[a] = y;
-            key[c] = x;
+    for (int shift = 24; shift >= 0; shift -= 8) {  // radix select of the rank-(s/2 - 1) key
+      if (split) {
+        const unsigned pref = spref[seg], hmask = shift == 24 ? 0u : 0xffffffffu << (shift + 8);
+#pragma unroll
+        for (int h = 0; h < E; ++h)
+          if (wbase + 32 * h + lane < N && ((v[h] ^ pref) & hmask) == 0u)
+            atomicAdd(&hist[seg][(v[h] >> shift) & 255u], 1u);
+      }
+      __syncthreads();
+      if (warp < nseg && N - warp * s > s / 2) {  // warp `warp` finds the digit of segment `warp`, clears its bins
+        const unsigned r = srank[warp];
+        unsigned cnt[8], loc = 0u;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          cnt[i] = hist[warp][lane * 8 + i];
+          hist[warp][lane * 8 + i] = 0u;
+          loc += cnt[i];
+        }
+        unsigned inc = loc;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+          const unsigned t = __shfl_up_sync(0xffffffffu, inc, d);
+          if (lane >= d) inc += t;
+        }
+        unsigned acc = inc - loc;
+        if (acc <= r && r < inc) {
+          bool found = false;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            if (!found && r < acc + cnt[i]) {
+              found = true;
+              spref[warp] |= (unsigned)(lane * 8 + i) << shift;
+              srank[warp] = r - acc;
+            }
+            acc += cnt[i];
           }
         }
-        __syncthreads();
       }
+      __syncthreads();
+    }
+    // partition: keys <= the selected one to the left half, the others after it
+    const unsigned m = split ? spref[seg] : 0u;
+    if (split) {
+      unsigned nl = 0u;
+#pragma unroll
+      for (int h = 0; h < E; ++h) nl += __popc(__ballot_sync(0xffffffffu, wbase + 32 * h + lane < N && v[h] <= m));
+      if (lane == 0) swl[warp] = nl;
+    }
+    __syncthreads();
+    if (split) {
+      unsigned before = 0u;  // left keys of the segment's earlier warps, then of earlier entries
+      for (int w = sbase / C; w < warp; ++w) before += swl[w];
+#pragma unroll
+      for (int h = 0; h < E; ++h) {
+        const int pos = wbase + 32 * h + lane;
+        const bool real = pos < N, left = real && v[h] <= m;
+        const unsigned bal = __ballot_sync(0xffffffffu, left);
+        const int lb = (int)(before + __popc(bal & ((1u << lane) - 1u)));
+        if (real) sid[left ? sbase + lb : sbase + s / 2 + (pos - sbase - lb)] = v[h] & kIdxMask;
+        before += __popc(bal);
+      }
+    }
+    __syncthreads();
   }
+  // warp-local levels: groups of G rows (32 G entries), G = E .. 2
+  if (active) {
+#pragma unroll
+    for (int h = 0; h < E; ++h) {
+      const int pos = wbase + 32 * h + lane;
+      v[h] = pos < N ? sid[pos] : kPadKey;
+    }
+    warp_levels<E, E>(p, v, lane);
+#pragma unroll
+    for (int h = 0; h < E; ++h) sid[wbase + 32 * h + lane] = v[h] & kIdxMask;
+  }
+  __syncthreads();
 
   for (int i = tid; i < N; i += kBuildThreads) {
-    const int id = (int)(key[i] & kIdxMask);
+    const int id = (int)sid[i];
     const float x = p[(size_t)id * 3], y = p[(size_t)id * 3 + 1], z = p[(size_t)id * 3 + 2];
     const float w = CHAMFER_NORM ? hg_dot3_fma(x, y, z, x, y, z) : hg_sumsq3_seq(x, y, z);
     o.pts[(size_t)b * N + i] = make_float4(x, y, z, w);
@@ -205,7 +375,7 @@ __global__ void __launch_bounds__(kBuildThreads) prune_order_kernel(const float 
     const int i = L * kLeaf + lane;
     float v[3] = {0.f, 0.f, 0.f};
     if (i < N) {
-      const int id = (int)(key[i] & kIdxMask);
+      const int id = (int)sid[i];
 #pragma unroll
       for (int c = 0; c < 3; ++c) v[c] = p[(size_t)id * 3 + c];
     }
@@ -666,10 +836,19 @@ int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, H
   }
   const size_t smem = (size_t)Np * sizeof(unsigned);
   static HgPerDeviceOnce once[2];
-  auto kernel = chamfer_norm ? prune_order_kernel<true> : prune_order_kernel<false>;
+  // entries per lane: 32 warps of Np / 32 entries from 2048 points up, else Np / 64 warps of 64
+  const int E = Np >= 32 * 64 ? Np / kBuildThreads : 2;
+  auto pick = [](bool chamfer, int e) {
+    if (chamfer) return e == 2 ? prune_order_kernel<true, 2> : e == 4 ? prune_order_kernel<true, 4>
+                      : e == 8 ? prune_order_kernel<true, 8> : prune_order_kernel<true, 16>;
+    return e == 2 ? prune_order_kernel<false, 2> : e == 4 ? prune_order_kernel<false, 4>
+           : e == 8 ? prune_order_kernel<false, 8> : prune_order_kernel<false, 16>;
+  };
+  auto kernel = pick(chamfer_norm, E);
   if (once[chamfer_norm ? 1 : 0].first())
-    HG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 HG_PRUNE_MAX_N * (int)sizeof(unsigned)));
+    for (int e = 2; e <= HG_PRUNE_MAX_N / kBuildThreads; e <<= 1)
+      HG_CUDA(cudaFuncSetAttribute(pick(chamfer_norm, e), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   HG_PRUNE_MAX_N * (int)sizeof(unsigned)));
   // with a state: the clouds the refit marked only (the others exit at entry), so no host decision is needed
   kernel<<<B, kBuildThreads, smem, stream>>>(pc, N, Np, *o, hdr, order_counters());
   HG_CHECK_LAUNCH("prune_order_kernel");
