@@ -66,6 +66,20 @@ static inline cudaStream_t hg_stream(hgStream s) { return reinterpret_cast<cudaS
 
 static inline size_t hg_align(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 
+// A workspace layout is written once, as a type constructed from (HgCarve &, arguments): take() hands out the next
+// region, rounded up to 256 bytes.  On a null base it only counts: hg_layout_bytes is the size, hg_layout_at the pointers.
+struct HgSpan { void *ptr; size_t bytes; };  // a region that a callee carves itself
+struct HgCarve {
+  char *base;
+  size_t bytes = 0;
+  explicit HgCarve(void *base_ = nullptr) : base((char *)base_) {}
+  char *here() const { return base ? base + bytes : nullptr; }
+  template <typename T> T *take(size_t n) { T *p = (T *)here(); bytes += hg_align(n * sizeof(T)); return p; }
+  HgSpan span(size_t n) { return {take<char>(n), hg_align(n)}; }
+};
+template <typename Layout, typename... A> size_t hg_layout_bytes(A... a) { HgCarve c; Layout(c, a...); return c.bytes; }
+template <typename Layout, typename... A> Layout hg_layout_at(void *base, A... a) { HgCarve c(base); return Layout(c, a...); }
+
 int hg_sm_count();
 // true the first time it is called on the current device with this flag array (function attributes such as the
 // dynamic shared-memory limit are per device: one `static` flag per process would miss the second GPU)
@@ -190,6 +204,14 @@ int hg_csr_build(const int *keys, int B, int E, int N, void *workspace, size_t w
 // hg_csr_next() to get ascending edge order (deterministic sums without a stable sort).
 int hg_csr_build_unordered(const int *keys, int B, int E, int N, void *workspace, size_t workspace_bytes, HgCsr *out,
                            cudaStream_t stream);
+// workspace of a scatter-style backward: keys [B,E], then the CSR build (stable or unordered) that groups them
+struct HgKeysCsr {
+  int *keys;
+  HgSpan csr;
+  HgKeysCsr(HgCarve &c, int B, int N, long long E, bool stable)
+      : keys(c.take<int>((size_t)B * E)),
+        csr(c.span(stable ? hg_csr_stable_workspace_bytes(B, N, (int)E) : hg_csr_workspace_bytes(B, N, (int)E))) {}
+};
 // smallest entry of list[p0..p1) that is greater than `last` (INT_MAX if none)
 __device__ __forceinline__ int hg_csr_next(const int *__restrict__ list, int p0, int p1, int last) {
   int best = 0x7fffffff;
@@ -233,7 +255,7 @@ int hg_knn3_launch_i32(int form, const float *q, const float *r, int B, int Nq, 
                        cudaStream_t stream);
 int hg_knn3_launch_i64(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals,
                        long long *idx, cudaStream_t stream);
-size_t hg_knn3_seed_workspace_bytes(int B, int N);
-int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, void *workspace,
-                            size_t workspace_bytes, cudaStream_t stream, int *idx_state = nullptr, int state_valid = 0,
-                            void *order = nullptr);
+// 3-D self-kNN (expanded form), every route: hg_knn_self_temporal_order_f32 with C = 3 (arguments checked there)
+size_t hg_knn3_self_workspace_bytes(int B, int N, int k1);
+int hg_knn3_self_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, int *idx_state, int state_valid,
+                     void *order, void *workspace, size_t workspace_bytes, cudaStream_t stream);

@@ -210,27 +210,27 @@ __global__ void __launch_bounds__(32 * W) csr_build_smem_kernel(const int *__res
 // ~20 us for 388 clouds x 6144 edges).  hg_csr_build_unordered switches on this and the workspace formula follows it.
 static inline bool csr_small(int E) { return E <= 2048; }
 
+// off [B,N+1], cursors (kCsrWarps per key for the stable builder, one for the atomic one), list [B,E]
+struct CsrLayout {
+  int *off, *cursor, *list;
+  CsrLayout(HgCarve &c, int B, int N, int E, bool stable)
+      : off(c.take<int>((size_t)B * (N + 1))), cursor(c.take<int>((size_t)B * (stable ? kCsrWarps : 1) * N)),
+        list(c.take<int>((size_t)B * E)) {}
+};
+
 size_t hg_csr_workspace_bytes(int B, int N, int E) {
-  const size_t cursors = csr_small(E) ? (size_t)kCsrWarps * N : (size_t)N;
-  return hg_align((size_t)B * (N + 1) * sizeof(int)) + hg_align((size_t)B * cursors * sizeof(int)) +
-         hg_align((size_t)B * E * sizeof(int));
+  return hg_layout_bytes<CsrLayout>(B, N, E, csr_small(E));
 }
 
 size_t hg_csr_stable_workspace_bytes(int B, int N, int E) {
-  return hg_align((size_t)B * (N + 1) * sizeof(int)) + hg_align((size_t)B * kCsrWarps * N * sizeof(int)) +
-         hg_align((size_t)B * E * sizeof(int));
+  return hg_layout_bytes<CsrLayout>(B, N, E, true);
 }
 
 int hg_csr_build(const int *keys, int B, int E, int N, void *workspace, size_t workspace_bytes, HgCsr *out,
                  cudaStream_t stream) {
   HG_REQUIRE(workspace && workspace_bytes >= hg_csr_stable_workspace_bytes(B, N, E), HG_E_WORKSPACE,
              "csr: workspace too small (%zu < %zu)", workspace_bytes, hg_csr_stable_workspace_bytes(B, N, E));
-  char *p = (char *)workspace;
-  int *off = (int *)p;
-  p += hg_align((size_t)B * (N + 1) * sizeof(int));
-  int *cursor = (int *)p;
-  p += hg_align((size_t)B * kCsrWarps * N * sizeof(int));
-  int *list = (int *)p;
+  const auto [off, cursor, list] = hg_layout_at<CsrLayout>(workspace, B, N, E, true);
   {
     // most warps whose cursors (and, if possible, the staged keys) fit in shared memory
     auto need = [&](int w, bool keys_too) {
@@ -338,12 +338,7 @@ int hg_csr_build_unordered(const int *keys, int B, int E, int N, void *workspace
   HG_REQUIRE(workspace && workspace_bytes >= hg_csr_workspace_bytes(B, N, E), HG_E_WORKSPACE,
              "csr: workspace too small (%zu < %zu)", workspace_bytes, hg_csr_workspace_bytes(B, N, E));
   if (csr_small(E)) return hg_csr_build(keys, B, E, N, workspace, workspace_bytes, out, stream);  // sorted is fine too
-  char *p = (char *)workspace;
-  int *off = (int *)p;
-  p += hg_align((size_t)B * (N + 1) * sizeof(int));
-  int *cursor = (int *)p;
-  p += hg_align((size_t)B * N * sizeof(int));
-  int *list = (int *)p;
+  const auto [off, cursor, list] = hg_layout_at<CsrLayout>(workspace, B, N, E, false);
   HG_CUDA(cudaMemsetAsync(off, 0, (size_t)B * (N + 1) * sizeof(int), stream));
   const long long total = (long long)B * E;
   long long blocks = (total + 255) / 256;

@@ -211,7 +211,7 @@ HG_API int hg_edge_feature_f32(const float *x, const int64_t *idx, int B, int C,
 
 HG_API size_t hg_edge_feature_grad_workspace_bytes(int B, int N, int k) {
   if (B <= 0 || N <= 0 || k <= 0) return 0;
-  return hg_align((size_t)B * N * k * sizeof(int)) + hg_csr_stable_workspace_bytes(B, N, N * k);
+  return hg_layout_bytes<HgKeysCsr>(B, N, (long long)N * k, true);
 }
 
 HG_API int hg_edge_feature_grad_f32(const float *grad_out, const int64_t *idx, int B, int C, int N, int k,
@@ -224,17 +224,16 @@ HG_API int hg_edge_feature_grad_f32(const float *grad_out, const int64_t *idx, i
   HG_REQUIRE(workspace && workspace_bytes >= hg_edge_feature_grad_workspace_bytes(B, N, k), HG_E_WORKSPACE,
              "edge_feature_grad: workspace too small");
   const int E = N * k;
-  int *keys = (int *)workspace;
-  void *csr_ws = (char *)workspace + hg_align((size_t)B * E * sizeof(int));
+  const auto w = hg_layout_at<HgKeysCsr>(workspace, B, N, (long long)E, true);
   const long long te = (long long)B * E;
   long long kb = (te + 255) / 256;
   if (kb > (long long)hg_sm_count() * 32) kb = (long long)hg_sm_count() * 32;
-  edge_keys_kernel<<<(int)kb, 256, 0, stream>>>((const long long *)idx, te, N, keys);
+  edge_keys_kernel<<<(int)kb, 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
   HG_CHECK_LAUNCH("edge_keys_kernel");
   HgCsr csr;
   // stable build (ascending edge order inside every segment): kNN graphs of high-dimensional features have hubs
   // with in-degrees in the hundreds, which rules out the unordered build + O(deg^2) ordered walk used elsewhere
-  int rc = hg_csr_build(keys, B, E, N, csr_ws, hg_csr_stable_workspace_bytes(B, N, E), &csr, stream);
+  int rc = hg_csr_build(w.keys, B, E, N, w.csr.ptr, w.csr.bytes, &csr, stream);
   if (rc) return rc;
   const long long planes = (long long)B * C;
   const size_t smem = ((size_t)E + (size_t)N) * sizeof(float);  // gA plane + hub queue

@@ -58,27 +58,6 @@ __global__ void knn_sumsq_kernel(const float *__restrict__ pc, long long total, 
   }
 }
 
-// 3-D clouds with long neighbour lists (DGCNN layer 1: k = 20) on the tensor-core kernel: the cloud is copied into 32-channel
-// rows (x, y, z, 0, ...: a 128-byte row is what the TMA boxes of hg_knn_tc.cu move) and the squared norms are taken with
-// the 3-D kernels' operation order.  The zero channels change nothing in the reference's FMA chain (fma(0, 0, acc) = acc),
-// so values and indices are the 3-D path's bit for bit.
-constexpr int kPadC = 32;
-__global__ void __launch_bounds__(256) knn_pad3_kernel(const float *__restrict__ pc, long long total,
-                                                       float4 *__restrict__ padded, float *__restrict__ xx) {
-  for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < total * (kPadC / 4);
-       g += (long long)gridDim.x * blockDim.x) {
-    const long long row = g / (kPadC / 4);
-    const int q = (int)(g - row * (kPadC / 4));
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (q == 0) {
-      const float x = __ldg(pc + row * 3), y = __ldg(pc + row * 3 + 1), z = __ldg(pc + row * 3 + 2);
-      v = make_float4(x, y, z, 0.f);
-      xx[row] = hg_sumsq3_seq(x, y, z);
-    }
-    padded[g] = v;
-  }
-}
-
 // dist tile: 128 rows x 128 columns per CTA, 8 x 8 per thread (columns as four packed pairs), channels consumed strictly
 // in order: every accumulator is the reference's sequential FMA chain (product of channel 0 first, then c = 1..C-1).
 // Per channel a thread reads 8 row values (two broadcast LDS.128) and 8 column values (two LDS.128) for 32 FFMA2:
@@ -583,25 +562,22 @@ int grid_for(long long total, int threads) {
 
 constexpr size_t kGenericScratchBytes = (size_t)256 << 20;
 
-}  // namespace
+// feature clouds: squared norms [B,K], then distance matrices for nb clouds (as many as kGenericScratchBytes holds, >= 1)
+struct KnnGenericWorkspace {
+  int nb;
+  float *xx, *dist;
+  KnnGenericWorkspace(HgCarve &c, int B, int K) {
+    const size_t per = (size_t)K * K, fit = kGenericScratchBytes / (per * sizeof(float));
+    nb = fit < 1 ? 1 : fit > (size_t)B ? B : (int)fit;
+    xx = c.take<float>((size_t)B * K), dist = c.take<float>(nb * per);
+  }
+};
 
-// 3-D self-kNN shapes that may take the tensor-core kernel on a padded copy (the dispatch also looks at the batch size)
-static bool knn3_pad_candidate(int K, int k1) { return k1 >= 12 && k1 <= 32 && hg_knn_tc_supported(K, kPadC, k1); }
+}  // namespace
 
 HG_API size_t hg_knn_self_workspace_bytes(int B, int K, int C, int k1) {
   if (B <= 0 || K <= 0 || C <= 0) return 0;
-  if (C == 3) {
-    size_t w = 0;
-    if (knn3_pad_candidate(K, k1))  // padded copy + squared norms for the tensor-core kernel
-      w = hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
-    const size_t order = hg_prune_order_bytes(B, K);  // kd-tree ordering of the pruned path, in the same place
-    return hg_knn3_seed_workspace_bytes(B, K) + (w > order ? w : order);
-  }
-  size_t per = (size_t)K * K * sizeof(float);
-  size_t nb = kGenericScratchBytes / per;
-  if (nb < 1) nb = 1;
-  if (nb > (size_t)B) nb = (size_t)B;
-  return hg_align((size_t)B * K * sizeof(float)) + hg_align(nb * per);
+  return C == 3 ? hg_knn3_self_workspace_bytes(B, K, k1) : hg_layout_bytes<KnnGenericWorkspace>(B, K);
 }
 
 HG_API int hg_knn_self_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, void *workspace,
@@ -627,34 +603,13 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   HG_REQUIRE(B > 0 && K > 0 && C > 0, HG_E_BADARG, "knn_self: sizes must be positive");
   HG_REQUIRE(k1 >= 1 && k1 <= 64 && k1 <= K, HG_E_BADARG, "knn_self: need 1 <= k <= min(64, K); got k=%d K=%d", k1, K);
   HG_REQUIRE(B <= 65535, HG_E_UNSUPPORTED, "knn_self: B=%d > 65535 clouds per call", B);
-  if (C == 3) {
-    // long lists on enough clouds to fill the machine: the tensor-core kernel on a 32-channel copy beats the 3-D
-    // small-cloud kernel up to ~8 CTAs per SM (k = 20, 1024 points: 16 clouds 62 against 131 us, 32: 78 / 136, 128: 221 / 236,
-    // 192: 326 / 313; 2048 points: 32 clouds 196 / 244, 96: 485 / 464); KNNDist's short lists (and its temporal state) stay 3-D
-    const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, K);
-    const size_t pad_ws = hg_align((size_t)B * K * kPadC * sizeof(float)) + hg_align((size_t)B * K * sizeof(float));
-    if (hg_prune_applies(K))  // large clouds: pruned search, whatever the list length
-      return hg_knn3_self_seeded_i32(pc, B, K, k1, vals, idx, workspace, workspace_bytes, stream, idx_state, state_valid,
-                                     order);
-    if (!idx_state && knn3_pad_candidate(K, k1) && g_hg_tune_knn_tc_off != 1 && workspace &&
-        workspace_bytes >= seed_ws + pad_ws &&
-        ((4LL * B * ((K + 127) / 128) >= hg_sm_count() && (long long)B * ((K + 127) / 128) <= 8LL * hg_sm_count()) ||
-         g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5)) {
-      float *padded = (float *)((char *)workspace + seed_ws);
-      float *xxp = (float *)((char *)padded + hg_align((size_t)B * K * kPadC * sizeof(float)));
-      const long long rows = (long long)B * K;
-      knn_pad3_kernel<<<grid_for(rows * (kPadC / 4), 256), 256, 0, stream>>>(pc, rows, (float4 *)padded, xxp);
-      HG_CHECK_LAUNCH("knn_pad3_kernel");
-      return hg_knn_tc_run(padded, xxp, B, K, kPadC, k1, vals, idx, stream);
-    }
-    return hg_knn3_self_seeded_i32(pc, B, K, k1, vals, idx, workspace, workspace_bytes, stream, idx_state, state_valid);
-  }
+  if (C == 3)
+    return hg_knn3_self_i32(pc, B, K, k1, vals, idx, idx_state, state_valid, order, workspace, workspace_bytes, stream);
   const size_t need = hg_knn_self_workspace_bytes(B, K, C, k1);
   HG_REQUIRE(workspace && workspace_bytes >= need, HG_E_WORKSPACE, "knn_self: workspace too small (%zu < %zu)",
              workspace_bytes, need);
   HG_REQUIRE((size_t)K * sizeof(float) * 4 <= 200 * 1024, HG_E_UNSUPPORTED, "knn_self: K=%d too large for C=%d path", K, C);
-  float *xx = (float *)workspace;
-  float *dist = (float *)((char *)workspace + hg_align((size_t)B * K * sizeof(float)));
+  const auto [nb, xx, dist] = hg_layout_at<KnnGenericWorkspace>(workspace, B, K);
   knn_sumsq_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, (long long)B * K, C, xx);
   HG_CHECK_LAUNCH("knn_sumsq_kernel");
   // feature clouds of DGCNN's shapes: tensor-core filter fused with the exact FP32 evaluation (hg_knn_tc.cu); everything
@@ -667,9 +622,6 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   const bool tc_fills = (k1 > 32 ? 2 : 4) * tc_ctas >= hg_sm_count() || g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5;
   if (g_hg_tune_knn_tc_off != 1 && tc_fills && hg_knn_tc_supported(K, C, k1) && (reinterpret_cast<uintptr_t>(pc) & 15) == 0)
     return hg_knn_tc_run(pc, xx, B, K, C, k1, vals, idx, stream);
-  const size_t per = (size_t)K * K * sizeof(float);
-  int nb = (int)(kGenericScratchBytes / per);
-  if (nb < 1) nb = 1;
   const bool long_list = k1 > 32;
   const size_t sel_smem = ((size_t)4 * K + (size_t)8 * knn_sel_cap(long_list)) * sizeof(float);
   if (sel_smem > 48 * 1024)
@@ -711,7 +663,7 @@ HG_API int hg_knn_outlier_fwd_f32(const float *vals, int B, int K, int k1, float
 
 HG_API size_t hg_knn_outlier_bwd_workspace_bytes(int B, int K, int k1) {
   if (B <= 0 || K <= 0 || k1 <= 0) return 0;
-  return hg_align((size_t)B * K * k1 * sizeof(int)) + hg_csr_workspace_bytes(B, K, K * k1);
+  return hg_layout_bytes<HgKeysCsr>(B, K, (long long)K * k1, false);
 }
 
 HG_API int hg_knn_outlier_bwd_f32(const float *pc, const int *idx, const float *mask, const float *g, int B, int K,
@@ -732,16 +684,15 @@ HG_API int hg_knn_outlier_bwd_f32(const float *pc, const int *idx, const float *
     HG_CHECK_LAUNCH("knn_outlier_bwd_small_kernel");
     return HG_OK;
   }
-  int *keys = (int *)workspace;
-  void *csr_ws = (char *)workspace + hg_align((size_t)B * K * k1 * sizeof(int));
+  const auto w = hg_layout_at<HgKeysCsr>(workspace, B, K, (long long)K * k1, false);
   const long long total = (long long)B * K * k1;
-  knn_bwd_keys_kernel<<<grid_for(total, 256), 256, 0, stream>>>(idx, mask, total, k1, keys);
+  knn_bwd_keys_kernel<<<grid_for(total, 256), 256, 0, stream>>>(idx, mask, total, k1, w.keys);
   HG_CHECK_LAUNCH("knn_bwd_keys_kernel");
   HgCsr csr;
-  int rc = hg_csr_build_unordered(keys, B, K * k1, K, csr_ws, hg_csr_workspace_bytes(B, K, K * k1), &csr, stream);
+  int rc = hg_csr_build_unordered(w.keys, B, K * k1, K, w.csr.ptr, w.csr.bytes, &csr, stream);
   if (rc) return rc;
-  knn_outlier_bwd_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, idx, mask, g, csr.off, csr.list, keys, B,
-                                                                              K, C, k1, grad_pc);
+  knn_outlier_bwd_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, idx, mask, g, csr.off, csr.list, w.keys,
+                                                                              B, K, C, k1, grad_pc);
   HG_CHECK_LAUNCH("knn_outlier_bwd_kernel");
   return HG_OK;
 }

@@ -950,7 +950,6 @@ int knn3_small_main(const float *pc, int B, int N, int k1, float *vals, int *idx
                     cudaStream_t stream, int *idx_state);
 
 // self-kNN of clouds that fit in shared memory: seeds (one CTA per cloud), then the deferred-drain kernel.
-// workspace: thr0 [B,N] floats, then sbound [B] stride 8.
 int knn3_small_self(const float *pc, int B, int N, int k1, float *vals, int *idx, float *thr0, float *sbound,
                     cudaStream_t stream, int *idx_state, bool state_valid) {
   if (idx_state && state_valid) {
@@ -1017,6 +1016,58 @@ int seed_grid(int N) {
   return G;
 }
 
+// 3-D clouds with long neighbour lists (DGCNN layer 1: k = 20) on the tensor-core kernel: the cloud is copied into 32-channel
+// rows (x, y, z, 0, ...: a 128-byte row is what the TMA boxes of hg_knn_tc.cu move) and the squared norms are taken with
+// the 3-D kernels' operation order.  The zero channels change nothing in the reference's FMA chain (fma(0, 0, acc) = acc),
+// so values and indices are the 3-D path's bit for bit.
+constexpr int kPadC = 32;
+__global__ void __launch_bounds__(256) knn_pad3_kernel(const float *__restrict__ pc, long long total,
+                                                       float4 *__restrict__ padded, float *__restrict__ xx) {
+  for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < total * (kPadC / 4);
+       g += (long long)gridDim.x * blockDim.x) {
+    const long long row = g / (kPadC / 4);
+    const int q = (int)(g - row * (kPadC / 4));
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (q == 0) {
+      const float x = __ldg(pc + row * 3), y = __ldg(pc + row * 3 + 1), z = __ldg(pc + row * 3 + 2);
+      v = make_float4(x, y, z, 0.f);
+      xx[row] = hg_sumsq3_seq(x, y, z);
+    }
+    padded[g] = v;
+  }
+}
+
+// shapes that may take the tensor-core kernel on a padded copy (the dispatch also looks at the batch size)
+bool knn3_pad_candidate(int N, int k1) { return k1 >= 12 && k1 <= 32 && hg_knn_tc_supported(N, kPadC, k1); }
+
+// Workspace of 3-D self-kNN: the seed area (grid cell of every point; per cloud, stride 8, the grid's origin and scale
+// and the bound on max |p|^2; thresholds; cell-sorted points; cell lists), then one region that holds either the padded
+// copy for the tensor-core kernel (counted for the shapes that may take it) or the pruned path's kd-tree ordering.
+// *_end: the bytes each route needs.
+struct Knn3SelfWorkspace {
+  int *cellid;
+  float *params, *thr0, *padded, *padded_xx;
+  float4 *sorted;
+  HgSpan cells;
+  void *order;
+  size_t seed_end, pad_end, order_end;
+  Knn3SelfWorkspace(HgCarve &c, int B, int N, int k1) {
+    const int G = seed_grid(N);
+    cellid = c.take<int>((size_t)B * N);
+    params = c.take<float>((size_t)B * 8);
+    thr0 = c.take<float>((size_t)B * N);
+    sorted = c.take<float4>((size_t)B * N);
+    cells = c.span(hg_csr_workspace_bytes(B, G * G * G, N));
+    HgCarve pad(c.here()), ord(c.here());
+    padded = pad.take<float>((size_t)B * N * kPadC);
+    padded_xx = pad.take<float>((size_t)B * N);
+    order = ord.span(hg_prune_order_bytes(B, N)).ptr;
+    seed_end = c.bytes, pad_end = seed_end + pad.bytes, order_end = seed_end + ord.bytes;
+    const size_t shared = knn3_pad_candidate(N, k1) ? pad.bytes : 0;
+    c.take<char>(shared > ord.bytes ? shared : ord.bytes);
+  }
+};
+
 }  // namespace
 
 int hg_knn3_launch_i32(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, int *idx,
@@ -1033,12 +1084,7 @@ int hg_knn3_launch_i64(int form, const float *q, const float *r, int B, int Nq, 
              : launch_form<HG_KNN_FORM_DIRECT, long long>(q, r, B, Nq, Nr, k1, vals, idx, nullptr, nullptr, stream);
 }
 
-size_t hg_knn3_seed_workspace_bytes(int B, int N) {
-  const int G = seed_grid(N);
-  return hg_align((size_t)B * N * sizeof(int)) + hg_align((size_t)B * 8 * sizeof(float)) +
-         hg_align((size_t)B * N * sizeof(float)) + hg_align((size_t)B * N * sizeof(float4)) +
-         hg_csr_workspace_bytes(B, G * G * G, N);
-}
+size_t hg_knn3_self_workspace_bytes(int B, int N, int k1) { return hg_layout_bytes<Knn3SelfWorkspace>(B, N, k1); }
 
 // Benchmark-only overrides: the smallest cloud that gets grid-seeded thresholds (0 = default) and the seed scan's
 // neighbourhood (0 = automatic, 1 = 2x2x2 cells, 2 = 3x3x3 cells).
@@ -1055,75 +1101,75 @@ HG_API void hg_knn_force_shape(int qt, int gp) {
 
 HG_API void hg_knn_tune_small(int small_max_n) { g_small_max_n = small_max_n; }
 
-// self-kNN (expanded form) with seeded thresholds; falls back to the unseeded launch when there is no workspace.
+// Self-kNN (expanded form) of 3-D clouds.  Routes by precedence: pruned search, tensor-core kernel on a padded copy,
+// unseeded all-pairs kernel, small-cloud kernel, then the streaming kernel with the 4-operation folded filter seeded
+// from the previous call's neighbours, from a bound alone or from the grid pre-pass.
 // idx_state (optional, [B,N,k1]): the neighbour indices of the previous call on a nearby cloud -- read as temporal
 // seeds when state_valid, and overwritten with this call's indices (a second copy of idx).
-// order (optional): an ordering state for the pruned path (hg_order_state_bytes), refit instead of rebuilt.
-int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, void *workspace,
-                            size_t workspace_bytes, cudaStream_t stream, int *idx_state, int state_valid, void *order) {
-  const size_t seed_ws = hg_knn3_seed_workspace_bytes(B, N);
-  if (hg_prune_applies(N) && workspace != nullptr && workspace_bytes >= seed_ws + hg_prune_order_bytes(B, N)) {
+int hg_knn3_self_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, int *idx_state, int state_valid,
+                     void *order, void *workspace, size_t workspace_bytes, cudaStream_t stream) {
+  const auto w = hg_layout_at<Knn3SelfWorkspace>(workspace, B, N, k1);
+  if (hg_prune_applies(N) && workspace != nullptr && workspace_bytes >= w.order_end) {
     // large clouds: kd-tree ordering and pruned search (hg_prune.cu), seeded from each query's own leaf or, with
     // temporal seeds, from the previous call's neighbours; clouds the ordering flags (non-finite coordinates) then
     // take the all-pairs kernel with the reference arithmetic
-    float *sb = (float *)((char *)workspace + hg_align((size_t)B * N * sizeof(int)));
-    float *thr = (float *)((char *)sb + hg_align((size_t)B * 8 * sizeof(float)));
     const float *thr0 = nullptr;
     if (idx_state && state_valid && k1 <= 32) {  // (the seed kernel bounds at most 32 previous neighbours)
-      int rc = launch_seed_prev(pc, B, N, k1, idx_state, thr, sb, stream);
+      int rc = launch_seed_prev(pc, B, N, k1, idx_state, w.thr0, w.params, stream);
       if (rc) return rc;
-      thr0 = thr;
+      thr0 = w.thr0;
     }
     HgPruneOrder o;
     const bool prof = hg_prof_begin(HG_PROF_KNN, stream);
-    int rc = hg_prune_build(pc, B, N, false, (char *)workspace + seed_ws, &o, stream, order);
+    int rc = hg_prune_build(pc, B, N, false, w.order, &o, stream, order);
     if (!rc) rc = hg_prune_knn_search(o, B, k1, thr0, vals, idx, idx_state, stream);
     hg_prof_end(HG_PROF_KNN, stream, prof);
     if (rc) return rc;
     return launch_form<HG_KNN_FORM_EXPANDED, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, nullptr, stream, idx_state,
                                                   o.info);
   }
-  if (k1 > 32 || workspace == nullptr || workspace_bytes < hg_knn3_seed_workspace_bytes(B, N))
+  // long lists on enough clouds to fill the machine: the tensor-core kernel on a 32-channel copy beats the 3-D
+  // small-cloud kernel up to ~8 CTAs per SM (k = 20, 1024 points: 16 clouds 62 against 131 us, 32: 78 / 136, 128: 221 / 236,
+  // 192: 326 / 313; 2048 points: 32 clouds 196 / 244, 96: 485 / 464); KNNDist's short lists (and its temporal state) stay 3-D
+  if (!hg_prune_applies(N) && !idx_state && knn3_pad_candidate(N, k1) && g_hg_tune_knn_tc_off != 1 && workspace &&
+      workspace_bytes >= w.pad_end &&
+      ((4LL * B * ((N + 127) / 128) >= hg_sm_count() && (long long)B * ((N + 127) / 128) <= 8LL * hg_sm_count()) ||
+       g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5)) {
+    const long long rows = (long long)B * N, blocks = (rows * (kPadC / 4) + 255) / 256, cap = 16LL * hg_sm_count();
+    knn_pad3_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, stream>>>(pc, rows, (float4 *)w.padded, w.padded_xx);
+    HG_CHECK_LAUNCH("knn_pad3_kernel");
+    return hg_knn_tc_run(w.padded, w.padded_xx, B, N, kPadC, k1, vals, idx, stream);
+  }
+  if (k1 > 32 || workspace == nullptr || workspace_bytes < w.seed_end)
     return launch_form<HG_KNN_FORM_EXPANDED, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, nullptr, stream, idx_state);
-  float *sb_slot = (float *)((char *)workspace + hg_align((size_t)B * N * sizeof(int)));  // `params`: [B] stride 8
-  float *thr_slot = (float *)((char *)sb_slot + hg_align((size_t)B * 8 * sizeof(float)));  // `thr0`: [B,N]
   // (tools/debug/knn_mid_sweep.py, B200, k+1 = 6: 2048 points 209 against 311 us streaming, 3000: 317 / 403, 4096: 444 / 458,
   // 8192: 1237 / 688)
   const int small_max = g_small_max_n > 0 ? (g_small_max_n < 8192 ? g_small_max_n : 8192) : (g_small_max_n < 0 ? -1 : 4096);
   if (N <= small_max)  // clouds that fit in shared memory: deferred-drain kernel
-    return knn3_small_self(pc, B, N, k1, vals, idx, thr_slot, sb_slot, stream, idx_state, state_valid != 0);
+    return knn3_small_self(pc, B, N, k1, vals, idx, w.thr0, w.params, stream, idx_state, state_valid != 0);
   if (idx_state && state_valid) {  // temporal seeds instead of the grid pre-pass
-    int rc = launch_seed_prev(pc, B, N, k1, idx_state, thr_slot, sb_slot, stream);
+    int rc = launch_seed_prev(pc, B, N, k1, idx_state, w.thr0, w.params, stream);
     if (rc) return rc;
-    return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, thr_slot, sb_slot, stream, idx_state);
+    return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, w.thr0, w.params, stream, idx_state);
   }
   if (N < (g_seed_min_n > 0 ? g_seed_min_n : 2048)) {
     // (benchmark-only, when the small-cloud path is switched off) cold thresholds with the 4-operation folded filter
-    knn_bound_kernel<<<B, 256, 0, stream>>>(pc, N, sb_slot);
+    knn_bound_kernel<<<B, 256, 0, stream>>>(pc, N, w.params);
     HG_CHECK_LAUNCH("knn_bound_kernel");
-    return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, sb_slot, stream, idx_state);
+    return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, nullptr, w.params, stream, idx_state);
   }
   const int G = seed_grid(N), ncell = G * G * G;
-  char *w = (char *)workspace;
-  int *cellid = (int *)w;
-  w += hg_align((size_t)B * N * sizeof(int));
-  float *params = (float *)w;
-  w += hg_align((size_t)B * 8 * sizeof(float));
-  float *thr0 = (float *)w;
-  w += hg_align((size_t)B * N * sizeof(float));
-  float4 *sorted = (float4 *)w;
-  w += hg_align((size_t)B * N * sizeof(float4));
-  knn_cells_kernel<<<B, 256, 0, stream>>>(pc, N, G, cellid, params);
+  knn_cells_kernel<<<B, 256, 0, stream>>>(pc, N, G, w.cellid, w.params);
   HG_CHECK_LAUNCH("knn_cells_kernel");
   HgCsr csr;
-  int rc = hg_csr_build_unordered(cellid, B, N, ncell, w, hg_csr_workspace_bytes(B, ncell, N), &csr, stream);
+  int rc = hg_csr_build_unordered(w.cellid, B, N, ncell, w.cells.ptr, w.cells.bytes, &csr, stream);
   if (rc) return rc;
   {
     const long long total = (long long)B * N;
     long long blocks = (total + 255) / 256;
     const long long cap = (long long)hg_sm_count() * 16;
     if (blocks > cap) blocks = cap;
-    knn_cell_sort_kernel<<<(int)blocks, 256, 0, stream>>>(pc, csr.list, total, N, sorted);
+    knn_cell_sort_kernel<<<(int)blocks, 256, 0, stream>>>(pc, csr.list, total, N, w.sorted);
     HG_CHECK_LAUNCH("knn_cell_sort_kernel");
   }
   dim3 grid((N + 127) / 128, B);
@@ -1132,12 +1178,12 @@ int hg_knn3_self_seeded_i32(const float *pc, int B, int N, int k1, float *vals, 
   // ~24 points of 8 cells cannot fill (tools/knn_seed_sweep.py)
   const int near8 = g_seed_near8 == 1 ? 1 : g_seed_near8 == 2 ? 0 : (k1 <= 20);
   if (k1 <= 6)
-    knn_seed_kernel<6><<<grid, 128, 0, stream>>>(sorted, N, G, params, csr.off, csr.list, thr0, near8);
+    knn_seed_kernel<6><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
   else if (k1 <= 20)
-    knn_seed_kernel<20><<<grid, 128, 0, stream>>>(sorted, N, G, params, csr.off, csr.list, thr0, near8);
+    knn_seed_kernel<20><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
   else
-    knn_seed_kernel<32><<<grid, 128, 0, stream>>>(sorted, N, G, params, csr.off, csr.list, thr0, near8);
+    knn_seed_kernel<32><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
   HG_CHECK_LAUNCH("knn_seed_kernel");
   // seeded path: the bounding box is known, so the main loop can run the 4-operation folded filter
-  return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, thr0, params + 6, stream, idx_state);
+  return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, w.thr0, w.params + 6, stream, idx_state);
 }

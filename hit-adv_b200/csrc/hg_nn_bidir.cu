@@ -967,17 +967,31 @@ HG_API void hg_nn_bidir_tune(int T, int RB) {
   g_force_RB = RB;
 }
 
-// merged (value, cell) keys, runner-up values, per-cloud error bound, ambiguity list
-static size_t nn_d3_bytes(int B, int N2, int N1) {
-  return hg_align((size_t)B * N1 * 8) + hg_align((size_t)B * N2 * 8) + hg_align((size_t)B * N1 * 4) +
-         hg_align((size_t)B * N2 * 4) + hg_align((size_t)B * 4) + hg_align(((size_t)B * (N1 + N2) + 1) * 4);
-}
+// D = 3: merged (value, cell) keys and runner-up values (the part each call resets to 0xff), per-cloud error bound,
+// ambiguity list, then the kd-tree orderings of both clouds (0 bytes where the pruned path does not apply)
+struct NnD3Workspace {
+  float *eps2;
+  void *gts_order, *preds_order;
+  NnD3Workspace(HgCarve &c, int B, int N2, int N1, NnParams *p) {
+    p->colres = c.take<unsigned long long>((size_t)B * N1);
+    p->rowres = c.take<unsigned long long>((size_t)B * N2);
+    p->colsec = c.take<unsigned>((size_t)B * N1);
+    p->rowsec = c.take<unsigned>((size_t)B * N2);
+    p->eps2 = eps2 = c.take<float>(B);
+    p->amb = c.take<int>((size_t)B * (N1 + N2) + 1);
+    gts_order = c.span(hg_prune_order_bytes(B, N2)).ptr;
+    preds_order = c.span(hg_prune_order_bytes(B, N1)).ptr;
+  }
+};
+struct NnGenericWorkspace {  // other D: P [B,N2,N1]
+  float *P;
+  NnGenericWorkspace(HgCarve &c, int B, int N2, int N1) : P(c.take<float>((size_t)B * N2 * N1)) {}
+};
 
 HG_API size_t hg_nn_bidir_workspace_bytes(int B, int N2, int N1, int D) {
   if (B <= 0 || N1 <= 0 || N2 <= 0 || D <= 0) return 0;
-  if (D == 3)  // + the kd-tree orderings of both clouds when the pruned path applies
-    return nn_d3_bytes(B, N2, N1) + hg_prune_order_bytes(B, N2) + hg_prune_order_bytes(B, N1);
-  return hg_align((size_t)B * N2 * N1 * sizeof(float));
+  NnParams p;
+  return D == 3 ? hg_layout_bytes<NnD3Workspace>(B, N2, N1, &p) : hg_layout_bytes<NnGenericWorkspace>(B, N2, N1);
 }
 
 HG_API int hg_nn_bidir_f32(const float *gts, const float *preds, int B, int N2, int N1, int D, float *min1, int *arg1,
@@ -1006,7 +1020,7 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
   if (D != 3) {
     HG_REQUIRE((double)B * N2 * N1 <= 2.0e9, HG_E_UNSUPPORTED,
                "nn_bidir: generic-D path materialises P; B*N2*N1 too large");
-    float *P = (float *)workspace;
+    float *P = hg_layout_at<NnGenericWorkspace>(workspace, B, N2, N1).P;
     const long long total = (long long)B * N2 * N1;
     nn_generic_p_kernel<<<grid_for(total, 256), 256, 0, stream>>>(gts, preds, B, N2, N1, D, P);
     HG_CHECK_LAUNCH("nn_generic_p_kernel");
@@ -1020,30 +1034,16 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
   p.preds = preds;
   p.N2 = N2;
   p.N1 = N1;
-  char *w = (char *)workspace;
-  p.colres = (unsigned long long *)w;
-  w += hg_align((size_t)B * N1 * 8);
-  p.rowres = (unsigned long long *)w;
-  w += hg_align((size_t)B * N2 * 8);
-  p.colsec = (unsigned *)w;
-  w += hg_align((size_t)B * N1 * 4);
-  p.rowsec = (unsigned *)w;
-  w += hg_align((size_t)B * N2 * 4);
-  float *eps2 = (float *)w;
-  p.eps2 = eps2;
-  w += hg_align((size_t)B * 4);
-  p.amb = (int *)w;
+  const auto w = hg_layout_at<NnD3Workspace>(workspace, B, N2, N1, &p);
   p.only_a = p.only_b = nullptr;
   // large clouds: kd-tree orderings and pruned 1-NN passes in both directions (hg_prune.cu); the all-pairs kernels below
   // then run on the clouds the ordering build flagged (non-finite coordinates) only
-  const bool prune = hg_prune_applies(N1) && hg_prune_applies(N2) &&
-                     workspace_bytes >= nn_d3_bytes(B, N2, N1) + hg_prune_order_bytes(B, N2) + hg_prune_order_bytes(B, N1);
+  const bool prune = hg_prune_applies(N1) && hg_prune_applies(N2);
   if (prune) {
-    char *ow = (char *)workspace + nn_d3_bytes(B, N2, N1);
     HgPruneOrder og, op;
     const bool prof = hg_prof_begin(HG_PROF_NN_BIDIR, stream);
-    int rc = hg_prune_build(gts, B, N2, true, ow, &og, stream, gts_order);
-    if (!rc) rc = hg_prune_build(preds, B, N1, true, ow + hg_prune_order_bytes(B, N2), &op, stream, preds_order);
+    int rc = hg_prune_build(gts, B, N2, true, w.gts_order, &og, stream, gts_order);
+    if (!rc) rc = hg_prune_build(preds, B, N1, true, w.preds_order, &op, stream, preds_order);
     if (!rc) rc = hg_prune_nn_search(op, og, B, min1, arg1, stream);  // column j (preds): nearest row (gts)
     if (!rc) rc = hg_prune_nn_search(og, op, B, min2, arg2, stream);  // row i (gts): nearest column (preds)
     hg_prof_end(HG_PROF_NN_BIDIR, stream, prof);
@@ -1053,10 +1053,10 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
   }
   // the approximate tracker (4 FMA-pipe operations per pair, exact recovery in the finish kernels) when switched on
   const bool approx = !prune && !g_hg_tune_nn_exact && (double)B * (N1 + N2) < 2.0e9;
-  HG_CUDA(cudaMemsetAsync(workspace, 0xff, (size_t)((char *)eps2 - (char *)workspace), stream));
+  HG_CUDA(cudaMemsetAsync(workspace, 0xff, (size_t)((char *)w.eps2 - (char *)workspace), stream));
   if (approx) {
     HG_CUDA(cudaMemsetAsync(p.amb, 0, sizeof(int), stream));
-    nn_eps_kernel<<<B, 256, 0, stream>>>(gts, preds, N2, N1, eps2);
+    nn_eps_kernel<<<B, 256, 0, stream>>>(gts, preds, N2, N1, w.eps2);
     HG_CHECK_LAUNCH("nn_eps_kernel");
   }
 
@@ -1137,10 +1137,16 @@ HG_API int hg_set_loss_f32(const float *min1, const float *min2, int B, int N1, 
   return HG_OK;
 }
 
+// reverse map of arg2 (N2 edges -> N1 keys), then of arg1 (N1 edges -> N2 keys)
+struct SetLossBwdWorkspace {
+  HgSpan rev2, rev1;
+  SetLossBwdWorkspace(HgCarve &c, int B, int N2, int N1)
+      : rev2(c.span(hg_csr_workspace_bytes(B, N1, N2))), rev1(c.span(hg_csr_workspace_bytes(B, N2, N1))) {}
+};
+
 HG_API size_t hg_set_loss_bwd_workspace_bytes(int B, int N2, int N1) {
   if (B <= 0 || N1 <= 0 || N2 <= 0) return 0;
-  // reverse map of arg2 (N2 edges -> N1 keys) and of arg1 (N1 edges -> N2 keys)
-  return hg_csr_workspace_bytes(B, N1, N2) + hg_csr_workspace_bytes(B, N2, N1);
+  return hg_layout_bytes<SetLossBwdWorkspace>(B, N2, N1);
 }
 
 HG_API int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *arg1, const int *arg2,
@@ -1156,13 +1162,14 @@ HG_API int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *
              "set_loss_bwd: bad mode / missing hausdorff arg-max indices");
   HG_REQUIRE(workspace && workspace_bytes >= hg_set_loss_bwd_workspace_bytes(B, N2, N1), HG_E_WORKSPACE,
              "set_loss_bwd: workspace too small");
+  const auto w = hg_layout_at<SetLossBwdWorkspace>(workspace, B, N2, N1);
   // preds (adv, "y"): gathers through arg1 (loss1), receives scatter from arg2 (loss2)
   HgCsr rev2;
   int rc = HG_OK;
   rev2.off = nullptr;
   rev2.list = nullptr;
   if (g2) {  // loss2 scatters into preds through arg2; unused (g2 == NULL) => no reverse map at all
-    rc = hg_csr_build_unordered(arg2, B, N2, N1, workspace, hg_csr_workspace_bytes(B, N1, N2), &rev2, stream);
+    rc = hg_csr_build_unordered(arg2, B, N2, N1, w.rev2.ptr, w.rev2.bytes, &rev2, stream);
     if (rc) return rc;
   }
   const long long tp = (long long)B * N1 * (D > 8 ? D : 1);
@@ -1171,11 +1178,10 @@ HG_API int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *
   HG_CHECK_LAUNCH("set_loss_bwd_kernel(preds)");
   if (grad_gts) {
     HgCsr rev1;
-    void *ws2 = (char *)workspace + hg_csr_workspace_bytes(B, N1, N2);
     rev1.off = nullptr;
     rev1.list = nullptr;
     if (g1) {
-      rc = hg_csr_build_unordered(arg1, B, N1, N2, ws2, hg_csr_workspace_bytes(B, N2, N1), &rev1, stream);
+      rc = hg_csr_build_unordered(arg1, B, N1, N2, w.rev1.ptr, w.rev1.bytes, &rev1, stream);
       if (rc) return rc;
     }
     const long long tg = (long long)B * N2 * (D > 8 ? D : 1);

@@ -749,10 +749,19 @@ unsigned long long *order_counters() {
   return (unsigned long long *)ptr;
 }
 
-// the state's header (one float4 per cloud) follows the permutations
-float4 *state_header(void *state, int B, int N) {
-  return (float4 *)((char *)state + hg_align((size_t)B * N * sizeof(int)));
-}
+// an ordering in the workspace: points, permutation (unused with an ordering state), leaf boxes, per-cloud info
+struct OrderLayout : HgPruneOrder {
+  OrderLayout(HgCarve &c, int B, int N)
+      : HgPruneOrder{c.take<float4>((size_t)B * N), c.take<int>((size_t)B * N),
+                     c.take<float4>((size_t)B * ((N + kLeaf - 1) / kLeaf) * 2), c.take<float4>(B), N} {}
+};
+
+// an ordering state: the permutations, then the header (one float4 per cloud)
+struct StateLayout {
+  int *perm;
+  float4 *hdr;
+  StateLayout(HgCarve &c, int B, int N) : perm(c.take<int>((size_t)B * N)), hdr(c.take<float4>(B)) {}
+};
 
 }  // namespace
 
@@ -793,31 +802,22 @@ bool hg_prune_applies(int N) {
 
 size_t hg_prune_order_bytes(int B, int N) {
   if (B <= 0 || !hg_prune_applies(N)) return 0;
-  const size_t nleaf = (size_t)(N + kLeaf - 1) / kLeaf;
-  return hg_align((size_t)B * N * sizeof(float4)) + hg_align((size_t)B * N * sizeof(int)) +
-         hg_align((size_t)B * nleaf * 2 * sizeof(float4)) + hg_align((size_t)B * sizeof(float4));
+  return hg_layout_bytes<OrderLayout>(B, N);
 }
 
 HG_API size_t hg_order_state_bytes(int B, int N) {
   if (B <= 0 || N <= 0) return 0;
-  return hg_align((size_t)B * N * sizeof(int)) + hg_align((size_t)B * sizeof(float4));
+  return hg_layout_bytes<StateLayout>(B, N);
 }
 
 int hg_prune_build(const float *pc, int B, int N, bool chamfer_norm, void *ws, HgPruneOrder *o, cudaStream_t stream,
                    void *state) {
-  const size_t nleaf = (size_t)(N + kLeaf - 1) / kLeaf;
-  char *w = (char *)ws;
-  o->N = N;
-  o->pts = (float4 *)w;
-  w += hg_align((size_t)B * N * sizeof(float4));
-  o->perm = state ? (int *)state : (int *)w;  // with a state, the permutation lives there (the workspace slot is unused)
-  w += hg_align((size_t)B * N * sizeof(int));
-  o->box = (float4 *)w;
-  w += hg_align((size_t)B * nleaf * 2 * sizeof(float4));
-  o->info = (float4 *)w;
+  *o = hg_layout_at<OrderLayout>(ws, B, N);
+  const StateLayout s = hg_layout_at<StateLayout>(state, B, N);  // null pointers without a state
+  float4 *hdr = s.hdr;
+  if (state) o->perm = s.perm;  // with a state, the permutation lives there (the workspace slot is unused)
   int Np = 2 * kLeaf;
   while (Np < N) Np <<= 1;
-  float4 *hdr = state ? state_header(state, B, N) : nullptr;
   if (state) {
     const bool stage = g_refit_stage == 0 ? kRefitDefaultStage : g_refit_stage == 1;
     const float tol = (g_refit_tol > 0 ? g_refit_tol : kRefitDefaultTolPermille) * 1e-3f;

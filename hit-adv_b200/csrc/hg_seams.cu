@@ -267,7 +267,7 @@ HG_API int hg_index_points_f32(const float *points, const int64_t *idx, int B, i
 
 HG_API size_t hg_index_points_grad_workspace_bytes(int B, int N, int M) {
   if (B <= 0 || N <= 0 || M <= 0) return 0;
-  return hg_align((size_t)B * M * sizeof(int)) + hg_csr_stable_workspace_bytes(B, N, M);
+  return hg_layout_bytes<HgKeysCsr>(B, N, (long long)M, true);
 }
 
 HG_API int hg_index_points_grad_f32(const float *grad_out, const int64_t *idx, int B, int N, int C, int M,
@@ -278,13 +278,12 @@ HG_API int hg_index_points_grad_f32(const float *grad_out, const int64_t *idx, i
   HG_REQUIRE(B > 0 && N > 0 && C > 0 && M > 0, HG_E_BADARG, "index_points_grad: sizes must be positive");
   HG_REQUIRE(workspace && workspace_bytes >= hg_index_points_grad_workspace_bytes(B, N, M), HG_E_WORKSPACE,
              "index_points_grad: workspace too small");
-  int *keys = (int *)workspace;
-  void *csr_ws = (char *)workspace + hg_align((size_t)B * M * sizeof(int));
+  const auto w = hg_layout_at<HgKeysCsr>(workspace, B, N, (long long)M, true);
   const long long te = (long long)B * M;
-  idx64_to_keys_kernel<<<grid_for(te, 256), 256, 0, stream>>>((const long long *)idx, te, N, keys);
+  idx64_to_keys_kernel<<<grid_for(te, 256), 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
   HG_CHECK_LAUNCH("idx64_to_keys");
   HgCsr csr;
-  int rc = hg_csr_build(keys, B, M, N, csr_ws, hg_csr_stable_workspace_bytes(B, N, M), &csr, stream);
+  int rc = hg_csr_build(w.keys, B, M, N, w.csr.ptr, w.csr.bytes, &csr, stream);
   if (rc) return rc;
   const long long total = (long long)B * N * C;
   index_points_grad_kernel<<<grid_for(total, 256), 256, 0, stream>>>(grad_out, csr.off, csr.list, B, N, C, M,
