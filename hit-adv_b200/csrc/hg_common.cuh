@@ -224,6 +224,7 @@ __device__ __forceinline__ int hg_csr_next(const int *__restrict__ list, int p0,
 
 // ---- tensor-core kNN prefilter for feature clouds (hg_knn_tc.cu) ---------------------------------------------------
 bool hg_knn_tc_supported(int K, int C, int k1);
+bool hg_knn_tc_supported_feature(int K, int C, int k1);
 int hg_knn_tc_run(const float *pc, const float *xx, int B, int K, int C, int k1, float *vals, int *idx, cudaStream_t stream);
 
 // ---- spatially pruned exact passes for large clouds (hg_prune.cu) ---------------------------------------------------

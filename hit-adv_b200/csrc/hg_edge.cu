@@ -18,12 +18,13 @@ namespace {
 
 // ---- forward: a CTA pass covers kEdgeCP channels of one cloud: their N source values are staged in shared memory
 // and every index load (the expensive part: 8 B per edge, L2) serves kEdgeCP x 2 output rows ----------------------
-constexpr int kEdgeCP = 4;
-template <bool VEC4>
+// Larger clouds stage fewer planes per pass (kEdgeCP = 2 up to 25600 points, 1 up to 51200); beyond that the pass reads
+// its four planes from x through L2 (STAGED = false), as the backward's unstaged variant does.
+template <int kEdgeCP, bool STAGED, bool VEC4>
 __global__ void __launch_bounds__(256) edge_feature_kernel(const float *__restrict__ x,
                                                            const long long *__restrict__ idx, int C, int N, int k,
                                                            long long groups, float *__restrict__ out) {
-  extern __shared__ float plane[];  // [kEdgeCP][N]
+  extern __shared__ float smem_planes[];  // STAGED: [kEdgeCP][N]
   const int E = N * k;
   const int gpc = (C + kEdgeCP - 1) / kEdgeCP;  // channel groups per cloud
   for (long long gi = blockIdx.y; gi < groups; gi += gridDim.y) {
@@ -31,9 +32,12 @@ __global__ void __launch_bounds__(256) edge_feature_kernel(const float *__restri
     const int c0 = (int)(gi % gpc) * kEdgeCP;
     const int nc = min(kEdgeCP, C - c0);
     const long long *id = idx + (size_t)b * E;
-    __syncthreads();
-    for (int i = threadIdx.x; i < nc * N; i += 256) plane[i] = __ldg(x + ((size_t)b * C + c0) * N + i);
-    __syncthreads();
+    const float *plane = STAGED ? smem_planes : x + ((size_t)b * C + c0) * N;
+    if (STAGED) {
+      __syncthreads();
+      for (int i = threadIdx.x; i < nc * N; i += 256) smem_planes[i] = __ldg(x + ((size_t)b * C + c0) * N + i);
+      __syncthreads();
+    }
     float *dstA = out + ((size_t)b * 2 * C + c0) * E;
     float *dstB = dstA + (size_t)C * E;
     if (VEC4) {  // k % 4 == 0: the four edges of a float4 share their centre point
@@ -61,8 +65,9 @@ __global__ void __launch_bounds__(256) edge_feature_kernel(const float *__restri
         const long long ii = id[e];
         const int n = e / k;
         for (int q = 0; q < nc; ++q) {
-          const float ctr = plane[q * N + n];
-          dstA[(size_t)q * E + e] = plane[q * N + ii] - ctr;
+          // unstaged, N may reach 2^31 / k, so q * N is taken in 64 bits (staged, q * N < 51200 * 4)
+          const float ctr = STAGED ? plane[q * N + n] : plane[(size_t)q * N + n];
+          dstA[(size_t)q * E + e] = (STAGED ? plane[q * N + ii] : plane[(size_t)q * N + ii]) - ctr;
           dstB[(size_t)q * E + e] = ctr;
         }
       }
@@ -171,18 +176,10 @@ __global__ void __launch_bounds__(kGradThreads) edge_feature_grad_kernel(const f
   }
 }
 
-}  // namespace
+constexpr size_t kEdgeStageBytes = 200 * 1024;  // shared memory a forward CTA may stage its planes in
 
-// dgcnn_cls.py:16-43 (feature build only; the neighbour search is hg_knn_self_f32 / model_seams.knn)
-HG_API int hg_edge_feature_f32(const float *x, const int64_t *idx, int B, int C, int N, int k, float *out,
-                               hgStream stream_) {
-  HG_NVTX_RANGE("hg_edge_feature_f32");
-  cudaStream_t stream = hg_stream(stream_);
-  HG_REQUIRE(x && idx && out, HG_E_BADARG, "edge_feature: null pointer");
-  HG_REQUIRE(B > 0 && C > 0 && N > 0 && k > 0, HG_E_BADARG, "edge_feature: sizes must be positive");
-  HG_REQUIRE((long long)N * k < (1LL << 31), HG_E_UNSUPPORTED, "edge_feature: N*k too large");
-  HG_REQUIRE((size_t)kEdgeCP * N * sizeof(float) <= 200 * 1024, HG_E_UNSUPPORTED,
-             "edge_feature: N=%d too large for the staged planes", N);
+template <int kEdgeCP, bool STAGED>
+int edge_feature_launch(const float *x, const int64_t *idx, int B, int C, int N, int k, float *out, cudaStream_t stream) {
   const long long groups = (long long)B * ((C + kEdgeCP - 1) / kEdgeCP);
   const int E = N * k;
   const bool vec = (k % 4 == 0) && ((reinterpret_cast<uintptr_t>(idx) | reinterpret_cast<uintptr_t>(out)) % 16 == 0);
@@ -193,20 +190,37 @@ HG_API int hg_edge_feature_f32(const float *x, const int64_t *idx, int B, int C,
   if (gx_cap < 1) gx_cap = 1;
   if (gx > gx_cap) gx = gx_cap;
   const int gy = (int)(groups < 65535 ? groups : 65535);
-  const size_t smem = (size_t)kEdgeCP * N * sizeof(float);
+  const size_t smem = STAGED ? (size_t)kEdgeCP * N * sizeof(float) : 0;
   const bool prof = hg_prof_begin(HG_PROF_GROUP, stream);
   if (vec) {
     if (smem > 48 * 1024)
-      HG_CUDA(cudaFuncSetAttribute(edge_feature_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    edge_feature_kernel<true><<<dim3(gx, gy), 256, smem, stream>>>(x, (const long long *)idx, C, N, k, groups, out);
+      HG_CUDA((cudaFuncSetAttribute(edge_feature_kernel<kEdgeCP, STAGED, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)));
+    edge_feature_kernel<kEdgeCP, STAGED, true><<<dim3(gx, gy), 256, smem, stream>>>(x, (const long long *)idx, C, N, k, groups, out);
   } else {
     if (smem > 48 * 1024)
-      HG_CUDA(cudaFuncSetAttribute(edge_feature_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    edge_feature_kernel<false><<<dim3(gx, gy), 256, smem, stream>>>(x, (const long long *)idx, C, N, k, groups, out);
+      HG_CUDA((cudaFuncSetAttribute(edge_feature_kernel<kEdgeCP, STAGED, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)));
+    edge_feature_kernel<kEdgeCP, STAGED, false><<<dim3(gx, gy), 256, smem, stream>>>(x, (const long long *)idx, C, N, k, groups, out);
   }
   hg_prof_end(HG_PROF_GROUP, stream, prof);
   HG_CHECK_LAUNCH("edge_feature_kernel");
   return HG_OK;
+}
+
+}  // namespace
+
+// dgcnn_cls.py:16-43 (feature build only; the neighbour search is hg_knn_self_f32 / model_seams.knn)
+HG_API int hg_edge_feature_f32(const float *x, const int64_t *idx, int B, int C, int N, int k, float *out,
+                               hgStream stream_) {
+  HG_NVTX_RANGE("hg_edge_feature_f32");
+  cudaStream_t stream = hg_stream(stream_);
+  HG_REQUIRE(x && idx && out, HG_E_BADARG, "edge_feature: null pointer");
+  HG_REQUIRE(B > 0 && C > 0 && N > 0 && k > 0, HG_E_BADARG, "edge_feature: sizes must be positive");
+  HG_REQUIRE((long long)N * k < (1LL << 31), HG_E_UNSUPPORTED, "edge_feature: N*k too large");
+  const size_t plane = (size_t)N * sizeof(float);
+  if (4 * plane <= kEdgeStageBytes) return edge_feature_launch<4, true>(x, idx, B, C, N, k, out, stream);
+  if (2 * plane <= kEdgeStageBytes) return edge_feature_launch<2, true>(x, idx, B, C, N, k, out, stream);
+  if (plane <= kEdgeStageBytes) return edge_feature_launch<1, true>(x, idx, B, C, N, k, out, stream);
+  return edge_feature_launch<4, false>(x, idx, B, C, N, k, out, stream);
 }
 
 HG_API size_t hg_edge_feature_grad_workspace_bytes(int B, int N, int k) {

@@ -608,7 +608,12 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   const size_t need = hg_knn_self_workspace_bytes(B, K, C, k1);
   HG_REQUIRE(workspace && workspace_bytes >= need, HG_E_WORKSPACE, "knn_self: workspace too small (%zu < %zu)",
              workspace_bytes, need);
-  HG_REQUIRE((size_t)K * sizeof(float) * 4 <= 200 * 1024, HG_E_UNSUPPORTED, "knn_self: K=%d too large for C=%d path", K, C);
+  // the FP32 row select stages four rows of K distances per CTA; beyond that only the tensor-core kernel runs
+  const bool rows_fit = (size_t)K * sizeof(float) * 4 <= 200 * 1024;
+  const bool tc_shape = hg_knn_tc_supported_feature(K, C, k1) && (reinterpret_cast<uintptr_t>(pc) & 15) == 0;
+  HG_REQUIRE(rows_fit || tc_shape, HG_E_UNSUPPORTED, "knn_self: K=%d too large for C=%d path", K, C);
+  HG_REQUIRE(rows_fit || g_hg_tune_knn_tc_off != 1, HG_E_UNSUPPORTED,
+             "knn_self: hg_tune(\"knn_tc\", 1) selects the FP32 path, which takes K <= 12800 (got K=%d)", K);
   const auto [nb, xx, dist] = hg_layout_at<KnnGenericWorkspace>(workspace, B, K);
   knn_sumsq_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, (long long)B * K, C, xx);
   HG_CHECK_LAUNCH("knn_sumsq_kernel");
@@ -617,10 +622,13 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   // (small batches leave the serial chain of a CTA exposed -- measured at K = 1024, C = 64: 16 clouds 85 us against
   // 143 us, 8 clouds 82 against 95, 4 clouds 79 against 65 -- so fewer CTAs than a quarter of the SMs stay on the FP32
   // path unless hg_tune("knn_tc", 2) forces the tensor-core kernel; long lists, k1 > 32, need half the SMs -- measured at
-  // 2048 x 64, k = 40: 4 clouds 143 us FP32 against 153 tensor-core, 8 clouds 283 against 157, 32 clouds 1121 against 393)
+  // 2048 x 64, k = 40: 4 clouds 143 us FP32 against 153 tensor-core, 8 clouds 283 against 157, 32 clouds 1121 against 393).
+  // Past 4096 points the batch rule does not apply: each CTA walks 17..64 tiles, and the tensor-core kernel won at every
+  // batch measured, from one cloud up (8192 x 64, k = 40: 362 us against 952 at one cloud, 907 against 7534 at eight;
+  // DESIGN.md section 5.2).  Past 12800 points it is the only route.
   const long long tc_ctas = (long long)B * ((K + 127) / 128);
   const bool tc_fills = (k1 > 32 ? 2 : 4) * tc_ctas >= hg_sm_count() || g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5;
-  if (g_hg_tune_knn_tc_off != 1 && tc_fills && hg_knn_tc_supported(K, C, k1) && (reinterpret_cast<uintptr_t>(pc) & 15) == 0)
+  if (g_hg_tune_knn_tc_off != 1 && tc_shape && (tc_fills || K > 4096))
     return hg_knn_tc_run(pc, xx, B, K, C, k1, vals, idx, stream);
   const bool long_list = k1 > 32;
   const size_t sel_smem = ((size_t)4 * K + (size_t)8 * knn_sel_cap(long_list)) * sizeof(float);

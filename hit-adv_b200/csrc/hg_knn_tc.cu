@@ -100,6 +100,19 @@ __host__ __device__ constexpr uint32_t tc_idesc(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// Column norms.  Up to 4096 points (kTileNorms = false) the norms of the whole cloud stay resident in shared memory,
+// ceil(K/256) * 1 KiB.  Beyond that (kTileNorms = true, up to 16384 points) only the current candidate tile's 256 norms
+// are: every thread loads two of them from global memory (L2) while the tile's TMA loads and MMAs are in flight, and
+// one barrier after those completes makes them visible to the CTA.  The B panels are single-buffered (the next tile is
+// loaded only once every warp has released the current one), so one 1 KiB slot is enough, and shared memory no longer
+// depends on K.  (Not a cp.async.bulk on the tile's mbarrier: a cloud's norms start at b * K floats, 16-byte
+// aligned only when K % 4 == 0.)  max|x|, the error bound's cloud term, is still taken over all K rows.
+__device__ __forceinline__ void tc_stage_tile_norms(float *slot, const float *xxb, int K, int t, int tid) {
+  const int j0 = t * kTcTile + tid, j1 = j0 + 128;
+  slot[tid] = j0 < K ? xxb[j0] : CUDART_INF_F;
+  slot[tid + 128] = j1 < K ? xxb[j1] : CUDART_INF_F;
+}
+
 // ---- fused single pass: tensor-core filter + exact FP32 evaluation out of the SAME shared-memory tiles --------------
 // The candidate tile that TMA brought in for the MMA holds, row by row, exactly the FP32 features the reference
 // arithmetic needs.  So a column the TF32 distances cannot rule out is evaluated on the spot -- the thread (= query row)
@@ -147,7 +160,7 @@ struct TcList {
   }
 };
 
-template <int C, int KM>
+template <int C, int KM, bool kTileNorms>
 __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     knn_tc_fused_kernel(const __grid_constant__ CUtensorMap map, int K, int k1, int two_pass,
                         const float *__restrict__ xx, float *__restrict__ vals, int *__restrict__ idx) {
@@ -178,10 +191,14 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   float xmax = 0.f;  // largest squared norm of the cloud (for the error bound below)
-  for (int j = tid; j < ntiles * kTcTile; j += 128) {
-    const float v = j < K ? xx[(size_t)b * K + j] : CUDART_INF_F;
-    sxx[j] = v;
-    if (j < K) xmax = fmaxf(xmax, v);
+  if (kTileNorms) {
+    for (int j = tid; j < K; j += 128) xmax = fmaxf(xmax, xx[(size_t)b * K + j]);
+  } else {
+    for (int j = tid; j < ntiles * kTcTile; j += 128) {
+      const float v = j < K ? xx[(size_t)b * K + j] : CUDART_INF_F;
+      sxx[j] = v;
+      if (j < K) xmax = fmaxf(xmax, v);
+    }
   }
   xmax = hg_warp_max_f32(xmax);
   if ((tid & 31) == 0) wmax[warp] = xmax;
@@ -198,7 +215,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
 
   const int i = row0 + tid;
   const bool live = i < K;
-  const float xi = live ? sxx[i] : 0.f;
+  const float xi = live ? (kTileNorms ? xx[(size_t)b * K + i] : sxx[i]) : 0.f;
   const float eps = 1.1f * 0.00390625f * sqrtf(xi * xmax) + 1e-5f * (xi + xmax);
   const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
   const unsigned sw = (unsigned)(tid & 7);  // swizzle phase of this thread's own row in the A panels
@@ -268,6 +285,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
                       (p | ks) ? 1u : 0u);
       tc_commit(&bar_mma);
     }
+    if (kTileNorms) tc_stage_tile_norms(sxx, xx + (size_t)b * K, K, t, tid);
     // every thread reads the tiles with ordinary loads below: each one observes the TMA completions itself
     if (step == 0) {
       tc_mbar_wait(&bar_a, 0);
@@ -286,6 +304,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     phase_m ^= 1;
     __syncwarp();
     tc_fence_after();
+    if (kTileNorms) __syncthreads();  // the tile's norms, stored by all four warps
 
     if (scan) {
       // first threshold: k1-th smallest of the 32 column-class minima of the approximate distances scanned so far
@@ -293,7 +312,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
       for (int q = 0; q < kTcTile / 32; ++q) {
         float acc[32];
         tc_ld32(trow + (uint32_t)(q * 32), acc);
-        const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q * 32);
+        const float4 *sx4 = reinterpret_cast<const float4 *>(kTileNorms ? sxx + q * 32 : sxx + t * kTcTile + q * 32);
 #pragma unroll
         for (int c4 = 0; c4 < 8; ++c4) {
           const float4 xj = sx4[c4];
@@ -336,7 +355,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     for (int q = 0; q < kTcTile / 32; ++q) {
       float acc[32];
       tc_ld32(trow + (uint32_t)(q * 32), acc);
-      const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q * 32);
+      const float4 *sx4 = reinterpret_cast<const float4 *>(kTileNorms ? sxx + q * 32 : sxx + t * kTcTile + q * 32);
       unsigned hits = 0u;
 #pragma unroll
       for (int c4 = 0; c4 < 8; ++c4) {
@@ -370,7 +389,8 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
         const int jr1 = next_hit();
         const int jrb = jr1 >= 0 ? jr1 : jr0;
         float d0, d1;
-        exact2(jr0, jrb, sxx[t * kTcTile + jr0], sxx[t * kTcTile + jrb], d0, d1);
+        exact2(jr0, jrb, kTileNorms ? sxx[jr0] : sxx[t * kTcTile + jr0], kTileNorms ? sxx[jrb] : sxx[t * kTcTile + jrb],
+               d0, d1);
         if (d0 < top.v[KM - 1]) top.push(d0, t * kTcTile + jr0);
         if (jr1 >= 0 && d1 < top.v[KM - 1]) top.push(d1, t * kTcTile + jr1);
       }
@@ -415,7 +435,7 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, float (&v)[16]) {
 // The first threshold is the k1-th smallest of 64 column-class minima (class = column mod 64; K >= 256, so tile 0 alone
 // already gives every class a real column): k1 <= 64 distinct columns have an approximate distance <= tau, so the
 // admission test  approx_j <= (k1-th exact so far) + 2 eps  is the short-list kernel's, and so are values and indices.
-template <int C>
+template <int C, bool kTileNorms>
 __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     knn_tc_long_kernel(const __grid_constant__ CUtensorMap map, int K, int k1, int two_pass,
                        const float *__restrict__ xx, float *__restrict__ vals, int *__restrict__ idx) {
@@ -446,10 +466,14 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   float xmax = 0.f;
-  for (int j = tid; j < ntiles * kTcTile; j += 128) {
-    const float v = j < K ? xx[(size_t)b * K + j] : CUDART_INF_F;
-    sxx[j] = v;
-    if (j < K) xmax = fmaxf(xmax, v);
+  if (kTileNorms) {
+    for (int j = tid; j < K; j += 128) xmax = fmaxf(xmax, xx[(size_t)b * K + j]);
+  } else {
+    for (int j = tid; j < ntiles * kTcTile; j += 128) {
+      const float v = j < K ? xx[(size_t)b * K + j] : CUDART_INF_F;
+      sxx[j] = v;
+      if (j < K) xmax = fmaxf(xmax, v);
+    }
   }
   xmax = hg_warp_max_f32(xmax);
   if ((tid & 31) == 0) wmax[warp] = xmax;
@@ -466,7 +490,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
 
   const int i = row0 + tid;
   const bool live = i < K;
-  const float xi = live ? sxx[i] : 0.f;
+  const float xi = live ? (kTileNorms ? xx[(size_t)b * K + i] : sxx[i]) : 0.f;
   const float eps = 1.1f * 0.00390625f * sqrtf(xi * xmax) + 1e-5f * (xi + xmax);
   const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
   const unsigned sw = (unsigned)(tid & 7);
@@ -492,6 +516,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
                       (p | ks) ? 1u : 0u);
       tc_commit(&bar_mma);
     }
+    if (kTileNorms) tc_stage_tile_norms(sxx, xx + (size_t)b * K, K, t, tid);
     if (first) tc_mbar_wait(&bar_a, 0);
     tc_mbar_wait(&bar_b, phase_b);
     phase_b ^= 1;
@@ -499,6 +524,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
     phase_m ^= 1;
     __syncwarp();
     tc_fence_after();
+    if (kTileNorms) __syncthreads();  // the tile's norms, stored by all four warps
   };
   auto release = [&]() {
     tc_fence_before();
@@ -521,7 +547,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
         for (int h = 0; h < 4; ++h) {  // columns q2 * 64 + h * 16 + c: class h * 16 + c
           float acc[16];
           tc_ld16(trow + (uint32_t)(q2 * 64 + h * 16), acc);
-          const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q2 * 64 + h * 16);
+          const float4 *sx4 = reinterpret_cast<const float4 *>((kTileNorms ? sxx : sxx + t * kTcTile) + q2 * 64 + h * 16);
 #pragma unroll
           for (int c4 = 0; c4 < 4; ++c4) {
             const float4 xj = sx4[c4];
@@ -568,7 +594,7 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
       for (int h = 0; h < 2; ++h) {
         float acc[16];
         tc_ld16(trow + (uint32_t)(q * 32 + h * 16), acc);
-        const float4 *sx4 = reinterpret_cast<const float4 *>(sxx + t * kTcTile + q * 32 + h * 16);
+        const float4 *sx4 = reinterpret_cast<const float4 *>((kTileNorms ? sxx : sxx + t * kTcTile) + q * 32 + h * 16);
 #pragma unroll
         for (int c4 = 0; c4 < 4; ++c4) {
           const float4 xj = sx4[c4];
@@ -623,8 +649,9 @@ __global__ void __launch_bounds__(128, C <= 64 ? 2 : 1)
             acc1 = __fmaf_rn(a.w, v1.w, acc1);
           }
         }
-        const float d0 = __fadd_rn(__fadd_rn(__fadd_rn(sxx[t * kTcTile + jr0], __fmul_rn(-2.0f, acc0)), xi), 0.0f);
-        const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(sxx[t * kTcTile + jrb], __fmul_rn(-2.0f, acc1)), xi), 0.0f);
+        const float *tnorm = kTileNorms ? sxx : sxx + t * kTcTile;
+        const float d0 = __fadd_rn(__fadd_rn(__fadd_rn(tnorm[jr0], __fmul_rn(-2.0f, acc0)), xi), 0.0f);
+        const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(tnorm[jrb], __fmul_rn(-2.0f, acc1)), xi), 0.0f);
         if (d0 < top.v[KM - 1]) top.push(d0, t * kTcTile + jr0);
         if (jr1 >= 0 && d1 < top.v[KM - 1]) top.push(d1, t * kTcTile + jr1);
       }
@@ -660,17 +687,18 @@ EncodeTiledFn encode_tiled() {
   return fn;
 }
 
-template <int C>
+template <int C, bool kTileNorms>
 int run_tc(const float *pc, const float *xx, int B, int K, int k1, float *vals, int *idx, cudaStream_t stream) {
   EncodeTiledFn enc = encode_tiled();
   HG_REQUIRE(enc != nullptr, HG_E_UNSUPPORTED, "knn (tensor-core path): cuTensorMapEncodeTiled is not available");
   constexpr int NP = C / kTcPanelK;
-  const size_t smem = (size_t)NP * (kTcRows + kTcTile) * 128 + (size_t)((K + kTcTile - 1) / kTcTile) * kTcTile * sizeof(float);
+  const size_t smem = (size_t)NP * (kTcRows + kTcTile) * 128 +
+                      (size_t)(kTileNorms ? 1 : (K + kTcTile - 1) / kTcTile) * kTcTile * sizeof(float);
   static HgPerDeviceOnce once;
   if (once.first()) {
-    HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 20>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
-    HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
-    HG_CUDA((cudaFuncSetAttribute(knn_tc_long_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
+    HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 20, kTileNorms>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
+    HG_CUDA((cudaFuncSetAttribute(knn_tc_fused_kernel<C, 32, kTileNorms>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
+    HG_CUDA((cudaFuncSetAttribute(knn_tc_long_kernel<C, kTileNorms>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)));
   }
   CUtensorMap map;
   const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)K, (cuuint64_t)B};
@@ -686,31 +714,37 @@ int run_tc(const float *pc, const float *xx, int B, int K, int k1, float *vals, 
   // forces the single sweep whose threshold starts from tile 0 only
   const int two_pass = g_hg_tune_knn_tc_off == 5 ? 0 : 1;
   if (k1 <= 20)
-    knn_tc_fused_kernel<C, 20><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
+    knn_tc_fused_kernel<C, 20, kTileNorms><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
   else if (k1 <= 32)
-    knn_tc_fused_kernel<C, 32><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
+    knn_tc_fused_kernel<C, 32, kTileNorms><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
   else
-    knn_tc_long_kernel<C><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
+    knn_tc_long_kernel<C, kTileNorms><<<grid, 128, smem, stream>>>(map, K, k1, two_pass, xx, vals, idx);
   HG_CHECK_LAUNCH("knn_tc_fused_kernel");
   return HG_OK;
 }
 
 }  // namespace
 
-// Shapes the tensor-core path takes: C a multiple of 32 up to 128 (DGCNN: 64, 64, 128), clouds of 256..4096 points,
-// lists of up to 64 neighbours.
+// Shapes the tensor-core path takes with the cloud's column norms resident: C a multiple of 32 up to 128 (DGCNN: 64, 64,
+// 128), clouds of 256..4096 points, lists of up to 64 neighbours.  (The padded 3-D route, hg_knn3.cu, is held to these.)
 bool hg_knn_tc_supported(int K, int C, int k1) {
   return (C == 32 || C == 64 || C == 96 || C == 128) && K >= 256 && K <= 4096 && k1 <= 64;
+}
+
+// Feature clouds: the same, up to 16384 points (per-tile column norms beyond 4096).
+bool hg_knn_tc_supported_feature(int K, int C, int k1) {
+  return (C == 32 || C == 64 || C == 96 || C == 128) && K >= 256 && K <= 16384 && k1 <= 64;
 }
 
 // xx [B,K] are the reference squared norms (knn_sumsq_kernel).  B <= 65535 (checked by the caller).
 int hg_knn_tc_run(const float *pc, const float *xx, int B, int K, int C, int k1, float *vals, int *idx,
                   cudaStream_t stream) {
+  const bool tile = K > 4096;
   switch (C) {
-    case 32: return run_tc<32>(pc, xx, B, K, k1, vals, idx, stream);
-    case 64: return run_tc<64>(pc, xx, B, K, k1, vals, idx, stream);
-    case 96: return run_tc<96>(pc, xx, B, K, k1, vals, idx, stream);
-    case 128: return run_tc<128>(pc, xx, B, K, k1, vals, idx, stream);
+    case 32: return tile ? run_tc<32, true>(pc, xx, B, K, k1, vals, idx, stream) : run_tc<32, false>(pc, xx, B, K, k1, vals, idx, stream);
+    case 64: return tile ? run_tc<64, true>(pc, xx, B, K, k1, vals, idx, stream) : run_tc<64, false>(pc, xx, B, K, k1, vals, idx, stream);
+    case 96: return tile ? run_tc<96, true>(pc, xx, B, K, k1, vals, idx, stream) : run_tc<96, false>(pc, xx, B, K, k1, vals, idx, stream);
+    case 128: return tile ? run_tc<128, true>(pc, xx, B, K, k1, vals, idx, stream) : run_tc<128, false>(pc, xx, B, K, k1, vals, idx, stream);
   }
   hg_set_error("knn (tensor-core path): unsupported channel count %d", C);
   return HG_E_UNSUPPORTED;

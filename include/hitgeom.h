@@ -143,6 +143,8 @@ int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *arg1, c
  * row of dist[i,j] = (xx_j + (-2*zz_ij)) + xx_i (DGCNN's pairwise_distance is exactly -dist).
  *   pc [B,K,C] point-major; vals [B,K,k1] ascending (may be NULL), idx [B,K,k1], lowest index first on ties.
  *   1 <= k1 <= 64 for every C, k1 <= K (DGCNN's k = 40 on its feature layers included).
+ *   C != 3: K <= 12800 for every C; C = 32, 64, 96 or 128 (DGCNN's 64, 64, 128) up to K = 16384, where clouds of more
+ *   than 12800 points take the tensor-core kernel only (hg_tune("knn_tc", 1) then fails with HG_E_UNSUPPORTED).
  * ------------------------------------------------------------------------------------------------------- */
 size_t hg_knn_self_workspace_bytes(int B, int K, int C, int k1);
 int hg_knn_self_f32(const float *pc, int B, int K, int C, int k1, float *vals, int *idx, void *workspace,
@@ -259,7 +261,7 @@ int hg_hitadv_deform_bwd_f32(const float *ori, const float *centers, const float
  *   out [B,2C,N,k]:  out[b,c,n,t] = x[b,c,idx[b,n,t]] - x[b,c,n],   out[b,C+c,n,t] = x[b,c,n]
  * written once in its final layout (the reference goes through gather + repeat + cat + permute().contiguous()).
  * The backward sums the incoming edges through a CSR reverse map in ascending edge order (deterministic; the
- * reference's index_put_(accumulate=True) uses floating-point atomics).
+ * reference's index_put_(accumulate=True) uses floating-point atomics).  Any N with N*k < 2^31, both directions.
  * ------------------------------------------------------------------------------------------------------- */
 int hg_edge_feature_f32(const float *x, const int64_t *idx, int B, int C, int N, int k, float *out, hgStream stream);
 size_t hg_edge_feature_grad_workspace_bytes(int B, int N, int k);
