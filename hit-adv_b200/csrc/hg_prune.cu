@@ -33,7 +33,8 @@ constexpr int kBuildThreads = 1024;
 constexpr int kSearchWarps = 4;
 constexpr float kSlack = 1.5e-6f;  // >= 24 u, u = 2^-24
 
-__device__ unsigned long long g_prune_tiles[4];  // nn: visited, total leaf pairs; knn: visited, total
+// nn: visited, total leaf pairs; knn: visited, total, then drains, candidates inserted, warp rounds of the drains
+__device__ unsigned long long g_prune_tiles[7];
 
 __device__ __forceinline__ float gap_rd(float alo, float ahi, float blo, float bhi) {
   return fmaxf(fmaxf(__fsub_rd(blo, ahi), __fsub_rd(alo, bhi)), 0.f);
@@ -480,52 +481,53 @@ struct PruneSearch {
   int *idx;           // same shape
   int *idx_state;     // kNN: second copy of idx or null
   const float *thr0;  // kNN: [B,Nq] exact upper bounds by original index, or null
-  unsigned long long *count;  // null, or {visited leaf pairs, all leaf pairs}
+  unsigned long long *count;  // null, or {visited leaf pairs, all leaf pairs} (kNN: then the three drain counts)
 };
 
-// Sorted list with the lexicographic (value, index) order, held in registers (static indexing only).
+// List of the k1 smallest (value, index) pairs in lexicographic order, ascending, held in registers and indexed only
+// by constants.  The k1 live entries are the tail [KM - k1, KM); the head holds (-inf, -1), which no candidate sorts
+// before, so the k1-th value is always v[KM - 1].
 template <int KM>
 struct LexTopK {
   float v[KM];
   int id[KM];
-  __device__ __forceinline__ void init() {
+  __device__ __forceinline__ void init(int k1) {
 #pragma unroll
     for (int t = 0; t < KM; ++t) {
-      v[t] = CUDART_INF_F;
-      id[t] = 0;
+      v[t] = t < KM - k1 ? -CUDART_INF_F : CUDART_INF_F;
+      id[t] = t < KM - k1 ? -1 : 0;
     }
   }
+  __device__ __forceinline__ bool sorts_before(float d, int j, int t) const {
+    return (d < v[t]) | ((d == v[t]) & (j < id[t]));  // no short-circuit: no branch
+  }
+  // Insertion as one pass of predicated compare-exchange steps: entry t takes entry t - 1 when (d, j) sorts before
+  // that, else (d, j) when it sorts before entry t.  (+inf, INT_MAX) sorts before nothing: a no-op.
   __device__ __forceinline__ void push(float d, int j) {
-    if (d < v[KM - 1] || (d == v[KM - 1] && j < id[KM - 1])) {
-      v[KM - 1] = d;
-      id[KM - 1] = j;
+    bool before = sorts_before(d, j, KM - 1);
 #pragma unroll
-      for (int t = KM - 1; t > 0; --t) {
-        if (v[t] < v[t - 1] || (v[t] == v[t - 1] && id[t] < id[t - 1])) {
-          const float tv = v[t];
-          v[t] = v[t - 1];
-          v[t - 1] = tv;
-          const int ti = id[t];
-          id[t] = id[t - 1];
-          id[t - 1] = ti;
-        }
-      }
+    for (int t = KM - 1; t > 0; --t) {
+      const bool prev = sorts_before(d, j, t - 1);
+      v[t] = prev ? v[t - 1] : before ? d : v[t];
+      id[t] = prev ? id[t - 1] : before ? j : id[t];
+      before = prev;
     }
-  }
-  __device__ __forceinline__ float kth(int k1) const {
-    float r = v[0];
-#pragma unroll
-    for (int t = 1; t < KM; ++t)
-      if (t == k1 - 1) r = v[t];
-    return r;
+    v[0] = before ? d : v[0];
+    id[0] = before ? j : id[0];
   }
 };
 
 __device__ __forceinline__ float nudge_up(float v) { return v < CUDART_INF_F ? nextafterf(v, CUDART_INF_F) : v; }
 
+// Resident CTAs per SM the search's register allocation must allow (0: no bound).  KM = 20: 4, since without a bound
+// ptxas stops at 96 registers and spills.  KM = 6 stays unbounded (72 registers, 7 CTAs): a bound of 8 CTAs
+// (64 registers) measured slower, 8.91 against 8.79 ms per 1024 x 16384 call (DESIGN 5.5).
+template <int KM>
+constexpr int kSearchMinCtas = KM == 20 ? 4 : 0;
+
 // KM == 1: 1-NN with the Chamfer arithmetic; KM > 1: kNN list with the KNNDist arithmetic and the folded filter.
 template <int KM>
-__global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSearch a) {
+__global__ void __launch_bounds__(kSearchWarps * 32, kSearchMinCtas<KM>) prune_search_kernel(PruneSearch a) {
   __shared__ float4 tile[kSearchWarps][kLeaf];  // 16 candidate pairs: (c0_j,c0_j1,c1_j,c1_j1), (c2_j,c2_j1,w_j,w_j1)
   __shared__ int tperm[kSearchWarps][kLeaf];
   constexpr bool kNN1 = KM == 1;
@@ -591,40 +593,74 @@ __global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSe
   int bid = 0x7fffffff;
   LexTopK<kNN1 ? 1 : KM> top;
   float seed = CUDART_INF_F, thr = CUDART_INF_F;
+  unsigned ndrain = 0u, nround = 0u, npush = 0u;  // kNN drains, warp-uniform; npush per lane
+  // exact values of the staged candidates in `sub` inserted into the list, all lanes in lockstep: a lane whose
+  // candidates are done inserts (+inf, INT_MAX)
+  auto drain = [&](unsigned sub) {
+    ++ndrain;
+    while (__any_sync(0xffffffffu, sub != 0u)) {
+      const int c = (__ffs(sub) - 1) & (kLeaf - 1);
+      const bool take = sub != 0u;
+      sub &= sub - 1u;
+      const int pp = c >> 1, h = c & 1;
+      const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
+      // knn_dist_exact<EXPANDED>: (xx_j + nzz) + xx_i
+      const float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
+      const int j = tperm[warp][c];
+      top.push(take ? d : CUDART_INF_F, take ? j : 0x7fffffff);
+      ++nround;
+      npush += take ? 1u : 0u;
+    }
+  };
+  int dfirst = 0;  // the first leaf Ls ^ d the main loop visits
+  unsigned long long visited = 0;
   if (!kNN1) {
+    top.init(a.k1);
     if (a.thr0 != nullptr) {
       seed = valid ? a.thr0[(size_t)b * Nq + qid] : CUDART_INF_F;
     } else if (KM <= kLeaf) {
-      // seed: the k1-th smallest exact distance over the own leaf (real candidates: an exact upper bound)
+      // seed: the k1-th smallest exact distance over the own leaf (real candidates: an exact upper bound), from a
+      // value-only min/max network over the list's layout
       stage(Ls);
-      top.init();
       for (int c = 0; c < kLeaf; ++c) {
         const int pp = c >> 1, h = c & 1;
         const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
         float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
 #pragma unroll
-        for (int u = 0; u < (kNN1 ? 1 : KM); ++u) {  // value-only insertion network
+        for (int u = 0; u < (kNN1 ? 1 : KM); ++u) {
           const float lo = fminf(top.v[u], d);
           d = fmaxf(top.v[u], d);
           top.v[u] = lo;
         }
       }
-      seed = valid ? nudge_up(top.kth(a.k1)) : CUDART_INF_F;
+      const float kth = top.v[KM - 1];
+      seed = valid ? nudge_up(kth) : CUDART_INF_F;
+      // the own leaf's visit: its candidates at or below the k1-th value fill the list, which leaves the threshold
+      // at the seed; the main loop starts at its sibling
+      top.init(a.k1);
+      unsigned sub = 0u;
+      for (int c = 0; c < kLeaf; ++c) {
+        const int pp = c >> 1, h = c & 1;
+        const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
+        const float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
+        sub |= (valid && d <= kth ? 1u : 0u) << c;
+      }
+      drain(sub);
+      visited = 1;
+      dfirst = 1;
     }
-    top.init();
     thr = seed;
   }
   if (!valid) thr = -CUDART_INF_F;  // padding lanes never need a leaf
 
   int P2 = 1;
   while (P2 < nlc) P2 <<= 1;
-  unsigned long long visited = 0;
   for (int d0 = 0; d0 < P2; d0 += 32) {
     // warp-uniform test of 32 leaves against the largest current threshold of the warp, box against box
     const float tw = hg_warp_max_f32(thr);
     const int Lt = Ls ^ (d0 + lane);
     bool pass = false;
-    if (Lt < nlc) pass = may_hold(box_d2_rd(qlo, qhi, cbox[2 * Lt], cbox[2 * Lt + 1]), tw, Sw);
+    if (Lt < nlc && d0 + lane >= dfirst) pass = may_hold(box_d2_rd(qlo, qhi, cbox[2 * Lt], cbox[2 * Lt + 1]), tw, Sw);
     unsigned m = __ballot_sync(0xffffffffu, pass);
     while (m) {
       const int bit = __ffs(m) - 1;
@@ -675,7 +711,7 @@ __global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSe
           o |= __float_as_uint(t.x) | __float_as_uint(t.y);
         }
         const bool hit = valid && (o >> 31) != 0u;
-        if (__any_sync(0xffffffffu, hit) && hit) {  // drain: which candidates, then exact values and insertion
+        if (__any_sync(0xffffffffu, hit)) {  // drain: which candidates, then exact values and insertion
           unsigned sub = 0u;
 #pragma unroll 4
           for (int pp = 0; pp < kLeaf / 2; ++pp) {
@@ -686,16 +722,8 @@ __global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSe
             t = __ffma2_rn(make_float2(a0, a0), make_float2(A.x, A.y), t);
             sub |= ((__float_as_uint(t.x) >> 31) << (2 * pp)) | ((__float_as_uint(t.y) >> 31) << (2 * pp + 1));
           }
-          while (sub) {
-            const int c = __ffs(sub) - 1;
-            sub &= sub - 1u;
-            const int pp = c >> 1, h = c & 1;
-            const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
-            // knn_dist_exact<EXPANDED>: (xx_j + nzz) + xx_i
-            const float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
-            top.push(d, tperm[warp][c]);
-          }
-          thr = fminf(seed, nudge_up(top.kth(a.k1)));
+          drain(hit ? sub : 0u);
+          if (hit) thr = fminf(seed, nudge_up(top.v[KM - 1]));
         }
       }
     }
@@ -704,6 +732,14 @@ __global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSe
     atomicAdd(a.count, visited);
     atomicAdd(a.count + 1, (unsigned long long)nlc);
   }
+  if (!kNN1 && a.count != nullptr) {
+    npush = __reduce_add_sync(0xffffffffu, npush);
+    if (lane == 0) {
+      atomicAdd(a.count + 2, (unsigned long long)ndrain);
+      atomicAdd(a.count + 3, (unsigned long long)npush);
+      atomicAdd(a.count + 4, (unsigned long long)nround);
+    }
+  }
   if (!valid) return;
   if (kNN1) {
     a.vals[(size_t)b * Nq + qid] = best;
@@ -711,11 +747,12 @@ __global__ void __launch_bounds__(kSearchWarps * 32) prune_search_kernel(PruneSe
   } else {
     const size_t o = ((size_t)b * Nq + qid) * a.k1;
 #pragma unroll
-    for (int s = 0; s < (kNN1 ? 1 : KM); ++s) {
-      if (s < a.k1) {
-        if (a.vals) a.vals[o + s] = top.v[s];
-        a.idx[o + s] = top.id[s];
-        if (a.idx_state) a.idx_state[o + s] = top.id[s];
+    for (int t = 0; t < (kNN1 ? 1 : KM); ++t) {
+      const int s = t - (KM - a.k1);  // the live entries are outputs 0 .. k1 - 1
+      if (s >= 0) {
+        if (a.vals) a.vals[o + s] = top.v[t];
+        a.idx[o + s] = top.id[t];
+        if (a.idx_state) a.idx_state[o + s] = top.id[t];
       }
     }
   }
@@ -896,6 +933,16 @@ HG_API int hg_prune_counters(unsigned long long *out4) {
   HG_CUDA(cudaMemcpyFromSymbol(out4, g_prune_tiles, sizeof(unsigned long long) * 4));
   const unsigned long long zero[4] = {0, 0, 0, 0};
   HG_CUDA(cudaMemcpyToSymbol(g_prune_tiles, zero, sizeof(zero)));
+  return HG_OK;
+}
+
+// kNN drains since the last call, {drains, candidates inserted, warp rounds}; synchronises the device.
+HG_API int hg_prune_drain_counters(unsigned long long *out3) {
+  HG_REQUIRE(out3, HG_E_BADARG, "prune_drain_counters: null pointer");
+  HG_CUDA(cudaDeviceSynchronize());
+  HG_CUDA(cudaMemcpyFromSymbol(out3, g_prune_tiles, sizeof(unsigned long long) * 3, sizeof(unsigned long long) * 4));
+  const unsigned long long zero[3] = {0, 0, 0};
+  HG_CUDA(cudaMemcpyToSymbol(g_prune_tiles, zero, sizeof(zero), sizeof(unsigned long long) * 4));
   return HG_OK;
 }
 

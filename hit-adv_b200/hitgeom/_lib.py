@@ -32,6 +32,7 @@ _SIGNATURES = {
     "hg_knn_tune_small": (None, [I]),
     "hg_tune": (I, [ctypes.c_char_p, I]),
     "hg_prune_counters": (I, [ctypes.POINTER(ctypes.c_ulonglong)]),
+    "hg_prune_drain_counters": (I, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "hg_prune_order_counters": (I, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "hg_launch_count": (ctypes.c_ulonglong, []),
     "hg_prof_enable": (None, [I]),

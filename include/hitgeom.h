@@ -63,13 +63,17 @@ int hg_probe_fp32_peak(float *tflops, float *device_scratch, hgStream stream);
  * (same results; the tests run both); "knn_win" = Z-order window of the small-cloud kNN seeds (0 = default);
  * "fps_threads" = 128 | 256 threads per cloud in furthest point sampling for clouds up to 2048 points (0 = default);
  * "prune" = 0 switches the pruned passes off, "prune_min_n" moves their size threshold, "prune_count" = 1 counts visited
- * leaf pairs and orderings; "prune_refit_tol" = rebuild tolerance of an ordering state's refit [permille] (0 = default),
- * "prune_refit_stage" = 1 stages the cloud in shared memory for the refit's gather, 2 reads it from global memory
- * (0 = default). */
+ * leaf pairs, self-kNN drains and orderings; "prune_refit_tol" = rebuild tolerance of an ordering state's refit
+ * [permille] (0 = default), "prune_refit_stage" = 1 stages the cloud in shared memory for the refit's gather, 2 reads it
+ * from global memory (0 = default). */
 int hg_tune(const char *key, int value);
 /* Leaf pairs the pruned passes visited and could have visited since the last call: {Chamfer visited, Chamfer total,
  * kNN visited, kNN total}, counted while hg_tune("prune_count", 1) is on.  Synchronises the device. */
 int hg_prune_counters(unsigned long long *out4);
+/* Drains of the pruned self-kNN search since the last call, counted while hg_tune("prune_count", 1) is on: {leaves
+ * drained (per warp of 32 queries), candidates inserted into a query's list, warp rounds of the drains (a round inserts
+ * one candidate on every lane that has one left)}.  Synchronises the device. */
+int hg_prune_drain_counters(unsigned long long *out3);
 /* Ordering builds since the last call, counted per cloud while hg_tune("prune_count", 1) is on: {refit and kept, rebuilt
  * from a state (invalid permutation or degraded leaf boxes), built without a state}.  Synchronises the device. */
 int hg_prune_order_counters(unsigned long long *out3);

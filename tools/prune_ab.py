@@ -3,7 +3,8 @@
 Per shape (bench.py's seeded make_clouds): hg_nn_bidir_f32 and hg_knn_self_f32 (k+1 = 6) timed with CUDA events,
 pruning off and on alternately; the ordering build on its own (torch.profiler, prune_order_kernel); the fraction of
 leaf pairs (32 x 32 point pairs each) the pruned passes visited, from their culling decisions; bit equality of every
-output over the whole batch.  Prints one JSON line per shape with the GPU name and power limit.
+output over the whole batch; the self-kNN search's drains (leaves drained, candidates inserted and warp rounds, from
+hg_prune_drain_counters).  Prints one JSON line per shape with the GPU name and power limit.
 
     python tools/prune_ab.py [--shapes 1024x16384,2048x8192,4096x4096] [--reps 10] [--out DIR]
 """
@@ -54,6 +55,12 @@ def counters():
     return list(c)
 
 
+def drain_counters():
+    c = (ctypes.c_ulonglong * 3)()
+    assert lib().hg_prune_drain_counters(c) == 0
+    return list(c)
+
+
 def run_shape(B, N, reps, k1):
     ori_np, adv_np = make_clouds(B, N, 1234)
     ori, adv = torch.from_numpy(ori_np).cuda(), torch.from_numpy(adv_np).cuda()
@@ -75,9 +82,11 @@ def run_shape(B, N, reps, k1):
     tune("prune", 1)
     tune("prune_count", 1)
     counters()
+    drain_counters()
     nn()
     kn()
     c = counters()
+    drains, pushes, rounds = drain_counters()
     tune("prune_count", 0)
     # ordering build on its own: kernel time from the profiler (three builds per step: ori and adv for the Chamfer
     # call, adv again for the kNN call)
@@ -105,7 +114,13 @@ def run_shape(B, N, reps, k1):
            "knn_self": {"off": stats(t[(0, "knn")]), "on": stats(t[(1, "knn")])},
            "ordering_build_ms_per_step_3_builds": build_us / 1e3,
            "search_kernel_ms": {k: v / 1e3 for k, v in search_us.items()},
-           "leaf_pairs_visited_fraction": {"chamfer": c[0] / max(c[1], 1), "knn": c[2] / max(c[3], 1)}}
+           "leaf_pairs_visited": {"chamfer": c[0], "chamfer_total": c[1], "knn": c[2], "knn_total": c[3]},
+           "leaf_pairs_visited_fraction": {"chamfer": c[0] / max(c[1], 1), "knn": c[2] / max(c[3], 1)},
+           # per drained leaf: candidates inserted per lane and warp rounds; busy lanes per round (of 32)
+           "knn_drains": {"drains": drains, "inserted": pushes, "rounds": rounds,
+                          "inserted_per_lane_per_drain": pushes / max(32 * drains, 1),
+                          "rounds_per_drain": rounds / max(drains, 1),
+                          "lanes_busy_per_round": pushes / max(rounds, 1)}}
     for w in ("nn_bidir", "knn_self"):
         rec[w]["speedup"] = rec[w]["off"]["median_ms"] / rec[w]["on"]["median_ms"]
     return rec
