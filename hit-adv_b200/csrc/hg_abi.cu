@@ -19,29 +19,10 @@ HG_API int hg_version(void) { return 200; }
 
 // Development knobs (benchmarks / A-B experiments only; not part of the stable ABI): small integer switches by name.
 int g_hg_tune_knn_tc_off = 0;
-int g_hg_tune_knn_win = 0;
-int g_hg_tune_scatter = 0;  // gather/group gradient: 0 auto, 1 single-buffer staged kernel, 2 bulk-copy pipeline
-int g_hg_tune_fps_threads = 0;  // furthest point sampling: threads per cloud for small clouds (0 = default)
 HG_API int hg_tune(const char *key, int value) {
   if (key == nullptr) return HG_E_BADARG;
-  if (!strcmp(key, "scatter")) {
-    g_hg_tune_scatter = value;
-    return HG_OK;
-  }
-  if (!strcmp(key, "knn_win")) {  // Z-order window of the small-cloud kNN seeds (0 = default)
-    g_hg_tune_knn_win = value;
-    return HG_OK;
-  }
   if (!strcmp(key, "knn_tc")) {  // 1 = tensor-core kNN prefilter off (FP32 tile + row-select path)
     g_hg_tune_knn_tc_off = value;
-    return HG_OK;
-  }
-  if (!strcmp(key, "nn_exact")) {
-    g_hg_tune_nn_exact = value;
-    return HG_OK;
-  }
-  if (!strcmp(key, "fps_threads")) {
-    g_hg_tune_fps_threads = value;
     return HG_OK;
   }
   if (!strcmp(key, "small_fused")) {  // 1 = small clouds use the general (multi-kernel) finish / kNN-backward paths

@@ -35,12 +35,8 @@ struct HgNvtxRange {
 };
 #define HG_NVTX_RANGE(name) HgNvtxRange hg_nvtx_range_(name)
 
-extern int g_hg_tune_knn_win;     // hg_tune("knn_win", n)
 extern int g_hg_tune_knn_tc_off;  // hg_tune("knn_tc", 1) switches the tensor-core kNN prefilter off
-extern int g_hg_tune_nn_exact;  // hg_tune("nn_exact", v), see hg_nn_bidir.cu
 extern int g_hg_tune_small_fused_off;  // hg_tune("small_fused", 1): general paths for small clouds too (A/B, tests)
-extern int g_hg_tune_fps_threads;  // hg_tune("fps_threads", 128|256): development knob
-extern int g_hg_tune_scatter;  // hg_tune("scatter", v): development knob, see hg_abi.cu
 extern unsigned long long g_hg_launches;  // kernels launched by this library (bench.py's gpu_launches)
 
 #define HG_CHECK_LAUNCH(name)                                            \

@@ -959,8 +959,7 @@ int knn3_small_self(const float *pc, int B, int N, int k1, float *vals, int *idx
   }
   const size_t seed_smem = (size_t)N * (sizeof(float4) + 2 * sizeof(int));
   // window of the Z-order scan: enough points for a k1-th smallest that is close to the true one
-  int win = k1 <= 8 ? 64 : (k1 <= 16 ? 80 : 96);  // measured (388 x 1024): 64 beats 32 by 5 % at k+1 = 6, 96 beats 64 by 6 % at 20
-  if (g_hg_tune_knn_win > 0) win = g_hg_tune_knn_win;  // hg_tune("knn_win", n): development knob
+  const int win = k1 <= 8 ? 64 : (k1 <= 16 ? 80 : 96);  // measured (388 x 1024): 64 beats 32 by 5 % at k+1 = 6, 96 beats 64 by 6 % at 20
   static HgPerDeviceOnce once[3];
   constexpr int kSeedMaxSmem = 8192 * (int)(sizeof(float4) + 2 * sizeof(int));
   if (k1 <= 6) {

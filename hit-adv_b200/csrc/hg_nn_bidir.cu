@@ -41,11 +41,6 @@ struct NnParams {
   int RB;                       // rows per CTA (multiple of kColBatch)
   unsigned long long *colres;   // [B,N1]  (ord(min over rows) << 32) | global row batch
   unsigned long long *rowres;   // [B,N2]  (ord(min over cols) << 32) | (column group << 5 | lane)
-  // approximate-tracker path only (see nn_bidir_d3a_kernel):
-  unsigned *colsec;             // [B,N1]  ord(smallest tracked value OUTSIDE the winning batch)
-  unsigned *rowsec;             // [B,N2]  ord(smallest tracked value outside the winning lane's columns)
-  const float *eps2;            // [B]     2 * (bound on |tracked - reference value|) for this pair of clouds
-  int *amb;                     // [1 + B*(N1+N2)]  counter, then the entries the finish kernel could not settle
   // null, or the per-cloud info of the two pruned-path orderings: only the clouds they flag are computed here
   const float4 *only_a, *only_b;
 };
@@ -408,337 +403,6 @@ static int launch_finish_small(const NnParams &p, int B, float *min1, int *arg1,
   return HG_OK;
 }
 
-// ================================================================================================================
-// Approximate tracker + exact recovery (round 2).
-//
-// The exact loop above sits on the floor of its formulation: 5 FMA-pipe operations and one 3-input min per pair.  The
-// loop below TRACKS a cheaper value,
-//     A(i,j) = fl( fma(y2,x2', fma(y1,x1', fma(y0,x0', rx_i))) + ry_j ),        x' = -2x,
-// four packed operations instead of five (tools/ubench/nn_approx4.cu on a B200: 54.5 % -> 62.7 % of the FP32 peak
-// with the bookkeeping below).  A is not the reference's rounding of P = (rx + ry) - 2zz, but both are a handful of
-// roundings of the same real number: |A - P| <= 9 u S with u = 2^-24 and S = (|x| + |y|)^2 >= every intermediate
-// (Cauchy-Schwarz on the partial dot products).  eps2 = 2 * 12 u S_max per pair of clouds (nn_eps_kernel).
-//
-// Exactness is restored by the finish kernel, which needs to know, for every column (row), whether a value within
-// eps2 of the tracked minimum exists OUTSIDE the coarse cell (32-row batch / the T columns of one lane) that holds it:
-//   * not so (the rule): the reference minimum and its first index lie inside the cell -- any entry outside has
-//     P >= A - eps > best + eps >= P(tracked winner) -- and the cell is re-evaluated with the reference arithmetic, as before;
-//   * so (near-ties, duplicated points): the entry goes on a list and a warp re-scans the whole row / column exactly
-//     (nn_resolve_kernel).  Correct for any input; costs one exact N-length scan per ambiguous entry.
-// The loop therefore keeps, per column, the minimum of the CURRENT batch (reset every 32 rows) and folds it into
-// (best, best batch, runner-up among the other batches) at the batch boundary; per row, one ballot of the lanes within
-// eps2 of the warp minimum replaces the equality ballot (a second set bit = a near-tie in another lane).  CTAs merge
-// with integer atomicMin as before; what an atomicMin displaces, or fails to displace, goes to the runner-up array.
-constexpr float kNnEpsFactor = 24.0f * 5.9604645e-8f;  // 2 * 12 u
-
-__global__ void __launch_bounds__(256) nn_eps_kernel(const float *__restrict__ gts, const float *__restrict__ preds,
-                                                     int N2, int N1, float *__restrict__ eps2) {
-  const int b = blockIdx.x, tid = threadIdx.x;
-  float mx = 0.f, my = 0.f;
-  const float *gx = gts + (size_t)b * N2 * 3, *gy = preds + (size_t)b * N1 * 3;
-  for (int i = tid; i < N2; i += 256) {
-    const float x0 = gx[(size_t)i * 3], x1 = gx[(size_t)i * 3 + 1], x2 = gx[(size_t)i * 3 + 2];
-    mx = fmaxf(mx, hg_dot3_fma(x0, x1, x2, x0, x1, x2));
-  }
-  for (int j = tid; j < N1; j += 256) {
-    const float y0 = gy[(size_t)j * 3], y1 = gy[(size_t)j * 3 + 1], y2 = gy[(size_t)j * 3 + 2];
-    my = fmaxf(my, hg_dot3_fma(y0, y1, y2, y0, y1, y2));
-  }
-  mx = hg_warp_max_f32(mx);
-  my = hg_warp_max_f32(my);
-  __shared__ float rx_s[8], ry_s[8];
-  if ((tid & 31) == 0) {
-    rx_s[tid >> 5] = mx;
-    ry_s[tid >> 5] = my;
-  }
-  __syncthreads();
-  if (tid == 0) {
-    for (int w = 1; w < 8; ++w) {
-      mx = fmaxf(mx, rx_s[w]);
-      my = fmaxf(my, ry_s[w]);
-    }
-    const float s = (sqrtf(mx) + sqrtf(my)) * (sqrtf(mx) + sqrtf(my));
-    eps2[b] = fmaxf(kNnEpsFactor * s * 1.001f, 1e-37f);  // NaN / inf inputs give a NaN / inf bound: everything ambiguous
-  }
-}
-
-template <int T, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, (T == 8 ? 16 : 12) / WARPS) nn_bidir_d3a_kernel(NnParams p) {
-  extern __shared__ float4 smem[];
-  float4 *xs = smem;  // as in nn_bidir_d3_kernel
-  uint4 *rowpart = reinterpret_cast<uint4 *>(smem + p.RB + 4);  // [WARPS][RB/2] (m_a,near_a,m_b,near_b)
-  float *sbest = reinterpret_cast<float *>(rowpart + (size_t)WARPS * (p.RB / 2));  // [T][WARPS*32] best batch minimum
-  float *ssec = sbest + T * WARPS * 32;                                            // [T][WARPS*32] runner-up
-  int *scid = reinterpret_cast<int *>(ssec + T * WARPS * 32);                      // [T][WARPS*32] best batch
-
-  const int b = blockIdx.z;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int cgroup = blockIdx.y * WARPS + warp;
-  const int cbase = cgroup * 32 * T + lane * T;
-  const int r0 = blockIdx.x * p.RB;
-  const bool warp_active = cgroup * 32 * T < p.N1;
-  const float eps2 = p.eps2[b];
-
-  const float *gx = p.gts + (size_t)b * p.N2 * 3;
-  for (int rp = threadIdx.x; rp < p.RB / 2 + 2; rp += WARPS * 32) {
-    float v[2][4];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int i = r0 + 2 * rp + h;
-      v[h][0] = v[h][1] = v[h][2] = 0.f;
-      v[h][3] = CUDART_INF_F;
-      if (i < p.N2 && 2 * rp + h < p.RB) {
-        const float x0 = __ldg(gx + (size_t)i * 3), x1 = __ldg(gx + (size_t)i * 3 + 1), x2 = __ldg(gx + (size_t)i * 3 + 2);
-        v[h][0] = -2.0f * x0;
-        v[h][1] = -2.0f * x1;
-        v[h][2] = -2.0f * x2;
-        v[h][3] = hg_dot3_fma(x0, x1, x2, x0, x1, x2);
-      }
-    }
-    xs[2 * rp] = make_float4(v[0][0], v[1][0], v[0][1], v[1][1]);
-    xs[2 * rp + 1] = make_float4(v[0][2], v[1][2], v[0][3], v[1][3]);
-  }
-  float y0[T], y1[T], y2[T], ry[T];
-  const float *gy = p.preds + (size_t)b * p.N1 * 3;
-#pragma unroll
-  for (int t = 0; t < T; ++t) {
-    const int j = cbase + t;
-    y0[t] = y1[t] = y2[t] = 0.f;
-    ry[t] = CUDART_INF_F;
-    if (j < p.N1) {
-      y0[t] = __ldg(gy + (size_t)j * 3);
-      y1[t] = __ldg(gy + (size_t)j * 3 + 1);
-      y2[t] = __ldg(gy + (size_t)j * 3 + 2);
-      ry[t] = hg_dot3_fma(y0[t], y1[t], y2[t], y0[t], y1[t], y2[t]);
-    }
-  }
-  __syncthreads();
-
-  if (warp_active) {
-    float cm[T];
-#pragma unroll
-    for (int t = 0; t < T; ++t) {
-      cm[t] = CUDART_INF_F;
-      sbest[t * WARPS * 32 + threadIdx.x] = CUDART_INF_F;
-      ssec[t * WARPS * 32 + threadIdx.x] = CUDART_INF_F;
-      scid[t * WARPS * 32 + threadIdx.x] = r0 / kColBatch;
-    }
-    uint4 *myrow = rowpart + (size_t)warp * (p.RB / 2);
-    float4 xA = xs[0], xB = xs[1], xC = xs[2], xD = xs[3];
-    for (int rb = 0; rb < p.RB; rb += kColBatch) {
-#pragma unroll 2
-      for (int rr = 0; rr < kColBatch; rr += 4) {
-        const int rq = (rb + rr) >> 1;
-        const float4 nA = xs[2 * rq + 4], nB = xs[2 * rq + 5], nC = xs[2 * rq + 6], nD = xs[2 * rq + 7];
-        const float2 X0 = make_float2(xA.x, xA.y), X1 = make_float2(xA.z, xA.w), X2 = make_float2(xB.x, xB.y),
-                     RX = make_float2(xB.z, xB.w);
-        const float2 Z0 = make_float2(xC.x, xC.y), Z1 = make_float2(xC.z, xC.w), Z2 = make_float2(xD.x, xD.y),
-                     RZ = make_float2(xD.z, xD.w);
-        float2 P[T], Q[T];
-#pragma unroll
-        for (int t = 0; t < T; ++t) {
-          float2 tt = __ffma2_rn(make_float2(y0[t], y0[t]), X0, RX);  // rows past N2 carry rx = +inf: A = +inf
-          float2 uu = __ffma2_rn(make_float2(y0[t], y0[t]), Z0, RZ);
-          tt = __ffma2_rn(make_float2(y1[t], y1[t]), X1, tt);
-          uu = __ffma2_rn(make_float2(y1[t], y1[t]), Z1, uu);
-          tt = __ffma2_rn(make_float2(y2[t], y2[t]), X2, tt);
-          uu = __ffma2_rn(make_float2(y2[t], y2[t]), Z2, uu);
-          P[t] = __fadd2_rn(tt, make_float2(ry[t], ry[t]));
-          Q[t] = __fadd2_rn(uu, make_float2(ry[t], ry[t]));
-          cm[t] = fminf(fminf(fminf(fminf(cm[t], P[t].x), P[t].y), Q[t].x), Q[t].y);  // 2 x FMNMX3, BATCH minimum
-        }
-        float ma = fminf(P[0].x, P[1].x), mb = fminf(P[0].y, P[1].y);
-        float mc = fminf(Q[0].x, Q[1].x), md = fminf(Q[0].y, Q[1].y);
-#pragma unroll
-        for (int t = 2; t < T; t += 2) {
-          ma = fminf(fminf(ma, P[t].x), P[t + 1].x);
-          mb = fminf(fminf(mb, P[t].y), P[t + 1].y);
-          mc = fminf(fminf(mc, Q[t].x), Q[t + 1].x);
-          md = fminf(fminf(md, Q[t].y), Q[t + 1].y);
-        }
-        const float wa = hg_warp_min_f32(ma), wb = hg_warp_min_f32(mb);
-        const float wc = hg_warp_min_f32(mc), wd = hg_warp_min_f32(md);
-        // lanes whose T columns hold a value within eps2 of the row's tracked minimum (the minimum's lane included)
-        const unsigned ka = __ballot_sync(0xffffffffu, ma <= wa + eps2), kb = __ballot_sync(0xffffffffu, mb <= wb + eps2);
-        const unsigned kc = __ballot_sync(0xffffffffu, mc <= wc + eps2), kd = __ballot_sync(0xffffffffu, md <= wd + eps2);
-        if (lane == 0) {
-          myrow[rq] = make_uint4(__float_as_uint(wa), ka, __float_as_uint(wb), kb);
-          myrow[rq + 1] = make_uint4(__float_as_uint(wc), kc, __float_as_uint(wd), kd);
-        }
-        xA = nA;
-        xB = nB;
-        xC = nC;
-        xD = nD;
-      }
-      const int batch = (r0 + rb) / kColBatch;
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        const int o = t * WARPS * 32 + threadIdx.x;
-        const float best = sbest[o], bm = cm[t];
-        const bool win = bm < best;  // strict: among equal batch minima the earliest batch stays the winner
-        ssec[o] = fminf(ssec[o], win ? best : bm);
-        if (win) {
-          sbest[o] = bm;
-          scid[o] = batch;
-        }
-        cm[t] = CUDART_INF_F;
-      }
-    }
-    unsigned long long *cr = p.colres + (size_t)b * p.N1;
-    unsigned *cs = p.colsec + (size_t)b * p.N1;
-#pragma unroll
-    for (int t = 0; t < T; ++t) {
-      const int j = cbase + t;
-      if (j < p.N1) {
-        const int o = t * WARPS * 32 + threadIdx.x;
-        const unsigned mine = hg_ord(sbest[o]);
-        const unsigned long long key = ((unsigned long long)mine << 32) | (unsigned)scid[o];
-        const unsigned long long old = atomicMin(cr + j, key);
-        // the value that did NOT end up as the winner of this exchange is a runner-up
-        const unsigned loser = key < old ? (unsigned)(old >> 32) : mine;
-        atomicMin(cs + j, min(loser, hg_ord(ssec[o])));
-      }
-    }
-  }
-  __syncthreads();
-
-  unsigned long long *rr_out = p.rowres + (size_t)b * p.N2;
-  unsigned *rs_out = p.rowsec + (size_t)b * p.N2;
-  for (int r = threadIdx.x; r < p.RB; r += WARPS * 32) {
-    const int i = r0 + r;
-    if (i >= p.N2) continue;
-    float best = CUDART_INF_F, second = CUDART_INF_F;
-    unsigned code = 0xffffffffu;
-    for (int w = 0; w < WARPS; ++w) {
-      if ((blockIdx.y * WARPS + w) * 32 * T >= p.N1) break;
-      const uint4 v = rowpart[(size_t)w * (p.RB / 2) + (r >> 1)];
-      const float m = __uint_as_float((r & 1) ? v.z : v.x);
-      const unsigned near = (r & 1) ? v.w : v.y;
-      // bit 31 of the code: another lane of the winning warp is within eps2 (the finish kernel treats it as ambiguous)
-      const unsigned c = ((unsigned)(blockIdx.y * WARPS + w) << 5) | (unsigned)(__ffs(near) - 1) |
-                         ((near & (near - 1u)) ? 0x80000000u : 0u);
-      if (m < best || code == 0xffffffffu) {
-        second = fminf(second, best);
-        best = m;
-        code = c;
-      } else {
-        second = fminf(second, m);
-      }
-    }
-    const unsigned mine = hg_ord(best);
-    const unsigned long long key = ((unsigned long long)mine << 32) | code;
-    const unsigned long long old = atomicMin(rr_out + i, key);
-    const unsigned loser = key < old ? (unsigned)(old >> 32) : mine;
-    atomicMin(rs_out + i, min(loser, hg_ord(second)));
-  }
-}
-
-// Finish of the approximate path: exact minimum and first index inside the recorded cell; entries with a runner-up
-// within eps2 outside the cell go on the ambiguity list (their provisional result is written all the same).
-template <int T>
-__global__ void __launch_bounds__(256) nn_bidir_d3a_finish_kernel(NnParams p, int B, float *__restrict__ min1,
-                                                                   int *__restrict__ arg1, float *__restrict__ min2,
-                                                                   int *__restrict__ arg2) {
-  const long long total = (long long)B * (p.N1 + p.N2);
-  for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < total;
-       g += (long long)gridDim.x * blockDim.x) {
-    const int b = (int)(g / (p.N1 + p.N2));
-    const int e = (int)(g % (p.N1 + p.N2));
-    const float *gx = p.gts + (size_t)b * p.N2 * 3;
-    const float *gy = p.preds + (size_t)b * p.N1 * 3;
-    const float eps2 = p.eps2[b];
-    float m = CUDART_INF_F;
-    int arg = 0;
-    bool ambiguous;
-    if (e < p.N1) {
-      const int j = e;
-      const unsigned long long key = p.colres[(size_t)b * p.N1 + j];
-      const float best = hg_unord((unsigned)(key >> 32)), sec = hg_unord(p.colsec[(size_t)b * p.N1 + j]);
-      ambiguous = !(sec > best + eps2);
-      const int i0 = (int)(unsigned)(key & 0xffffffffu) * kColBatch;
-      const float y0 = __ldg(gy + (size_t)j * 3), y1 = __ldg(gy + (size_t)j * 3 + 1), y2 = __ldg(gy + (size_t)j * 3 + 2);
-#pragma unroll 4
-      for (int d = 0; d < kColBatch; ++d) {
-        const int i = i0 + d;
-        if (i < p.N2) {
-          const float v = nn_p_exact(__ldg(gx + (size_t)i * 3), __ldg(gx + (size_t)i * 3 + 1),
-                                     __ldg(gx + (size_t)i * 3 + 2), y0, y1, y2);
-          if (v < m) {
-            m = v;
-            arg = i;
-          }
-        }
-      }
-      min1[(size_t)b * p.N1 + j] = m;
-      arg1[(size_t)b * p.N1 + j] = arg;
-    } else {
-      const int i = e - p.N1;
-      const unsigned long long key = p.rowres[(size_t)b * p.N2 + i];
-      const float best = hg_unord((unsigned)(key >> 32)), sec = hg_unord(p.rowsec[(size_t)b * p.N2 + i]);
-      const unsigned code = (unsigned)(key & 0xffffffffu);
-      ambiguous = (code & 0x80000000u) != 0u || !(sec > best + eps2);
-      const unsigned cell = code & 0x7fffffffu;
-      const int j0 = (int)(cell >> 5) * 32 * T + (int)(cell & 31u) * T;
-      const float x0 = __ldg(gx + (size_t)i * 3), x1 = __ldg(gx + (size_t)i * 3 + 1), x2 = __ldg(gx + (size_t)i * 3 + 2);
-#pragma unroll
-      for (int d = 0; d < T; ++d) {
-        const int j = j0 + d;
-        if (j < p.N1) {
-          const float v = nn_p_exact(x0, x1, x2, __ldg(gy + (size_t)j * 3), __ldg(gy + (size_t)j * 3 + 1),
-                                     __ldg(gy + (size_t)j * 3 + 2));
-          if (v < m) {
-            m = v;
-            arg = j;
-          }
-        }
-      }
-      min2[(size_t)b * p.N2 + i] = m;
-      arg2[(size_t)b * p.N2 + i] = arg;
-    }
-    if (ambiguous) p.amb[1 + atomicAdd(p.amb, 1)] = (int)g;  // g < 2^31 is checked on the host
-  }
-}
-
-// One warp per ambiguous entry: exact scan of the whole row / column, first index among equal values.
-__global__ void __launch_bounds__(128) nn_resolve_kernel(NnParams p, float *__restrict__ min1, int *__restrict__ arg1,
-                                                         float *__restrict__ min2, int *__restrict__ arg2) {
-  const int lane = threadIdx.x & 31;
-  const int nwarps = gridDim.x * (blockDim.x >> 5);
-  const int count = p.amb[0];
-  for (int it = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); it < count; it += nwarps) {
-    const int g = p.amb[1 + it];
-    const int b = g / (p.N1 + p.N2), e = g % (p.N1 + p.N2);
-    const float *gx = p.gts + (size_t)b * p.N2 * 3;
-    const float *gy = p.preds + (size_t)b * p.N1 * 3;
-    const bool col = e < p.N1;
-    const int self = col ? e : e - p.N1, n_other = col ? p.N2 : p.N1;
-    const float *ps = (col ? gy : gx) + (size_t)self * 3, *po = col ? gx : gy;
-    const float s0 = __ldg(ps), s1 = __ldg(ps + 1), s2 = __ldg(ps + 2);
-    float m = CUDART_INF_F;
-    int arg = 0x7fffffff;
-    for (int o = lane; o < n_other; o += 32) {  // ascending per lane + strict '<': the lane's first minimum
-      const float o0 = __ldg(po + (size_t)o * 3), o1 = __ldg(po + (size_t)o * 3 + 1), o2 = __ldg(po + (size_t)o * 3 + 2);
-      const float v = col ? nn_p_exact(o0, o1, o2, s0, s1, s2) : nn_p_exact(s0, s1, s2, o0, o1, o2);
-      if (v < m) {
-        m = v;
-        arg = o;
-      }
-    }
-    const float wm = hg_warp_min_f32(m);
-    const int wa = __reduce_min_sync(0xffffffffu, (m == wm) ? arg : 0x7fffffff);
-    if (lane == 0) {
-      const int a = wa == 0x7fffffff ? 0 : wa;  // all +inf / NaN: index 0, as the exact path
-      if (col) {
-        min1[(size_t)b * p.N1 + self] = wm;
-        arg1[(size_t)b * p.N1 + self] = a;
-      } else {
-        min2[(size_t)b * p.N2 + self] = wm;
-        arg2[(size_t)b * p.N2 + self] = a;
-      }
-    }
-  }
-}
-
 // ---- generic inner dimension (R3: HiT_ADV.py:229-231 feeds [B,3,K], i.e. N=3 "points" of dimension K) ------
 // One thread per matrix entry, sequential FMA chain over D (the order the oracle uses).  Small problems only.
 __global__ void nn_generic_p_kernel(const float *__restrict__ gts, const float *__restrict__ preds, int B, int N2,
@@ -918,13 +582,13 @@ __global__ void __launch_bounds__(256) set_loss_bwd_kernel(
   }
 }
 
-template <int T, int WARPS, bool APPROX>
+template <int T, int WARPS>
 int launch_main(const NnParams &p, int B, cudaStream_t stream) {
   const int ncg = (p.N1 + 32 * T - 1) / (32 * T);
   dim3 grid((p.N2 + p.RB - 1) / p.RB, (ncg + WARPS - 1) / WARPS, B);
   const size_t smem = (size_t)(p.RB + 4) * sizeof(float4) + (size_t)WARPS * (p.RB / 2) * sizeof(uint4) +
-                      (size_t)(APPROX ? 3 : 2) * T * WARPS * 32 * sizeof(float);
-  auto kernel = APPROX ? nn_bidir_d3a_kernel<T, WARPS> : nn_bidir_d3_kernel<T, WARPS>;
+                      (size_t)2 * T * WARPS * 32 * sizeof(float);
+  auto kernel = nn_bidir_d3_kernel<T, WARPS>;
   if (smem > 48 * 1024) {
     HG_REQUIRE(smem <= 200 * 1024, HG_E_UNSUPPORTED, "nn_bidir: RB=%d needs %zu bytes of shared memory", p.RB, smem);
     HG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -936,11 +600,11 @@ int launch_main(const NnParams &p, int B, cudaStream_t stream) {
   return HG_OK;
 }
 
-template <int T, bool APPROX>
+template <int T>
 int launch_warps(const NnParams &p, int B, int ncg, cudaStream_t stream) {
-  return (ncg >= 4 && ncg % 4 == 0) ? launch_main<T, 4, APPROX>(p, B, stream)
-         : (ncg >= 2)               ? launch_main<T, 2, APPROX>(p, B, stream)
-                                    : launch_main<T, 1, APPROX>(p, B, stream);
+  return (ncg >= 4 && ncg % 4 == 0) ? launch_main<T, 4>(p, B, stream)
+         : (ncg >= 2)               ? launch_main<T, 2>(p, B, stream)
+                                    : launch_main<T, 1>(p, B, stream);
 }
 
 int grid_for(long long total, int threads) {
@@ -956,29 +620,24 @@ int grid_for(long long total, int threads) {
 // Tunables exposed for the benchmark sweep (not part of the stable ABI): T (columns per lane: 8 or 16) and
 // rows per CTA.  0 = automatic.
 static int g_force_T = 0, g_force_RB = 0;
-// hg_tune("nn_exact", 0) selects the approximate tracker (nn_bidir_d3a_kernel).  It is NOT the default: on a B200 its
-// main loop runs at 58.0 % of the FP32 peak against 53.6 % for the exact tracker (1024 x 16384), but 2.4 % of the
-// entries are near-ties at that density and their exact re-scans cost more than the loop saves (whole call 80 ms
-// against 57 ms; profiles/r02_experiment_nn_approx_tracker.txt).  Kept, tested bit for bit, as the measured experiment.
-int g_hg_tune_nn_exact = 1;
 int g_hg_tune_small_fused_off = 0;
 HG_API void hg_nn_bidir_tune(int T, int RB) {
   g_force_T = T;
   g_force_RB = RB;
 }
 
-// D = 3: merged (value, cell) keys and runner-up values (the part each call resets to 0xff), per-cloud error bound,
-// ambiguity list, then the kd-tree orderings of both clouds (0 bytes where the pruned path does not apply)
+// D = 3: merged (value, cell) keys of both directions (the part each call resets to 0xff), a reserved region, then the
+// kd-tree orderings of both clouds (0 bytes where the pruned path does not apply)
 struct NnD3Workspace {
-  float *eps2;
+  size_t keys_bytes;
   void *gts_order, *preds_order;
   NnD3Workspace(HgCarve &c, int B, int N2, int N1, NnParams *p) {
     p->colres = c.take<unsigned long long>((size_t)B * N1);
     p->rowres = c.take<unsigned long long>((size_t)B * N2);
-    p->colsec = c.take<unsigned>((size_t)B * N1);
-    p->rowsec = c.take<unsigned>((size_t)B * N2);
-    p->eps2 = eps2 = c.take<float>(B);
-    p->amb = c.take<int>((size_t)B * (N1 + N2) + 1);
+    keys_bytes = c.bytes;
+    // unused: keeps hg_nn_bidir_workspace_bytes at the sizes tests/test_cpu_workspace_sizes.py pins as C ABI
+    c.take<char>(hg_align((size_t)B * N1 * 4) + hg_align((size_t)B * N2 * 4) + hg_align((size_t)B * 4) +
+                 hg_align(((size_t)B * (N1 + N2) + 1) * 4));
     gts_order = c.span(hg_prune_order_bytes(B, N2)).ptr;
     preds_order = c.span(hg_prune_order_bytes(B, N1)).ptr;
   }
@@ -1051,14 +710,7 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
     p.only_a = og.info;
     p.only_b = op.info;
   }
-  // the approximate tracker (4 FMA-pipe operations per pair, exact recovery in the finish kernels) when switched on
-  const bool approx = !prune && !g_hg_tune_nn_exact && (double)B * (N1 + N2) < 2.0e9;
-  HG_CUDA(cudaMemsetAsync(workspace, 0xff, (size_t)((char *)w.eps2 - (char *)workspace), stream));
-  if (approx) {
-    HG_CUDA(cudaMemsetAsync(p.amb, 0, sizeof(int), stream));
-    nn_eps_kernel<<<B, 256, 0, stream>>>(gts, preds, N2, N1, w.eps2);
-    HG_CHECK_LAUNCH("nn_eps_kernel");
-  }
+  HG_CUDA(cudaMemsetAsync(workspace, 0xff, w.keys_bytes, stream));
 
   // columns per lane: 16 halves the row broadcasts per pair but needs 12-warp occupancy to pay (tools/debug/nn_sweep.py,
   // B200: 8 wins by 6 % at 2048 points, 2 % at 4096, level at 8192, loses from there)
@@ -1082,23 +734,9 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
   p.RB = RB;
   if (T != 16) T = 8;
   const int ncg = (N1 + 32 * T - 1) / (32 * T);
-  int rc;
-  if (approx)
-    rc = T == 16 ? launch_warps<16, true>(p, B, ncg, stream) : launch_warps<8, true>(p, B, ncg, stream);
-  else
-    rc = T == 16 ? launch_warps<16, false>(p, B, ncg, stream) : launch_warps<8, false>(p, B, ncg, stream);
+  const int rc = T == 16 ? launch_warps<16>(p, B, ncg, stream) : launch_warps<8>(p, B, ncg, stream);
   if (rc) return rc;
   const long long total = (long long)B * (N1 + N2);
-  if (approx) {
-    if (T == 16)
-      nn_bidir_d3a_finish_kernel<16><<<grid_for(total, 256), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
-    else
-      nn_bidir_d3a_finish_kernel<8><<<grid_for(total, 256), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
-    HG_CHECK_LAUNCH("nn_bidir_d3a_finish_kernel");
-    nn_resolve_kernel<<<hg_sm_count() * 4, 128, 0, stream>>>(p, min1, arg1, min2, arg2);
-    HG_CHECK_LAUNCH("nn_resolve_kernel");
-    return HG_OK;
-  }
   {
     const int tshift = T == 16 ? 4 : 3;
     const size_t sx = (size_t)(N2 + (N2 >> 5) + 1), sy = (size_t)(N1 + (N1 >> tshift) + 1);

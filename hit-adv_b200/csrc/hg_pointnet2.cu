@@ -335,7 +335,7 @@ int launch_scatter_unweighted(const float *grad_out, const HgCsr &csr, int b, in
   const size_t smem = (size_t)E * sizeof(float);
   const long long planes = (long long)b * c;
   const bool bulk_ok = 2 * smem <= 200 * 1024 && E >= n && (E & 3) == 0 && (reinterpret_cast<uintptr_t>(grad_out) & 15) == 0;
-  if (bulk_ok && g_hg_tune_scatter != 1 && (planes >= 2LL * hg_sm_count() || g_hg_tune_scatter >= 2)) {
+  if (bulk_ok && planes >= 2LL * hg_sm_count()) {
     static HgPerDeviceOnce once;
     if (once.first()) {
       HG_CUDA(cudaFuncSetAttribute(scatter_bulk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
@@ -347,7 +347,7 @@ int launch_scatter_unweighted(const float *grad_out, const HgCsr &csr, int b, in
     const size_t limit = 220 * 1024;
     long long cap = fixed < limit ? (long long)((limit - fixed) / sizeof(unsigned short)) : 0;
     if (cap > 4LL * E) cap = 4LL * E;
-    const bool list_smem = cap >= (long long)E + 32LL * ((n + 31) / 32) && E <= 65535 && g_hg_tune_scatter != 3;
+    const bool list_smem = cap >= (long long)E + 32LL * ((n + 31) / 32) && E <= 65535;
     const size_t dyn = list_smem ? fixed + (size_t)cap * sizeof(unsigned short) : 2 * smem;
     const int per_sm = (dyn <= 100 * 1024) ? 2 : 1;
     long long grid = (long long)hg_sm_count() * per_sm;
@@ -702,8 +702,7 @@ int launch_fps(const float *dataset, int b, int n, int m, const long long *start
   }
   // threads per cloud: the round is a latency chain (update -> warp max -> barrier -> block max), so small clouds run
   // on ONE warp per scheduler (128 threads, <= 8 points per thread) and do not contend for issue slots
-  int th = n > 4096 ? 1024 : (n > 2048 ? 256 : 128);
-  if (g_hg_tune_fps_threads == 128 || g_hg_tune_fps_threads == 256) th = n <= 128 * 16 ? g_hg_tune_fps_threads : th;
+  const int th = n > 4096 ? 1024 : (n > 2048 ? 256 : 128);
   const int ppt = (n + th - 1) / th;
 #define HG_FPS_CASE(P, TH)                                                                                \
   if (th == TH && ppt <= P) {                                                                             \
@@ -718,10 +717,6 @@ int launch_fps(const float *dataset, int b, int n, int m, const long long *start
   HG_FPS_CASE(4, 128)
   HG_FPS_CASE(8, 128)
   HG_FPS_CASE(16, 128)
-  HG_FPS_CASE(1, 256)
-  HG_FPS_CASE(2, 256)
-  HG_FPS_CASE(4, 256)
-  HG_FPS_CASE(8, 256)
   HG_FPS_CASE(16, 256)
   HG_FPS_CASE(8, 1024)
   HG_FPS_CASE(16, 1024)

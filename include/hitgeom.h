@@ -54,14 +54,11 @@ int hg_probe_fp32_peak(float *tflops, float *device_scratch, hgStream stream);
 #define HG_PROF_FPS 2      /* fps_kernel */
 #define HG_PROF_GROUP 3    /* gather_channel_major_kernel (group_points / gather_points) */
 #define HG_PROF_NTAGS 4
-/* Development knobs for A/B measurements (not part of the stable ABI): "scatter" = 0 auto / 1 staged / 2 bulk-copy;
+/* Development knobs for A/B measurements (not part of the stable ABI; an unknown key returns HG_E_BADARG):
  * "knn_tc" = 1 switches the tensor-core kNN kernel off, 2 forces it for small batches, 5 forces it with the
  * single-sweep threshold;
- * "nn_exact" = 0 runs the experimental 4-operation approximate tracker (+ exact recovery) in hg_nn_bidir_f32
- * instead of the default 5-operation exact tracker (same results; see hg_nn_bidir.cu for why it is not the default);
  * "small_fused" = 1 sends clouds that fit in shared memory down the general finish / kNN-backward kernels as well
- * (same results; the tests run both); "knn_win" = Z-order window of the small-cloud kNN seeds (0 = default);
- * "fps_threads" = 128 | 256 threads per cloud in furthest point sampling for clouds up to 2048 points (0 = default);
+ * (same results; the tests run both);
  * "prune" = 0 switches the pruned passes off, "prune_min_n" moves their size threshold, "prune_count" = 1 counts visited
  * leaf pairs, self-kNN drains and orderings; "prune_refit_tol" = rebuild tolerance of an ordering state's refit
  * [permille] (0 = default), "prune_refit_stage" = 1 stages the cloud in shared memory for the refit's gather, 2 reads it

@@ -48,6 +48,20 @@ def test_packed_fp32_and_warp_reduce_instructions_present():
         assert mnemonic in sass, mnemonic
 
 
+def test_tune_keys():
+    """hg_tune accepts the knobs the suite sets and refuses removed ones (it only sets host flags: no device needed)."""
+    import hitgeom
+
+    L = hitgeom.lib()
+    for key in (b"nn_exact", b"fps_threads", b"scatter", b"knn_win"):
+        assert L.hg_tune(key, 0) != 0, key
+        assert key in L.hg_last_error()
+    defaults = {b"knn_tc": 0, b"small_fused": 0, b"prune": 1, b"prune_min_n": 0, b"prune_count": 0,
+                b"prune_refit_stage": 0}
+    for key, value in defaults.items():
+        assert L.hg_tune(key, value) == 0, key
+
+
 def test_product_never_imports_the_oracle():
     bad = []
     for dirpath, _, files in os.walk(PKG):

@@ -21,18 +21,15 @@ def F():
     return functional
 
 
-@pytest.fixture(autouse=True, params=["approx-tracker", "exact-tracker", "exact-tracker-gather-finish"])
+@pytest.fixture(autouse=True, params=["exact-tracker", "exact-tracker-gather-finish"])
 def _tracker(request):
-    """Every test of this module runs three times: with the default distance pass (5-operation exact tracker; clouds
-    that fit in shared memory finish in nn_bidir_d3_finish_small_kernel), with the general gather finish kernel forced
-    for small clouds too (hg_tune("small_fused", 1)), and with the experimental 4-operation approximate tracker + exact
-    recovery in the finish kernels (hg_tune("nn_exact", 0), hg_nn_bidir.cu).  All must give the reference's bits."""
+    """Every test of this module runs twice: with the default distance pass (5-operation exact tracker; clouds that fit
+    in shared memory finish in nn_bidir_d3_finish_small_kernel), and with the general gather finish kernel forced for
+    small clouds too (hg_tune("small_fused", 1)).  Both must give the reference's bits."""
     from hitgeom._lib import lib
 
-    lib().hg_tune(b"nn_exact", 0 if request.param == "approx-tracker" else 1)
     lib().hg_tune(b"small_fused", 1 if request.param == "exact-tracker-gather-finish" else 0)
     yield request.param
-    lib().hg_tune(b"nn_exact", 1)
     lib().hg_tune(b"small_fused", 0)
 
 
@@ -266,10 +263,10 @@ def test_backward_with_hub_points_vs_oracle(oracle):
 
 @pytest.mark.parametrize("case", ["dups across batches", "far from origin", "all equal", "lattice", "tiny spacings"])
 def test_nn_bidir_ambiguous_inputs_vs_oracle(oracle, F, case):
-    """Inputs built to defeat the approximate tracker: exact duplicates spread over different 32-row batches and
-    different lanes (runner-up == winner), clouds far from the origin (the error bound eps2 ~ 1e-6 * |p|^2 exceeds the
-    nearest-neighbour gaps: everything is ambiguous), a cloud of identical points, an integer lattice (massive exact
-    ties), and spacings of a few ulp.  Values and first indices must be the oracle's, bit for bit."""
+    """Inputs full of ties and near-ties: exact duplicates spread over different 32-row batches and different lanes,
+    clouds far from the origin (rounding of |p|^2 larger than the nearest-neighbour gaps), a cloud of identical points,
+    an integer lattice (massive exact ties), and spacings of a few ulp.  Values and first indices must be the oracle's,
+    bit for bit."""
     rng = np.random.default_rng(len(case))
     B, N = 2, 1500
     gts = clouds(B, N, 17, "gauss")

@@ -4,10 +4,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 for p in (ROOT, os.path.join(ROOT, "hit-adv_b200"), os.path.join(ROOT, "tools")):
     sys.path.insert(0, p)
 import torch
-from hitgeom import functional as F, _lib
+from hitgeom import functional as F
 from bench import make_clouds
 from bench_ops import timeit
-from hitgeom.pointnet2_ops import _ext
 
 flush = (torch.empty(256 << 20, dtype=torch.uint8, device="cuda"), torch.zeros(64 << 20, dtype=torch.float32, device="cuda"))
 SHAPES = ((32, 1024, 20), (32, 1024, 6), (388, 1024, 6), (388, 1024, 20), (64, 2048, 6), (32, 2048, 20), (16, 4096, 6))
@@ -28,13 +27,4 @@ for B, N, k1 in SHAPES:
             except Exception as e:
                 line += f" q{qt}g{gp} n/a"
     F.force_knn_shape(0, 0)
-    print(line, flush=True)
-for B, N, M in ((64, 3000, 512), (64, 4096, 512), (16, 4096, 1024)):
-    x = torch.randn(B, N, 3, device="cuda")
-    line = f"FPS B={B} N={N} M={M}:"
-    for th in (128, 256):
-        _lib.lib().hg_tune(b"fps_threads", th)
-        line += f" threads={th} {timeit(lambda: _ext.furthest_point_sampling(x, M), flush=flush) * 1e3:7.1f} us"
-    _lib.lib().hg_tune(b"fps_threads", 0)
-    line += f" auto {timeit(lambda: _ext.furthest_point_sampling(x, M), flush=flush) * 1e3:7.1f} us"
     print(line, flush=True)
