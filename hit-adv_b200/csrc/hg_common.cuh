@@ -77,6 +77,14 @@ template <typename Layout, typename... A> size_t hg_layout_bytes(A... a) { HgCar
 template <typename Layout, typename... A> Layout hg_layout_at(void *base, A... a) { HgCarve c(base); return Layout(c, a...); }
 
 int hg_sm_count();
+// blocks of `threads` for a grid-stride loop over `total` items: enough to cover them, at most per_sm per SM, at least one
+static inline int hg_grid_for(long long total, int threads, int per_sm) {
+  long long blocks = (total + threads - 1) / threads;
+  const long long cap = (long long)hg_sm_count() * per_sm;
+  if (blocks > cap) blocks = cap;
+  if (blocks < 1) blocks = 1;
+  return (int)blocks;
+}
 // true the first time it is called on the current device with this flag array (function attributes such as the
 // dynamic shared-memory limit are per device: one `static` flag per process would miss the second GPU)
 struct HgPerDeviceOnce {
@@ -125,6 +133,23 @@ __device__ __forceinline__ unsigned hg_ord(float f) {
 }
 __device__ __forceinline__ float hg_unord(unsigned u) {
   return __uint_as_float((u & 0x80000000u) ? (u ^ 0x80000000u) : ~u);
+}
+
+// d into the ascending list v of the KM smallest values so far, without branches: each level keeps the smaller and passes
+// the larger on.  fminf / fmaxf drop a NaN d, and the level then duplicates its entry: keep NaN out of d.
+template <int KM>
+__device__ __forceinline__ void hg_sorted_min_insert(float (&v)[KM], float d) {
+#pragma unroll
+  for (int u = 0; u < KM; ++u) {
+    const float lo = fminf(v[u], d);
+    d = fmaxf(v[u], d);
+    v[u] = lo;
+  }
+}
+
+// the next float above v (+inf for +inf and NaN): turns a bound that a strict '<' filter tests into one that keeps ties
+__device__ __forceinline__ float hg_nudge_up(float v) {
+  return v < CUDART_INF_F ? nextafterf(v, CUDART_INF_F) : CUDART_INF_F;
 }
 
 __device__ __forceinline__ float hg_warp_min_f32(float v) {
@@ -246,12 +271,9 @@ int hg_prune_knn_search(const HgPruneOrder &o, int B, int k1, const float *thr0,
                         cudaStream_t stream);
 
 // ---- 3-D streaming kNN (hg_knn3.cu) ---------------------------------------------------------------------------
-#define HG_KNN_FORM_EXPANDED 0  // dist = (xx_j + (-2 zz)) + xx_i   (KNNDist / DGCNN)
-#define HG_KNN_FORM_DIRECT 1    // dist = fma(dz,dz, fma(dy,dy, dx*dx))   (pytorch3d knn_points)
-int hg_knn3_launch_i32(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, int *idx,
+// pytorch3d knn_points: the K nearest of p2 to every point of p1, with its arithmetic (arguments checked by the caller)
+int hg_knn3_points_i64(const float *p1, const float *p2, int B, int N, int M, int K, float *dists, long long *idx,
                        cudaStream_t stream);
-int hg_knn3_launch_i64(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals,
-                       long long *idx, cudaStream_t stream);
 // 3-D self-kNN (expanded form), every route: hg_knn_self_temporal_order_f32 with C = 3 (arguments checked there)
 size_t hg_knn3_self_workspace_bytes(int B, int N, int k1);
 int hg_knn3_self_i32(const float *pc, int B, int N, int k1, float *vals, int *idx, int *idx_state, int state_valid,

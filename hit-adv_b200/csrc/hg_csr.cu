@@ -341,14 +341,12 @@ int hg_csr_build_unordered(const int *keys, int B, int E, int N, void *workspace
   const auto [off, cursor, list] = hg_layout_at<CsrLayout>(workspace, B, N, E, false);
   HG_CUDA(cudaMemsetAsync(off, 0, (size_t)B * (N + 1) * sizeof(int), stream));
   const long long total = (long long)B * E;
-  long long blocks = (total + 255) / 256;
-  const long long cap = (long long)hg_sm_count() * 16;
-  if (blocks > cap) blocks = cap;
-  csr_count_kernel<<<(int)blocks, 256, 0, stream>>>(keys, total, E, N, off);
+  const int blocks = hg_grid_for(total, 256, 16);
+  csr_count_kernel<<<blocks, 256, 0, stream>>>(keys, total, E, N, off);
   HG_CHECK_LAUNCH("csr_count_kernel");
   csr_scan_kernel<<<B, 256, 0, stream>>>(N, off, cursor);
   HG_CHECK_LAUNCH("csr_scan_kernel");
-  csr_fill_kernel<<<(int)blocks, 256, 0, stream>>>(keys, total, E, N, cursor, list);
+  csr_fill_kernel<<<blocks, 256, 0, stream>>>(keys, total, E, N, cursor, list);
   HG_CHECK_LAUNCH("csr_fill_kernel");
   out->off = off;
   out->list = list;

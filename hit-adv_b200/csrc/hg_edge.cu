@@ -240,9 +240,7 @@ HG_API int hg_edge_feature_grad_f32(const float *grad_out, const int64_t *idx, i
   const int E = N * k;
   const auto w = hg_layout_at<HgKeysCsr>(workspace, B, N, (long long)E, true);
   const long long te = (long long)B * E;
-  long long kb = (te + 255) / 256;
-  if (kb > (long long)hg_sm_count() * 32) kb = (long long)hg_sm_count() * 32;
-  edge_keys_kernel<<<(int)kb, 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
+  edge_keys_kernel<<<hg_grid_for(te, 256, 32), 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
   HG_CHECK_LAUNCH("edge_keys_kernel");
   HgCsr csr;
   // stable build (ascending edge order inside every segment): kNN graphs of high-dimensional features have hubs

@@ -237,10 +237,7 @@ HG_API int hg_chamfer_knn_step_host_f32(hgHostStep *s, const float *adv_h, const
     if (rc) return rc;
     {
       const long long n = (long long)pts * 3;
-      long long blocks = (n + 255) / 256;
-      const long long cap = (long long)hg_sm_count() * 16;
-      if (blocks > cap) blocks = cap;
-      host_step_add_kernel<<<(int)blocks, 256, 0, st>>>(sl.grad_ch, sl.grad_knn, n);
+      host_step_add_kernel<<<hg_grid_for(n, 256, 16), 256, 0, st>>>(sl.grad_ch, sl.grad_knn, n);
       HG_CHECK_LAUNCH("host_step_add_kernel");
     }
     HG_CUDA(cudaEventRecord(sl.comp_done, st));

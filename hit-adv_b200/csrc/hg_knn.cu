@@ -552,14 +552,6 @@ __global__ void __launch_bounds__(256) knn_outlier_bwd_small_kernel(const float 
   }
 }
 
-int grid_for(long long total, int threads) {
-  long long blocks = (total + threads - 1) / threads;
-  const long long cap = (long long)hg_sm_count() * 16;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  return (int)blocks;
-}
-
 constexpr size_t kGenericScratchBytes = (size_t)256 << 20;
 
 // feature clouds: squared norms [B,K], then distance matrices for nb clouds (as many as kGenericScratchBytes holds, >= 1)
@@ -615,7 +607,7 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
   HG_REQUIRE(rows_fit || g_hg_tune_knn_tc_off != 1, HG_E_UNSUPPORTED,
              "knn_self: hg_tune(\"knn_tc\", 1) selects the FP32 path, which takes K <= 12800 (got K=%d)", K);
   const auto [nb, xx, dist] = hg_layout_at<KnnGenericWorkspace>(workspace, B, K);
-  knn_sumsq_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, (long long)B * K, C, xx);
+  knn_sumsq_kernel<<<hg_grid_for((long long)B * K, 256, 16), 256, 0, stream>>>(pc, (long long)B * K, C, xx);
   HG_CHECK_LAUNCH("knn_sumsq_kernel");
   // feature clouds of DGCNN's shapes: tensor-core filter fused with the exact FP32 evaluation (hg_knn_tc.cu); everything
   // else (and hg_tune("knn_tc", 1)) takes the FP32 distance tile + row select below
@@ -641,7 +633,7 @@ HG_API int hg_knn_self_temporal_order_f32(const float *pc, int B, int K, int C, 
     knn_dist_generic_kernel<<<grid, 256, 0, stream>>>(pc + (size_t)b0 * K * C, xx + (size_t)b0 * K, K, C, dist);
     HG_CHECK_LAUNCH("knn_dist_generic_kernel");
     const int nrows = cb * K;
-    (long_list ? knn_select_rows_kernel<true> : knn_select_rows_kernel<false>)<<<grid_for((long long)nrows * 32, 128),
+    (long_list ? knn_select_rows_kernel<true> : knn_select_rows_kernel<false>)<<<hg_grid_for((long long)nrows * 32, 128, 16),
                                                                                  128, sel_smem, stream>>>(
         dist, nrows, K, k1, vals ? vals + (size_t)b0 * K * k1 : nullptr, idx + (size_t)b0 * K * k1);
     HG_CHECK_LAUNCH("knn_select_rows_kernel");
@@ -656,7 +648,7 @@ HG_API int hg_knn_points_f32(const float *p1, const float *p2, int B, int N, int
   HG_REQUIRE(B > 0 && N > 0 && M > 0, HG_E_BADARG, "knn_points: sizes must be positive");
   HG_REQUIRE(K >= 1 && K <= 64 && K <= M, HG_E_BADARG, "knn_points: need 1 <= K <= min(64, M); got K=%d M=%d", K, M);
   HG_REQUIRE(B <= 65535, HG_E_UNSUPPORTED, "knn_points: B=%d > 65535 clouds per call", B);
-  return hg_knn3_launch_i64(HG_KNN_FORM_DIRECT, p1, p2, B, N, M, K, dists, (long long *)idx, hg_stream(stream_));
+  return hg_knn3_points_i64(p1, p2, B, N, M, K, dists, (long long *)idx, hg_stream(stream_));
 }
 
 HG_API int hg_knn_outlier_fwd_f32(const float *vals, int B, int K, int k1, float alpha, const float *weights,
@@ -694,13 +686,13 @@ HG_API int hg_knn_outlier_bwd_f32(const float *pc, const int *idx, const float *
   }
   const auto w = hg_layout_at<HgKeysCsr>(workspace, B, K, (long long)K * k1, false);
   const long long total = (long long)B * K * k1;
-  knn_bwd_keys_kernel<<<grid_for(total, 256), 256, 0, stream>>>(idx, mask, total, k1, w.keys);
+  knn_bwd_keys_kernel<<<hg_grid_for(total, 256, 16), 256, 0, stream>>>(idx, mask, total, k1, w.keys);
   HG_CHECK_LAUNCH("knn_bwd_keys_kernel");
   HgCsr csr;
   int rc = hg_csr_build_unordered(w.keys, B, K * k1, K, w.csr.ptr, w.csr.bytes, &csr, stream);
   if (rc) return rc;
-  knn_outlier_bwd_kernel<<<grid_for((long long)B * K, 256), 256, 0, stream>>>(pc, idx, mask, g, csr.off, csr.list, w.keys,
-                                                                              B, K, C, k1, grad_pc);
+  knn_outlier_bwd_kernel<<<hg_grid_for((long long)B * K, 256, 16), 256, 0, stream>>>(pc, idx, mask, g, csr.off, csr.list, w.keys,
+                                                                                     B, K, C, k1, grad_pc);
   HG_CHECK_LAUNCH("knn_outlier_bwd_kernel");
   return HG_OK;
 }

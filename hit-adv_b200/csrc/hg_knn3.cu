@@ -21,10 +21,14 @@
 // strict '<' => equal values keep the lowest index first: the canonical tie order of the oracle.
 #include "hg_common.cuh"
 
+#include <type_traits>
+
 namespace {
 
 constexpr int kThreads = 128;
 
+#define HG_KNN_FORM_EXPANDED 0  // dist = (xx_j + (-2 zz)) + xx_i   (KNNDist / DGCNN)
+#define HG_KNN_FORM_DIRECT 1    // dist = fma(dz,dz, fma(dy,dy, dx*dx))   (pytorch3d knn_points)
 // internal third form (see filter_addend): EXPANDED values and indices, 4-operation folded filter
 #define HG_KNN_FORM_EXPANDED_FOLD4 2
 __host__ __device__ constexpr bool knn_form_expanded(int form) { return form != HG_KNN_FORM_DIRECT; }
@@ -131,6 +135,49 @@ struct TopK {
     }
   }
 };
+
+// Drain of flagged group grp of the staged pairs (candidates base + 2*GP*grp ...): the group is re-evaluated with the
+// same packed filter arithmetic to find WHICH of its 2*GP candidates are below the threshold, and only those are
+// evaluated exactly and inserted.  The insertion code (the expensive part) is thus reached once per group by all lanes
+// together, not once per candidate slot.
+template <int FORM, int KM, int GP>
+__device__ __forceinline__ void knn_drain_group(float a0, float a1, float a2, float a3, float af, TopK<KM> &top,
+                                                const float4 *cand, int grp, int base) {
+  const float4 *cp = cand + 2 * GP * grp;
+  unsigned sub = 0u;  // after 2*GP shifts, bit 2*GP-1-c belongs to candidate c of the group
+#pragma unroll
+  for (int u = 0; u < GP; ++u) {
+    const float4 cA = cp[2 * u], cB = cp[2 * u + 1];
+    const float2 e = filter_value<FORM>(a0, a1, a2, af, cA, cB);
+    sub = __funnelshift_l(__float_as_uint(e.x), sub, 1);
+    sub = __funnelshift_l(__float_as_uint(e.y), sub, 1);
+  }
+  while (sub) {
+    const int sp = 31 - __clz(sub);
+    sub &= ~(1u << sp);
+    const int c = 2 * GP - 1 - sp;
+    const float4 cA = cp[2 * (c >> 1)], cB = cp[2 * (c >> 1) + 1];
+    const bool hi = c & 1;
+    top.push(knn_dist_exact<FORM>(a0, a1, a2, a3, hi ? cA.y : cA.x, hi ? cA.w : cA.z, hi ? cB.y : cB.x, hi ? cB.w : cB.z),
+             base + 2 * GP * grp + c);
+  }
+}
+
+// the first k1 entries of query i's list (nothing past Nq); idx_state, when given, gets a second copy of the indices
+template <int KM, typename IdxT>
+__device__ __forceinline__ void knn_write_list(const TopK<KM> &top, int b, int i, int Nq, int k1, float *vals, IdxT *idx,
+                                               int *idx_state) {
+  if (i < Nq) {
+#pragma unroll
+    for (int s = 0; s < KM; ++s) {
+      if (s < k1) {
+        if (vals) vals[((size_t)b * Nq + i) * k1 + s] = top.v[s];
+        idx[((size_t)b * Nq + i) * k1 + s] = (IdxT)top.id[s];
+        if (idx_state) idx_state[((size_t)b * Nq + i) * k1 + s] = top.id[s];
+      }
+    }
+  }
+}
 
 // KM >= k1 list entries are kept; the first k1 are written out.
 // GP = candidate pairs per hit bit; a tile is 32 groups (one 32-bit mask per query) = 64*GP candidates.
@@ -254,25 +301,7 @@ __global__ void __launch_bounds__(kThreads) knn3_kernel(const float *__restrict_
           const int pos = 31 - __clz(m);
           m &= ~(1u << pos);
           const int grp = g0 + cnt - 1 - pos;
-          const float4 *cp = cand + 2 * GP * grp;
-          unsigned sub = 0u;  // after 2*GP shifts, bit 2*GP-1-c belongs to candidate c of the group
-#pragma unroll
-          for (int u = 0; u < GP; ++u) {
-            const float4 cA = cp[2 * u], cB = cp[2 * u + 1];
-            const float2 e = filter_value<FORM>(a0[t], a1[t], a2[t], af[t], cA, cB);
-            sub = __funnelshift_l(__float_as_uint(e.x), sub, 1);
-            sub = __funnelshift_l(__float_as_uint(e.y), sub, 1);
-          }
-          while (sub) {
-            const int sp = 31 - __clz(sub);
-            sub &= ~(1u << sp);
-            const int c = 2 * GP - 1 - sp;
-            const float4 cA = cp[2 * (c >> 1)], cB = cp[2 * (c >> 1) + 1];
-            const bool hi = c & 1;
-            top[t].push(knn_dist_exact<FORM>(a0[t], a1[t], a2[t], a3[t], hi ? cA.y : cA.x, hi ? cA.w : cA.z,
-                                             hi ? cB.y : cB.x, hi ? cB.w : cB.z),
-                        base + 2 * GP * grp + c);
-          }
+          knn_drain_group<FORM, KM, GP>(a0[t], a1[t], a2[t], a3[t], af[t], top[t], cand, grp, base);
         }
         mask[t] = 0u;
         af[t] = filter_addend<FORM>(a3[t], fminf(seed[t], top[t].v[KM - 1]), S[t]);
@@ -283,19 +312,8 @@ __global__ void __launch_bounds__(kThreads) knn3_kernel(const float *__restrict_
   }
 
 #pragma unroll
-  for (int t = 0; t < QT; ++t) {
-    const int i = (blockIdx.x * QT + t) * kThreads + tid;
-    if (i < Nq) {
-#pragma unroll
-      for (int s = 0; s < KM; ++s) {
-        if (s < k1) {
-          if (vals) vals[((size_t)b * Nq + i) * k1 + s] = top[t].v[s];
-          idx[((size_t)b * Nq + i) * k1 + s] = (IdxT)top[t].id[s];
-          if (idx_state) idx_state[((size_t)b * Nq + i) * k1 + s] = top[t].id[s];
-        }
-      }
-    }
-  }
+  for (int t = 0; t < QT; ++t)
+    knn_write_list(top[t], b, (blockIdx.x * QT + t) * kThreads + tid, Nq, k1, vals, idx, idx_state);
 }
 
 // ---- small clouds (< 2k points): whole candidate set resident in shared memory, drain deferred -----------------
@@ -368,7 +386,9 @@ __global__ void __launch_bounds__(kThreads) knn3_small_kernel(const float *__res
   }
   __syncthreads();
 
-  // flagged groups of the pending words of query t, ascending; thresholds refreshed after every group
+  // flagged groups of the pending words of query t, ascending; thresholds refreshed after every group.  The group drain
+  // (and the staging, query set-up and filter above) repeat knn3_kernel's: the shared helpers compile to different
+  // machine code for this kernel, knn_drain_group included.
   auto drain = [&](int t) {
     unsigned pend = nz[t], m = 0u;
     int w = 0;
@@ -447,19 +467,8 @@ __global__ void __launch_bounds__(kThreads) knn3_small_kernel(const float *__res
   for (int t = 0; t < QT; ++t) drain(t);
 
 #pragma unroll
-  for (int t = 0; t < QT; ++t) {
-    const int i = (blockIdx.x * QT + t) * kThreads + tid;
-    if (i < N) {
-#pragma unroll
-      for (int s = 0; s < KM; ++s) {
-        if (s < k1) {
-          if (vals) vals[((size_t)b * N + i) * k1 + s] = top[t].v[s];
-          idx[((size_t)b * N + i) * k1 + s] = top[t].id[s];
-          if (idx_state) idx_state[((size_t)b * N + i) * k1 + s] = top[t].id[s];
-        }
-      }
-    }
-  }
+  for (int t = 0; t < QT; ++t)
+    knn_write_list(top[t], b, (blockIdx.x * QT + t) * kThreads + tid, N, k1, vals, idx, idx_state);
 }
 
 // Seeds for the small-cloud kernel.  One CTA per cloud sorts the cloud along a Z-order (Morton) curve in shared memory
@@ -470,6 +479,27 @@ __global__ void __launch_bounds__(kThreads) knn3_small_kernel(const float *__res
 // to the local density, where a fixed neighbourhood of grid cells is empty in the tails of a cloud and crowded at its
 // centre.  Any bound would be CORRECT -- the main kernel drains early when a bound is loose -- a good one keeps it fast.
 constexpr int kMortonBits = 4, kMortonCells = 1 << (3 * kMortonBits);
+
+// Upper bound on max |p|^2 over a bounding box whose lo x, y, z, hi x, y, z lie `stride` floats apart: its farthest
+// corner, widened for rounding (the folded filter's slack needs it)
+__device__ __forceinline__ float knn_box_sbound(const float *box, int stride) {
+  float sb = 0.f;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) sb += fmaxf(box[c * stride] * box[c * stride], box[(3 + c) * stride] * box[(3 + c) * stride]);
+  return sb * 1.0001f;
+}
+
+// sbound[b * 8] = the largest m of a 256-thread CTA (each thread's bound on max |p|^2 over its points), widened for rounding
+__device__ __forceinline__ void knn_block_sbound(float m, int tid, float *sbound, int b) {
+  __shared__ float red[8];
+  m = hg_warp_max_f32(m);
+  if ((tid & 31) == 0) red[tid >> 5] = m;
+  __syncthreads();
+  if (tid == 0) {
+    for (int w = 1; w < 8; ++w) m = fmaxf(m, red[w]);
+    sbound[(size_t)b * 8] = m * 1.0001f;
+  }
+}
 
 __device__ __forceinline__ int morton3_4bit(int x, int y, int z) {
   auto spread = [](int v) { return (v & 1) | ((v & 2) << 2) | ((v & 4) << 4) | ((v & 8) << 6); };
@@ -523,12 +553,7 @@ __global__ void __launch_bounds__(256) knn_seed_small_kernel(const float *__rest
     const float ext = sbox[3 + c] - mn[c];
     inv[c] = (ext > 0.f && ext < CUDART_INF_F) ? (float)(1 << kMortonBits) / ext : 0.f;
   }
-  if (tid == 0) {  // upper bound on max |p|^2 (farthest bounding-box corner), for the folded filter's slack
-    float sb = 0.f;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) sb += fmaxf(sbox[c] * sbox[c], sbox[3 + c] * sbox[3 + c]);
-    sbound[(size_t)b * 8] = sb * 1.0001f;
-  }
+  if (tid == 0) sbound[(size_t)b * 8] = knn_box_sbound(sbox, 1);
   for (int i = tid; i < N; i += 256) {
     int cc[3];
 #pragma unroll
@@ -586,25 +611,49 @@ __global__ void __launch_bounds__(256) knn_seed_small_kernel(const float *__rest
     const int t0 = max(0, min(s - win / 2, N - win)), t1 = min(N, t0 + win);
     for (int t = t0; t < t1; ++t) {
       const float4 r = spts[t];
-      float d = knn_seed_dist(a0, a1, a2, a3, r.x, r.y, r.z, r.w);
-#pragma unroll
-      for (int u = 0; u < KM; ++u) {  // v stays sorted ascending: each level keeps the smaller, passes the larger on
-        const float l = fminf(v[u], d);
-        d = fmaxf(v[u], d);
-        v[u] = l;
-      }
+      hg_sorted_min_insert(v, knn_seed_dist(a0, a1, a2, a3, r.x, r.y, r.z, r.w));
     }
     float bound = -CUDART_INF_F;  // v[k1-1] = the largest of the first k1 entries (v is ascending); written as a max
 #pragma unroll                    // so that the list stays in registers (a runtime index would move it to local memory)
     for (int t = 0; t < KM; ++t)
       if (t < k1) bound = fmaxf(bound, v[t]);
-    thr0[(size_t)b * N + sidx[s]] = (bound < CUDART_INF_F) ? nextafterf(bound, CUDART_INF_F) : CUDART_INF_F;
+    thr0[(size_t)b * N + sidx[s]] = hg_nudge_up(bound);
   }
 }
 
 // Test-only override of the instantiation launch_form / launch_qt would pick from the problem size (0 = automatic):
 // lets small seeded inputs reach every (QT, GP) variant, including the ones only large batches select.
 static int g_force_qt = 0, g_force_gp = 0;
+
+// k1 -> the list length KM that serves it: f(std::integral_constant<int, KM>{}) with KM = 6, 20, 32 and, for kernels
+// instantiated with lists of 64, 64
+template <int kMaxKM, typename F>
+auto with_km(int k1, F &&f) {
+  if (k1 <= 6) return f(std::integral_constant<int, 6>{});
+  if (k1 <= 20) return f(std::integral_constant<int, 20>{});
+  if constexpr (kMaxKM > 32) {
+    if (k1 > 32) return f(std::integral_constant<int, 64>{});
+  }
+  return f(std::integral_constant<int, 32>{});
+}
+
+// One dispatch over the instantiated (KM, QT) set of both kNN kernels: up to 4 queries per lane with 6-entry lists, 2
+// with 20, 1 beyond.  A QT outside it (forced through hg_knn_force_shape) is an error.
+template <int kMaxKM, typename F>
+int with_km_qt(int k1, int qt, F &&f) {
+  return with_km<kMaxKM>(k1, [&](auto km) -> int {
+    constexpr int KM = decltype(km)::value;
+    if (qt == 1) return f(km, std::integral_constant<int, 1>{});
+    if constexpr (KM <= 20) {
+      if (qt == 2) return f(km, std::integral_constant<int, 2>{});
+    }
+    if constexpr (KM <= 6) {
+      if (qt == 4) return f(km, std::integral_constant<int, 4>{});
+    }
+    hg_set_error("knn: forced QT=%d has no instantiation for k=%d", qt, k1);
+    return HG_E_UNSUPPORTED;
+  });
+}
 
 template <int FORM, int QT, int KM, typename IdxT>
 int launch_qt(const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, IdxT *idx,
@@ -635,41 +684,28 @@ int launch_form(const float *q, const float *r, int B, int Nq, int Nr, int k1, f
   // pays on long candidate lists; on short ones (< 2k candidates) the cold-start drains dominate and run one query
   // after the other, so fewer queries per lane win (measured, k+1 = 6: 16384 points 5.96 / 6.33 / 8.72 ms for QT = 4 /
   // 2 / 1; 1024 points 2.46 / 2.14 / 2.28 ms).  Small batches additionally drop QT until the grid fills the machine.
-  const long long want = 2LL * hg_sm_count();
-  auto ctas = [&](int qt) { return (long long)B * ((Nq + qt * kThreads - 1) / (qt * kThreads)); };
-  const bool short_list = Nr < 2048;
-  if (g_force_qt) {
-    const int qt = g_force_qt;
-    if (k1 <= 6 && qt == 4) return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 <= 6 && qt == 2) return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 <= 6 && qt == 1) return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 > 6 && k1 <= 20 && qt == 2)
-      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 > 6 && k1 <= 20 && qt == 1)
-      return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 > 20 && k1 <= 32 && qt == 1)
-      return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (k1 > 32 && qt == 1) return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    hg_set_error("knn: forced QT=%d has no instantiation for k=%d", qt, k1);
-    return HG_E_UNSUPPORTED;
+  int qt = g_force_qt;
+  if (!qt) {
+    const long long want = 2LL * hg_sm_count();
+    auto ctas = [&](int qt) { return (long long)B * ((Nq + qt * kThreads - 1) / (qt * kThreads)); };
+    const bool short_list = Nr < 2048;
+    qt = 1;
+    if (k1 <= 6) {
+      // (four queries per lane need twice the CTAs to pay: 32 x 8192: 654 us with two against 695, 16 x 16384: 1080 / 1128;
+      // 64 x 8192 and up: four win -- tools/debug/knn_small_shapes.py big)
+      if (!short_list && Nq >= 3 * kThreads && ctas(4) >= 2 * want)
+        qt = 4;
+      else if (Nq > kThreads && ctas(2) >= want)
+        qt = 2;
+    } else if (k1 <= 20 && !short_list && Nq > kThreads && ctas(2) >= want) {
+      qt = 2;
+    }
   }
-  if (k1 <= 6) {
-    // (four queries per lane need twice the CTAs to pay: 32 x 8192: 654 us with two against 695, 16 x 16384: 1080 / 1128;
-    // 64 x 8192 and up: four win -- tools/debug/knn_small_shapes.py big)
-    if (!short_list && Nq >= 3 * kThreads && ctas(4) >= 2 * want)
-      return launch_qt<FORM, 4, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    if (Nq > kThreads && ctas(2) >= want)
-      return launch_qt<FORM, 2, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    return launch_qt<FORM, 1, 6, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-  }
-  if (k1 <= 20) {
-    if (!short_list && Nq > kThreads && ctas(2) >= want)
-      return launch_qt<FORM, 2, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-    return launch_qt<FORM, 1, 20, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
-  }
-  if (k1 <= 32) return launch_qt<FORM, 1, 32, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
   // 33..64 neighbours (HiT-ADV's default curv_loss_knn = 32 asks knn_points for 33): a 64-entry register list
-  return launch_qt<FORM, 1, 64, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound, stream, idx_state, only);
+  return with_km_qt<64>(k1, qt, [&](auto km, auto qt_) -> int {
+    return launch_qt<FORM, decltype(qt_)::value, decltype(km)::value, IdxT>(q, r, B, Nq, Nr, k1, vals, idx, thr0, sbound,
+                                                                            stream, idx_state, only);
+  });
 }
 
 // ---- threshold seeding for self-kNN ---------------------------------------------------------------------------
@@ -721,12 +757,7 @@ __global__ void __launch_bounds__(256) knn_cells_kernel(const float *__restrict_
     params[b * 8 + tid] = mn[tid];
     params[b * 8 + 3 + tid] = inv[tid];
   }
-  if (tid == 0) {  // upper bound on max |p|^2 over the cloud (the farthest bounding-box corner), for the folded filter
-    float sb = 0.f;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) sb += fmaxf(red[c][0] * red[c][0], red[3 + c][0] * red[3 + c][0]);
-    params[b * 8 + 6] = sb * 1.0001f;
-  }
+  if (tid == 0) params[b * 8 + 6] = knn_box_sbound(&red[0][0], 256);
   for (int i = tid; i < N; i += 256) {
     int cc[3];
 #pragma unroll
@@ -803,34 +834,17 @@ __global__ void __launch_bounds__(128) knn_seed_kernel(const float4 *__restrict_
     seen += max(te - t, 0);
     for (; t + 1 < te; t += 2) {  // two candidates in flight; insertion without branches (values only)
       const float4 r0 = pts[t], r1 = pts[t + 1];
-      float d0 = knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
-      float d1 = knn_seed_dist(a0, a1, a2, a3, r1.x, r1.y, r1.z, r1.w);
-#pragma unroll
-      for (int u = 0; u < KM; ++u) {  // v stays sorted ascending: each level keeps the smaller, passes the larger on
-        const float lo0 = fminf(v[u], d0);
-        d0 = fmaxf(v[u], d0);
-        v[u] = lo0;
-      }
-#pragma unroll
-      for (int u = 0; u < KM; ++u) {
-        const float lo1 = fminf(v[u], d1);
-        d1 = fmaxf(v[u], d1);
-        v[u] = lo1;
-      }
+      const float d0 = knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
+      const float d1 = knn_seed_dist(a0, a1, a2, a3, r1.x, r1.y, r1.z, r1.w);
+      hg_sorted_min_insert(v, d0);
+      hg_sorted_min_insert(v, d1);
     }
     if (t < te) {
       const float4 r0 = pts[t];
-      float d0 = knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w);
-#pragma unroll
-      for (int u = 0; u < KM; ++u) {
-        const float lo0 = fminf(v[u], d0);
-        d0 = fmaxf(v[u], d0);
-        v[u] = lo0;
-      }
+      hg_sorted_min_insert(v, knn_seed_dist(a0, a1, a2, a3, r0.x, r0.y, r0.z, r0.w));
     }
   }
-  const float bound = v[KM - 1];
-  thr0[(size_t)b * N + list[(size_t)b * N + s_q]] = (bound < CUDART_INF_F) ? nextafterf(bound, CUDART_INF_F) : CUDART_INF_F;
+  thr0[(size_t)b * N + list[(size_t)b * N + s_q]] = hg_nudge_up(v[KM - 1]);
 }
 
 // upper bound on max |p|^2 per cloud for the folded filter when no grid pre-pass runs: sbound[b*8] (stride 8, like params+6)
@@ -842,14 +856,7 @@ __global__ void __launch_bounds__(256) knn_bound_kernel(const float *__restrict_
     const float x = p[(size_t)i * 3], y = p[(size_t)i * 3 + 1], z = p[(size_t)i * 3 + 2];
     m = fmaxf(m, fmaf(z, z, fmaf(y, y, x * x)));
   }
-  m = hg_warp_max_f32(m);
-  __shared__ float red[8];
-  if ((tid & 31) == 0) red[tid >> 5] = m;
-  __syncthreads();
-  if (tid == 0) {
-    for (int w = 1; w < 8; ++w) m = fmaxf(m, red[w]);
-    sbound[(size_t)b * 8] = m * 1.0001f;
-  }
+  knn_block_sbound(m, tid, sbound, b);
 }
 
 // Temporal seeds (attack loops call KNNDist thousands of times on a slowly moving cloud, CW/kNN.py:77-111): the
@@ -865,7 +872,6 @@ __global__ void __launch_bounds__(256) knn_seed_prev_kernel(const float *__restr
                                                             float *__restrict__ thr0, float *__restrict__ sbound) {
   const int b = blockIdx.x, tid = threadIdx.x;
   const float *p = pc + (size_t)b * N * 3;
-  __shared__ float red[8];
   float m = 0.f;
   for (int i = tid; i < N; i += 256) {
     const float x = __ldg(p + (size_t)i * 3), y = __ldg(p + (size_t)i * 3 + 1), z = __ldg(p + (size_t)i * 3 + 2);
@@ -893,25 +899,16 @@ __global__ void __launch_bounds__(256) knn_seed_prev_kernel(const float *__restr
     for (int t = 1; t < KM; ++t)
 #pragma unroll
       for (int u = 0; u < t; ++u) ok = ok && (id[t] != id[u]);
-    thr0[(size_t)b * N + i] = (ok && bound < CUDART_INF_F) ? nextafterf(bound, CUDART_INF_F) : CUDART_INF_F;
+    thr0[(size_t)b * N + i] = ok ? hg_nudge_up(bound) : CUDART_INF_F;
   }
-  m = hg_warp_max_f32(m);
-  if ((tid & 31) == 0) red[tid >> 5] = m;
-  __syncthreads();
-  if (tid == 0) {
-    for (int w = 1; w < 8; ++w) m = fmaxf(m, red[w]);
-    sbound[(size_t)b * 8] = m * 1.0001f;
-  }
+  knn_block_sbound(m, tid, sbound, b);
 }
 
 int launch_seed_prev(const float *pc, int B, int N, int k1, const int *prev, float *thr0, float *sbound,
                      cudaStream_t stream) {
-  if (k1 <= 6)
-    knn_seed_prev_kernel<6><<<B, 256, 0, stream>>>(pc, N, k1, prev, thr0, sbound);
-  else if (k1 <= 20)
-    knn_seed_prev_kernel<20><<<B, 256, 0, stream>>>(pc, N, k1, prev, thr0, sbound);
-  else
-    knn_seed_prev_kernel<32><<<B, 256, 0, stream>>>(pc, N, k1, prev, thr0, sbound);
+  with_km<32>(k1, [&](auto km) {
+    knn_seed_prev_kernel<decltype(km)::value><<<B, 256, 0, stream>>>(pc, N, k1, prev, thr0, sbound);
+  });
   HG_CHECK_LAUNCH("knn_seed_prev_kernel");
   return HG_OK;
 }
@@ -960,21 +957,16 @@ int knn3_small_self(const float *pc, int B, int N, int k1, float *vals, int *idx
   const size_t seed_smem = (size_t)N * (sizeof(float4) + 2 * sizeof(int));
   // window of the Z-order scan: enough points for a k1-th smallest that is close to the true one
   const int win = k1 <= 8 ? 64 : (k1 <= 16 ? 80 : 96);  // measured (388 x 1024): 64 beats 32 by 5 % at k+1 = 6, 96 beats 64 by 6 % at 20
-  static HgPerDeviceOnce once[3];
-  constexpr int kSeedMaxSmem = 8192 * (int)(sizeof(float4) + 2 * sizeof(int));
-  if (k1 <= 6) {
-    if (once[0].first())
-      HG_CUDA(cudaFuncSetAttribute(knn_seed_small_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSeedMaxSmem));
-    knn_seed_small_kernel<6><<<B, 256, seed_smem, stream>>>(pc, N, k1, win, thr0, sbound);
-  } else if (k1 <= 20) {
-    if (once[1].first())
-      HG_CUDA(cudaFuncSetAttribute(knn_seed_small_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSeedMaxSmem));
-    knn_seed_small_kernel<20><<<B, 256, seed_smem, stream>>>(pc, N, k1, win, thr0, sbound);
-  } else {
-    if (once[2].first())
-      HG_CUDA(cudaFuncSetAttribute(knn_seed_small_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSeedMaxSmem));
-    knn_seed_small_kernel<32><<<B, 256, seed_smem, stream>>>(pc, N, k1, win, thr0, sbound);
-  }
+  const int rc = with_km<32>(k1, [&](auto km) -> int {
+    constexpr int kSeedMaxSmem = 8192 * (int)(sizeof(float4) + 2 * sizeof(int));
+    static HgPerDeviceOnce once;  // one per instantiation
+    if (once.first())
+      HG_CUDA(cudaFuncSetAttribute(knn_seed_small_kernel<decltype(km)::value>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   kSeedMaxSmem));
+    knn_seed_small_kernel<decltype(km)::value><<<B, 256, seed_smem, stream>>>(pc, N, k1, win, thr0, sbound);
+    return HG_OK;
+  });
+  if (rc) return rc;
   HG_CHECK_LAUNCH("knn_seed_small_kernel");
   return knn3_small_main(pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
 }
@@ -988,24 +980,15 @@ int knn3_small_main(const float *pc, int B, int N, int k1, float *vals, int *idx
   if (N > 2048 && gp < 2) gp = 2;
   if (N > 4096 && gp < 4) gp = 4;
   if (!g_force_gp && k1 > 6 && N > 3072) gp = 4;  // longer lists: 1001 against 1257 us at 64 x 4096, k+1 = 20
-  int qt = g_force_qt ? g_force_qt : 2;
   // small batches: one query per lane doubles the CTAs (32 x 1024, k+1 = 6: 51 against 65 us; tools/debug/knn_small_shapes.py)
-  // (short candidate lists only: at 16 x 4096 two queries per lane still win, 176 against 212 us)
-  if (!g_force_qt && N <= 1536 && (long long)B * ((N + 2 * kThreads - 1) / (2 * kThreads)) < 2LL * hg_sm_count()) qt = 1;
-  if (k1 <= 6) {
-    if (qt == 4) return launch_small_gp<4, 6>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (qt == 2) return launch_small_gp<2, 6>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (qt == 1) return launch_small_gp<1, 6>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-  } else if (k1 <= 20) {
-    if (!g_force_qt) qt = 1;
-    if (qt == 2) return launch_small_gp<2, 20>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-    if (qt == 1) return launch_small_gp<1, 20>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-  } else {
-    if (!g_force_qt) qt = 1;
-    if (qt == 1) return launch_small_gp<1, 32>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream, idx_state);
-  }
-  hg_set_error("knn: forced QT=%d has no instantiation for k=%d", qt, k1);
-  return HG_E_UNSUPPORTED;
+  // (short candidate lists only: at 16 x 4096 two queries per lane still win, 176 against 212 us); longer lists: one
+  int qt = g_force_qt;
+  if (!qt)
+    qt = (k1 > 6 || (N <= 1536 && (long long)B * ((N + 2 * kThreads - 1) / (2 * kThreads)) < 2LL * hg_sm_count())) ? 1 : 2;
+  return with_km_qt<32>(k1, qt, [&](auto km, auto qt_) -> int {
+    return launch_small_gp<decltype(qt_)::value, decltype(km)::value>(gp, pc, B, N, k1, vals, idx, thr0, sbound, stream,
+                                                                       idx_state);
+  });
 }
 
 int seed_grid(int N) {
@@ -1069,18 +1052,9 @@ struct Knn3SelfWorkspace {
 
 }  // namespace
 
-int hg_knn3_launch_i32(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals, int *idx,
+int hg_knn3_points_i64(const float *p1, const float *p2, int B, int N, int M, int K, float *dists, long long *idx,
                        cudaStream_t stream) {
-  return form == HG_KNN_FORM_EXPANDED
-             ? launch_form<HG_KNN_FORM_EXPANDED, int>(q, r, B, Nq, Nr, k1, vals, idx, nullptr, nullptr, stream)
-             : launch_form<HG_KNN_FORM_DIRECT, int>(q, r, B, Nq, Nr, k1, vals, idx, nullptr, nullptr, stream);
-}
-
-int hg_knn3_launch_i64(int form, const float *q, const float *r, int B, int Nq, int Nr, int k1, float *vals,
-                       long long *idx, cudaStream_t stream) {
-  return form == HG_KNN_FORM_EXPANDED
-             ? launch_form<HG_KNN_FORM_EXPANDED, long long>(q, r, B, Nq, Nr, k1, vals, idx, nullptr, nullptr, stream)
-             : launch_form<HG_KNN_FORM_DIRECT, long long>(q, r, B, Nq, Nr, k1, vals, idx, nullptr, nullptr, stream);
+  return launch_form<HG_KNN_FORM_DIRECT, long long>(p1, p2, B, N, M, K, dists, idx, nullptr, nullptr, stream);
 }
 
 size_t hg_knn3_self_workspace_bytes(int B, int N, int k1) { return hg_layout_bytes<Knn3SelfWorkspace>(B, N, k1); }
@@ -1134,8 +1108,8 @@ int hg_knn3_self_i32(const float *pc, int B, int N, int k1, float *vals, int *id
       workspace_bytes >= w.pad_end &&
       ((4LL * B * ((N + 127) / 128) >= hg_sm_count() && (long long)B * ((N + 127) / 128) <= 8LL * hg_sm_count()) ||
        g_hg_tune_knn_tc_off == 2 || g_hg_tune_knn_tc_off == 5)) {
-    const long long rows = (long long)B * N, blocks = (rows * (kPadC / 4) + 255) / 256, cap = 16LL * hg_sm_count();
-    knn_pad3_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, stream>>>(pc, rows, (float4 *)w.padded, w.padded_xx);
+    const long long rows = (long long)B * N;
+    knn_pad3_kernel<<<hg_grid_for(rows * (kPadC / 4), 256, 16), 256, 0, stream>>>(pc, rows, (float4 *)w.padded, w.padded_xx);
     HG_CHECK_LAUNCH("knn_pad3_kernel");
     return hg_knn_tc_run(w.padded, w.padded_xx, B, N, kPadC, k1, vals, idx, stream);
   }
@@ -1163,25 +1137,18 @@ int hg_knn3_self_i32(const float *pc, int B, int N, int k1, float *vals, int *id
   HgCsr csr;
   int rc = hg_csr_build_unordered(w.cellid, B, N, ncell, w.cells.ptr, w.cells.bytes, &csr, stream);
   if (rc) return rc;
-  {
-    const long long total = (long long)B * N;
-    long long blocks = (total + 255) / 256;
-    const long long cap = (long long)hg_sm_count() * 16;
-    if (blocks > cap) blocks = cap;
-    knn_cell_sort_kernel<<<(int)blocks, 256, 0, stream>>>(pc, csr.list, total, N, w.sorted);
-    HG_CHECK_LAUNCH("knn_cell_sort_kernel");
-  }
+  knn_cell_sort_kernel<<<hg_grid_for((long long)B * N, 256, 16), 256, 0, stream>>>(pc, csr.list, (long long)B * N, N,
+                                                                                     w.sorted);
+  HG_CHECK_LAUNCH("knn_cell_sort_kernel");
   dim3 grid((N + 127) / 128, B);
   // neighbourhood of the seed scan: the 2x2x2 cells nearest to the query (3.4x fewer candidates, a slightly looser
   // bound: measured 5-9 % faster end to end at k+1 = 6, 2-5 % at k+1 = 20), all 27 cells for longer lists, which the
   // ~24 points of 8 cells cannot fill (tools/knn_seed_sweep.py)
   const int near8 = g_seed_near8 == 1 ? 1 : g_seed_near8 == 2 ? 0 : (k1 <= 20);
-  if (k1 <= 6)
-    knn_seed_kernel<6><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
-  else if (k1 <= 20)
-    knn_seed_kernel<20><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
-  else
-    knn_seed_kernel<32><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0, near8);
+  with_km<32>(k1, [&](auto km) {
+    knn_seed_kernel<decltype(km)::value><<<grid, 128, 0, stream>>>(w.sorted, N, G, w.params, csr.off, csr.list, w.thr0,
+                                                                   near8);
+  });
   HG_CHECK_LAUNCH("knn_seed_kernel");
   // seeded path: the bounding box is known, so the main loop can run the 4-operation folded filter
   return launch_form<HG_KNN_FORM_EXPANDED_FOLD4, int>(pc, pc, B, N, N, k1, vals, idx, w.thr0, w.params + 6, stream, idx_state);

@@ -607,14 +607,6 @@ int launch_warps(const NnParams &p, int B, int ncg, cudaStream_t stream) {
                                     : launch_main<T, 1>(p, B, stream);
 }
 
-int grid_for(long long total, int threads) {
-  long long blocks = (total + threads - 1) / threads;
-  const long long cap = (long long)hg_sm_count() * 16;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  return (int)blocks;
-}
-
 }  // namespace
 
 // Tunables exposed for the benchmark sweep (not part of the stable ABI): T (columns per lane: 8 or 16) and
@@ -681,10 +673,10 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
                "nn_bidir: generic-D path materialises P; B*N2*N1 too large");
     float *P = hg_layout_at<NnGenericWorkspace>(workspace, B, N2, N1).P;
     const long long total = (long long)B * N2 * N1;
-    nn_generic_p_kernel<<<grid_for(total, 256), 256, 0, stream>>>(gts, preds, B, N2, N1, D, P);
+    nn_generic_p_kernel<<<hg_grid_for(total, 256, 16), 256, 0, stream>>>(gts, preds, B, N2, N1, D, P);
     HG_CHECK_LAUNCH("nn_generic_p_kernel");
-    nn_generic_min_kernel<<<grid_for((long long)B * (N1 + N2), 128), 128, 0, stream>>>(P, B, N2, N1, min1, arg1, min2,
-                                                                                         arg2);
+    nn_generic_min_kernel<<<hg_grid_for((long long)B * (N1 + N2), 128, 16), 128, 0, stream>>>(P, B, N2, N1, min1, arg1, min2,
+                                                                                                arg2);
     HG_CHECK_LAUNCH("nn_generic_min_kernel");
     return HG_OK;
   }
@@ -746,9 +738,9 @@ HG_API int hg_nn_bidir_temporal_f32(const float *gts, const float *preds, int B,
                      : launch_finish_small<8>(p, B, min1, arg1, min2, arg2, smem, stream);
   }
   if (T == 16)
-    nn_bidir_d3_finish_kernel<16><<<grid_for(total, 256), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
+    nn_bidir_d3_finish_kernel<16><<<hg_grid_for(total, 256, 16), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
   else
-    nn_bidir_d3_finish_kernel<8><<<grid_for(total, 256), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
+    nn_bidir_d3_finish_kernel<8><<<hg_grid_for(total, 256, 16), 256, 0, stream>>>(p, B, min1, arg1, min2, arg2);
   HG_CHECK_LAUNCH("nn_bidir_d3_finish_kernel");
   return HG_OK;
 }
@@ -759,7 +751,7 @@ HG_API int hg_pairwise_dist_f32(const float *x, const float *y, int B, int Nx, i
   HG_REQUIRE(x && y && P, HG_E_BADARG, "pairwise_dist: null pointer");
   HG_REQUIRE(B > 0 && Nx > 0 && Ny > 0 && D > 0, HG_E_BADARG, "pairwise_dist: sizes must be positive");
   const long long total = (long long)B * Nx * Ny;
-  nn_generic_p_kernel<<<grid_for(total, 256), 256, 0, hg_stream(stream_)>>>(x, y, B, Nx, Ny, D, P);
+  nn_generic_p_kernel<<<hg_grid_for(total, 256, 16), 256, 0, hg_stream(stream_)>>>(x, y, B, Nx, Ny, D, P);
   HG_CHECK_LAUNCH("nn_generic_p_kernel");
   return HG_OK;
 }
@@ -811,8 +803,8 @@ HG_API int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *
     if (rc) return rc;
   }
   const long long tp = (long long)B * N1 * (D > 8 ? D : 1);
-  set_loss_bwd_kernel<<<grid_for(tp, 256), 256, 0, stream>>>(preds, gts, arg1, rev2.off, rev2.list, arg2, g1, g2,
-                                                             hd_arg1, hd_arg2, B, N1, N2, D, mode, grad_preds);
+  set_loss_bwd_kernel<<<hg_grid_for(tp, 256, 16), 256, 0, stream>>>(preds, gts, arg1, rev2.off, rev2.list, arg2, g1, g2,
+                                                                    hd_arg1, hd_arg2, B, N1, N2, D, mode, grad_preds);
   HG_CHECK_LAUNCH("set_loss_bwd_kernel(preds)");
   if (grad_gts) {
     HgCsr rev1;
@@ -823,8 +815,8 @@ HG_API int hg_set_loss_bwd_f32(const float *gts, const float *preds, const int *
       if (rc) return rc;
     }
     const long long tg = (long long)B * N2 * (D > 8 ? D : 1);
-    set_loss_bwd_kernel<<<grid_for(tg, 256), 256, 0, stream>>>(gts, preds, arg2, rev1.off, rev1.list, arg1, g2, g1,
-                                                               hd_arg2, hd_arg1, B, N2, N1, D, mode, grad_gts);
+    set_loss_bwd_kernel<<<hg_grid_for(tg, 256, 16), 256, 0, stream>>>(gts, preds, arg2, rev1.off, rev1.list, arg1, g2, g1,
+                                                                      hd_arg2, hd_arg1, B, N2, N1, D, mode, grad_gts);
     HG_CHECK_LAUNCH("set_loss_bwd_kernel(gts)");
   }
   return HG_OK;

@@ -15,14 +15,6 @@
 
 namespace {
 
-int grid_for(long long total, int threads) {
-  long long blocks = (total + threads - 1) / threads;
-  const long long cap = (long long)hg_sm_count() * 32;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  return (int)blocks;
-}
-
 // cuda_utils.h:13-17 opt_n_threads -- only its value matters here: it fixes the reference FPS tie order.
 int ref_opt_n_threads(int work_size) {
   const int pow_2 = (int)(std::log((double)work_size) / std::log(2.0));
@@ -368,9 +360,9 @@ int launch_scatter_unweighted(const float *grad_out, const HgCsr &csr, int b, in
                                                                        grad_points, sc_total, sc_off);
   } else {
     const long long total = (long long)b * c * n;
-    scatter_channel_major_kernel<1, false><<<grid_for(total, 256), 256, 0, stream>>>(grad_out, nullptr, csr.off, csr.list,
-                                                                                     b, c, n, E, grad_points, sc_total,
-                                                                                     sc_off);
+    scatter_channel_major_kernel<1, false><<<hg_grid_for(total, 256, 32), 256, 0, stream>>>(grad_out, nullptr, csr.off, csr.list,
+                                                                                            b, c, n, E, grad_points, sc_total,
+                                                                                            sc_off);
   }
   return HG_OK;
 }
@@ -808,8 +800,8 @@ HG_API int hg_p2_group_concat(int b, int c, int n, int npoints, int nsample, con
   HG_REQUIRE(b > 0 && c >= 0 && n > 0 && npoints > 0 && nsample > 0, HG_E_BADARG, "group_concat: bad sizes");
   HG_REQUIRE(c == 0 || features, HG_E_BADARG, "group_concat: features is null but c > 0");
   const long long total = (long long)b * npoints * nsample;
-  group_xyz_rel_kernel<<<grid_for(total, 256), 256, 0, stream>>>(xyz, new_xyz, idx, n, npoints, nsample, 3 + c, total,
-                                                                 out);
+  group_xyz_rel_kernel<<<hg_grid_for(total, 256, 32), 256, 0, stream>>>(xyz, new_xyz, idx, n, npoints, nsample, 3 + c, total,
+                                                                        out);
   HG_CHECK_LAUNCH("group_xyz_rel_kernel");
   if (c > 0) return launch_gather(features, idx, b, c, n, npoints * nsample, out, stream, HG_PROF_GROUP, 3 + c, 3);
   return HG_OK;
@@ -888,7 +880,7 @@ HG_API int hg_p2_three_interpolate(int b, int c, int m, int n, const float *poin
         c, m, n, groups, points, idx, weight, out);
   } else {
     const long long total = (long long)b * c * n;
-    three_interpolate_kernel<<<grid_for(total, 256), 256, 0, hg_stream(stream_)>>>(b, c, m, n, points, idx, weight, out);
+    three_interpolate_kernel<<<hg_grid_for(total, 256, 32), 256, 0, hg_stream(stream_)>>>(b, c, m, n, points, idx, weight, out);
   }
   HG_CHECK_LAUNCH("three_interpolate");
   return HG_OK;
@@ -905,8 +897,8 @@ HG_API int hg_p2_three_interpolate_grad(int b, int c, int n, int m, const float 
   int rc = hg_csr_build(idx, b, n * 3, m, workspace, workspace_bytes, &csr, stream);
   if (rc) return rc;
   const long long total = (long long)b * c * m;
-  scatter_channel_major_kernel<3, true><<<grid_for(total, 256), 256, 0, stream>>>(grad_out, weight, csr.off, csr.list, b,
-                                                                                  c, m, n * 3, grad_points);
+  scatter_channel_major_kernel<3, true><<<hg_grid_for(total, 256, 32), 256, 0, stream>>>(grad_out, weight, csr.off, csr.list, b,
+                                                                                         c, m, n * 3, grad_points);
   HG_CHECK_LAUNCH("three_interpolate_grad");
   return HG_OK;
 }

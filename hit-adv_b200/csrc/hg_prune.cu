@@ -517,6 +517,7 @@ struct LexTopK {
   }
 };
 
+// not hg_nudge_up, which maps NaN to +inf: with that form prune_search_kernel compiles to different machine code
 __device__ __forceinline__ float nudge_up(float v) { return v < CUDART_INF_F ? nextafterf(v, CUDART_INF_F) : v; }
 
 // Resident CTAs per SM the search's register allocation must allow (0: no bound).  KM = 20: 4, since without a bound
@@ -625,13 +626,7 @@ __global__ void __launch_bounds__(kSearchWarps * 32, kSearchMinCtas<KM>) prune_s
       for (int c = 0; c < kLeaf; ++c) {
         const int pp = c >> 1, h = c & 1;
         const float c0 = tf[8 * pp + h], c1 = tf[8 * pp + 2 + h], c2 = tf[8 * pp + 4 + h], cw = tf[8 * pp + 6 + h];
-        float d = __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq);
-#pragma unroll
-        for (int u = 0; u < (kNN1 ? 1 : KM); ++u) {
-          const float lo = fminf(top.v[u], d);
-          d = fmaxf(top.v[u], d);
-          top.v[u] = lo;
-        }
+        hg_sorted_min_insert(top.v, __fadd_rn(__fadd_rn(cw, __fmaf_rn(a2, c2, __fmaf_rn(a1, c1, __fmul_rn(a0, c0)))), rq));
       }
       const float kth = top.v[KM - 1];
       seed = valid ? nudge_up(kth) : CUDART_INF_F;

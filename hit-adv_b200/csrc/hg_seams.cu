@@ -11,14 +11,6 @@
 
 namespace {
 
-int grid_for(long long total, int threads) {
-  long long blocks = (total + threads - 1) / threads;
-  const long long cap = (long long)hg_sm_count() * 32;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  return (int)blocks;
-}
-
 __device__ __forceinline__ float sumsq_cascade(const float *a, int C) {
   float acc0 = 0.f, acc1 = 0.f, acc2 = 0.f;
   for (int c = 0; c < C; ++c) {
@@ -226,7 +218,7 @@ HG_API int hg_square_distance_f32(const float *src, const float *dst, int B, int
     square_distance_small_c_kernel<<<grid, 256, 0, hg_stream(stream_)>>>(src, dst, N, M, C, out);
   } else {
     const long long total = (long long)B * N * M;
-    square_distance_kernel<<<grid_for(total, 256), 256, 0, hg_stream(stream_)>>>(src, dst, B, N, M, C, out);
+    square_distance_kernel<<<hg_grid_for(total, 256, 32), 256, 0, hg_stream(stream_)>>>(src, dst, B, N, M, C, out);
   }
   HG_CHECK_LAUNCH("square_distance");
   return HG_OK;
@@ -252,14 +244,14 @@ HG_API int hg_index_points_f32(const float *points, const int64_t *idx, int B, i
   const long long total = (long long)B * M * C, rows = (long long)B * M;
   const bool aligned = ((reinterpret_cast<uintptr_t>(points) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
   if (C == 3 && rows < (1LL << 31)) {
-    index_points_rows_kernel<3><<<grid_for(rows, 256), 256, 0, hg_stream(stream_)>>>(points, (const long long *)idx, N, M,
-                                                                                    (unsigned)rows, out);
+    index_points_rows_kernel<3><<<hg_grid_for(rows, 256, 32), 256, 0, hg_stream(stream_)>>>(points, (const long long *)idx, N, M,
+                                                                                           (unsigned)rows, out);
   } else if ((C & 3) == 0 && aligned && total / 4 < (1LL << 31)) {
-    index_points_vec4_kernel<<<grid_for(total / 4, 256), 256, 0, hg_stream(stream_)>>>(
+    index_points_vec4_kernel<<<hg_grid_for(total / 4, 256, 32), 256, 0, hg_stream(stream_)>>>(
         points, (const long long *)idx, N, M, C / 4, (unsigned)(total / 4), reinterpret_cast<float4 *>(out));
   } else {
-    index_points_kernel<<<grid_for(total, 256), 256, 0, hg_stream(stream_)>>>(points, (const long long *)idx, B, N, C, M,
-                                                                              out);
+    index_points_kernel<<<hg_grid_for(total, 256, 32), 256, 0, hg_stream(stream_)>>>(points, (const long long *)idx, B, N, C, M,
+                                                                                     out);
   }
   HG_CHECK_LAUNCH("index_points");
   return HG_OK;
@@ -280,14 +272,14 @@ HG_API int hg_index_points_grad_f32(const float *grad_out, const int64_t *idx, i
              "index_points_grad: workspace too small");
   const auto w = hg_layout_at<HgKeysCsr>(workspace, B, N, (long long)M, true);
   const long long te = (long long)B * M;
-  idx64_to_keys_kernel<<<grid_for(te, 256), 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
+  idx64_to_keys_kernel<<<hg_grid_for(te, 256, 32), 256, 0, stream>>>((const long long *)idx, te, N, w.keys);
   HG_CHECK_LAUNCH("idx64_to_keys");
   HgCsr csr;
   int rc = hg_csr_build(w.keys, B, M, N, w.csr.ptr, w.csr.bytes, &csr, stream);
   if (rc) return rc;
   const long long total = (long long)B * N * C;
-  index_points_grad_kernel<<<grid_for(total, 256), 256, 0, stream>>>(grad_out, csr.off, csr.list, B, N, C, M,
-                                                                     grad_points);
+  index_points_grad_kernel<<<hg_grid_for(total, 256, 32), 256, 0, stream>>>(grad_out, csr.off, csr.list, B, N, C, M,
+                                                                            grad_points);
   HG_CHECK_LAUNCH("index_points_grad");
   return HG_OK;
 }
